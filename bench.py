@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--clips C | --total-clips T] [--precision bf16|fp32|tf32x3]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's outputs as DIR/<name>.npy
     python bench.py --impl reference ...      # the UNMODIFIED reference's per-frame loop on the host cores
     python bench.py --workload match_sweep    # BASELINE config 3 alone (4096 queries x --sweep-rows rows x 23040)
     python -m torch.distributed.run ... bench.py --workload match_sharded --gpus N   # BASELINE config 5 alone
@@ -57,7 +58,12 @@ def parse_args():
     ap.add_argument("--latency-frames", type=int, default=200)
     ap.add_argument("--no-latency", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last of them computed (every rank's clips) as DIR/<name>.npy "
+                    "in float32 / float64, at most 64 MB in all (a fixed, seeded sample of clips beyond that)")
     a = ap.parse_args()
+    if a.dump_outputs and (a.impl != "b200" or a.workload != "characterize"):
+        ap.error("--dump-outputs needs --impl b200 --workload characterize")
     if a.total_clips:
         a.clips = max(1, a.total_clips // max(1, int(os.environ.get("WORLD_SIZE", "1"))))
     return a
@@ -562,6 +568,8 @@ def run_b200(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_total = float(t.item())
     value = world * B * K / (ms_total * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, sess, dist, rank, world)   # before the end-to-end pass below advances the session
 
     # ---- end to end through the public API with HOST buffers: every step copies its inputs from pinned
     # host memory, runs the frame and copies the pose structs back; the H2D of step i+1 overlaps step i ----
@@ -643,6 +651,40 @@ def run_b200(args):
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         line["cpu_baseline"], _, _ = cpu_baseline_record(args)
     finish(line)
+
+
+DUMP_LIMIT_BYTES = 63_000_000      # array bytes; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir, sess, dist=None, rank=0, world=1):
+    """What the timed step hands its caller, as of the step that ran last: the FrameOut fields of every clip (pose,
+    blended and IK poses, source root: what CharacterizationSession.collect() returns, float64), the network output Y
+    and the matched DB row and its distance. Every rank's clips are gathered (rank r holds clips r*B .. r*B+B-1) and
+    rank 0 writes them. Above DUMP_LIMIT_BYTES a fixed, seeded sample of clips is written; clip_index.npy says which
+    clips the rows are."""
+    import numpy as np
+    import torch
+    torch.cuda.synchronize()
+    outs = sess.post.read()
+    outs["Y"] = sess.Y.cpu().numpy()
+    outs["match_idx"] = sess.match_idx.cpu().numpy().astype(np.float64)
+    outs["match_dist"] = sess.match_dist.cpu().numpy()
+    if world > 1:
+        parts = [None] * world
+        dist.all_gather_object(parts, outs)
+        if rank != 0:
+            return
+        outs = {k: np.concatenate([p[k] for p in parts]) for k in outs}
+    B = len(outs["Y"])
+    per_clip = sum(a.nbytes for a in outs.values()) // B + 8
+    keep = np.arange(B)
+    if per_clip * B > DUMP_LIMIT_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(B, DUMP_LIMIT_BYTES // per_clip, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    outs = {k: v[keep] for k, v in outs.items()}
+    outs["clip_index"] = keep.astype(np.float64)
+    for name, a in outs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 def roofline_pass(args, sess, torch, lib, _lib):

@@ -44,7 +44,11 @@ def _final_payload(rot, pos, parents_t):
 
 
 def characterize(src_clip: dict, cha_clip: dict, raw_stats: dict, gen_sd=None, cvae_sd=None, eps_seq=None,
-                 precision: str = "fp32", encode_batch: int = 32, deterministic: bool = False) -> dict:
+                 precision: str = "fp32", encode_batch: int = 32, deterministic: bool = False,
+                 with_cm_path: bool = False) -> dict:
+    """with_cm_path: also run the reference loop's second decode of every frame, the matched DB row's ("cm_trans",
+    :465-472), and return its network output rows (Ytil_cm_rows) and the condition and normalised sample of the first
+    CVAE call (cvae_cond0, cvae_out0, frame 1)."""
     dev = "cuda"
     gen_sd = gen_sd or weights.generator_state_dict(1777)
     cvae_sd = cvae_sd or weights.cvae_state_dict(1778)
@@ -67,11 +71,12 @@ def characterize(src_clip: dict, cha_clip: dict, raw_stats: dict, gen_sd=None, c
         nms.append(enc_sess.cnt_nm[:m].clone())
     del enc_sess
     sess = CharacterizationSession(gen_sd, cvae_sd, weights.DEFAULT_MODEL_CFG, stats, torch.cat(encs), torch.cat(nms),
-                                   batch=1, device=dev, precision=precision, match_tensor_cores=False)
+                                   batch=1, device=dev, precision=precision, match_tensor_cores=False,
+                                   with_cm_path=with_cm_path)
     sess.deterministic = deterministic
     nwin = src["X"].shape[0]
     T = sess.T
-    frames, match, ytil_rows = [], [], []
+    frames, match, ytil_rows, cm_rows, extra = [], [], [], [], {}
     for i in range(nwin):
         sess.X.copy_(src["X"][i:i + 1])
         sess.side[:, :T * 3].copy_(src["Yvel"][i, :, 1].reshape(1, T * 3))
@@ -89,6 +94,10 @@ def characterize(src_clip: dict, cha_clip: dict, raw_stats: dict, gen_sd=None, c
         frames.append(sess.post.read())
         match.append(int(sess.match_idx[0, 0]))
         ytil_rows.append(((sess.Y[0, -1] - sess.Y_mean) / sess.Y_std).cpu().numpy())
+        if with_cm_path:
+            cm_rows.append(((sess.cm_Y[0, -1] - sess.Y_mean) / sess.Y_std).cpu().numpy())
+            if i == 1:      # read before capture() at frame 2, whose warm-up frame overwrites these buffers
+                extra = {"cvae_cond0": sess.cond.cpu().numpy(), "cvae_out0": sess.cvae_out.cpu().numpy()}
     par = kin.parents_tensor(skeleton.BONE_PARENTS, dev)
     # source pose sequence: local pose of each window's last frame with the integrated root (:480-488)
     src_pos = src["Ypos"][:, -1].cpu().numpy().astype(np.float32)
@@ -99,7 +108,9 @@ def characterize(src_clip: dict, cha_clip: dict, raw_stats: dict, gen_sd=None, c
     ik_rot = np.stack([f["ik_rot"][0] for f in frames])
     src_eul, src_p = _final_payload(src_rot, src_pos, par)
     our_eul, our_p = _final_payload(ik_rot, ik_pos, par)
-    return {"src_rotations": src_eul, "src_positions": src_p, "ours_rotations": our_eul, "ours_positions": our_p,
+    if with_cm_path:
+        extra["Ytil_cm_rows"] = np.stack(cm_rows)
+    return {**extra, "src_rotations": src_eul, "src_positions": src_p, "ours_rotations": our_eul, "ours_positions": our_p,
             "match": np.array(match), "Ytil_last_rows": np.stack(ytil_rows),
             "trans_pos": np.stack([f["blend_pos"][0] for f in frames]),
             "trans_rot": np.stack([f["rot"][0] for f in frames]), "n_db": int(n_cha)}

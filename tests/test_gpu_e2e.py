@@ -62,6 +62,33 @@ def test_characterised_payload(run):
 
 
 # ---------------------------------------------------------------------------------------------------
+# the reference loop's second decode of every frame (the matched DB row's, 'cm_trans') and its first CVAE call
+# ---------------------------------------------------------------------------------------------------
+@pytest.fixture(scope="module")
+def run_cm(golden_dir):
+    g = np.load(os.path.join(golden_dir, "e2e.npz"))
+    out = characterize(synthetic.make_clip(240, 0), synthetic.make_clip(400, 1), synthetic.make_norm_stats(),
+                       eps_seq=g["eps"], precision="fp32", with_cm_path=True)
+    return g, out
+
+
+def test_first_cvae_call(run_cm):
+    g, out = run_cm
+    np.testing.assert_allclose(out["cvae_cond0"], g["cvae_cond0"], rtol=1e-4, atol=1e-4)
+    err = np.abs(out["cvae_out0"] - g["cvae_out0"]).max() / np.abs(g["cvae_out0"]).max()
+    assert err < 1e-4, err
+
+
+def test_network_outputs_both_decodes(run_cm):
+    g, out = run_cm
+    ref = g["Ytil_last_rows"]                   # per frame: the 'trans' decode, then the 'cm_trans' decode
+    got = np.stack([out["Ytil_last_rows"], out["Ytil_cm_rows"]], axis=1).reshape(ref.shape)
+    rel = np.abs(got - ref).reshape(len(ref), -1).max(axis=1) / np.abs(ref).max()
+    assert rel[:4].max() < 1e-4, rel[:4]
+    assert rel.max() < 2e-3, (rel.argmax(), rel.max())         # 224 autoregressive CVAE steps
+
+
+# ---------------------------------------------------------------------------------------------------
 # the same 225-frame clip in the throughput mode (bf16 operands on tcgen05): 224 autoregressive CVAE steps
 # ---------------------------------------------------------------------------------------------------
 @pytest.fixture(scope="module")
