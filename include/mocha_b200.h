@@ -295,6 +295,13 @@ int mocha_db_pack_bf16(const float* d_rows, long long N, int D, void* d_rows16, 
 int mocha_topk_merge(const double* d_dist, const int64_t* d_idx, int nshard, int nq, int k,
                      double* d_out_dist, int64_t* d_out_idx, mocha_stream_t stream);
 
+/* Seed of the autoregression for clips that start on this frame (test_fullframework.py:298, per clip): for every
+ * b < B with d_start[b] != 0, d_dst[b] = d_table[d_idx[b * idx_stride]] (rows of row_elems floats, e.g. prev_cha[b] =
+ * cha_encoded[match_idx[b, 0]]); other rows are not touched, and an index outside [0, N) leaves the row unchanged.
+ * d_start uint8 [B]; d_table [N, row_elems] and d_dst [B, row_elems] 16 B aligned, row_elems % 4 == 0. */
+int mocha_seed_rows(const uint8_t* d_start, const int64_t* d_idx, int idx_stride, const float* d_table, long long N,
+                    long long row_elems, float* d_dst, int B, mocha_stream_t stream);
+
 /* ---- peer-memory exchange of the DB-sharded matcher (one process per GPU, NVLink / NVSwitch P2P) ----
  * Fused replacement of "all-gather the [nq,k] lists, then merge" (sharded.py): ONE kernel per rank stores
  * its local lists into a slot of every peer's exchange buffer (plain P2P stores over NVLink), raises a
@@ -406,6 +413,14 @@ int mocha_post_frame(const mocha_post_params* params, const float* d_Y, const fl
 int mocha_post_frame_packed(const mocha_post_params* params, const float* d_Y, const float* d_side, int side_stride,
                             const uint8_t* d_contacts, int B, int T, int V, int Cin, int init,
                             mocha_clip_state* d_state, mocha_frame_out* d_out, mocha_stream_t stream);
+
+/* Same as mocha_post_frame_packed with the frame-0 decision made per clip on the device (clip admission): clip b runs
+ * the init frame (:337-434: root from the identity, blend / IK lists from the raw pose, contacts reset from the toe FK)
+ * iff d_start[b] != 0 and a steady-state step otherwise, bit-identical to the init = 1 / init = 0 calls above.
+ * d_start uint8 [B]. */
+int mocha_post_frame_packed_masked(const mocha_post_params* params, const float* d_Y, const float* d_side, int side_stride,
+                                   const uint8_t* d_contacts, const uint8_t* d_start, int B, int T, int V, int Cin,
+                                   mocha_clip_state* d_state, mocha_frame_out* d_out, mocha_stream_t stream);
 
 /* ---- window feature extraction: re-rooting block of the driver's set-up (test_fullframework.py:148-158,:180-186) ---
  * Inputs are quat.fk_vel's outputs over all frames of all windows, [W,T,J,{4,3,3,3}] fp32. Every window is expressed

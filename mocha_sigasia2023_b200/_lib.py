@@ -185,6 +185,8 @@ SIGNATURES = {
     "mocha_quat_op": (_I, [_I, _I, _P, _P, _L, C.c_double, _P, _P]),
     "mocha_fk_chain": (_I, [_I, _P, _P, _P, _P, _L, _I, _P, _P, _P]),
     "mocha_post_frame_packed": (_I, [C.POINTER(PostParams), _P, _P, _I, _P, _I, _I, _I, _I, _I, _P, _P, _P]),
+    "mocha_post_frame_packed_masked": (_I, [C.POINTER(PostParams), _P, _P, _I, _P, _P, _I, _I, _I, _I, _P, _P, _P]),
+    "mocha_seed_rows": (_I, [_P, _P, _I, _P, _L, _L, _P, _I, _P]),
     "mocha_contact_update": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _L, _D, _D, _D, _D, _P]),
     "mocha_ik_two_bone": (_I, [_P] * 10 + [_D, _L, _P, _P, _P]),
     "mocha_pose_transition": (_I, [_P] * 16 + [_L, _I, _P, _P, _P, _P, _P]),

@@ -500,21 +500,57 @@ __device__ void ik_two_bone_dev(D3 bone_root, D3 bone_mid, D3 bone_end, D3 targe
 }
 
 // ------------------------------------------------------------------------------------------------
+// Frame-0 pieces shared by both post-process kernels (one definition, so the general kernel's init frame and the
+// step kernel's per-clip init agree bit for bit).
+// ------------------------------------------------------------------------------------------------
+// source root at frame 0 (:476-483): integrated from the identity in fp64, stored as float32 values like the reference
+__device__ __forceinline__ void src_root_init_dev(mocha_frame_out& O, V3<float> rv, V3<float> ra, double dt) {
+  const D3 p0 = dt * v3<double>((double)rv.x, (double)rv.y, (double)rv.z);
+  const DQ r0 = q_from_scaled_angle_axis(dt * v3<double>((double)ra.x, (double)ra.y, (double)ra.z));
+  st3(O.src_root_vel, v3<double>((double)rv.x, (double)rv.y, (double)rv.z));
+  st3(O.src_root_ang, v3<double>((double)ra.x, (double)ra.y, (double)ra.z));
+  st3(O.src_root_pos, v3<double>((double)(float)p0.x, (double)(float)p0.y, (double)(float)p0.z));
+  st4(O.src_root_rot, q4<double>((double)(float)r0.w, (double)(float)r0.x, (double)(float)r0.y, (double)(float)r0.z));
+}
+
+// contact reset of foot f at frame 0 (:403-431): quat.fk_vel_bone (motion/quat.py:207-237) along the toe's ancestor
+// chain (chain[0] = toe ... chain[n-1] = root) on the raw pose, then position = point = target = the toe
+__device__ __forceinline__ void contact_init_dev(mocha_clip_state& S, const mocha_frame_out& O, const int* chain, int n,
+                                                 int f) {
+  D3 gp = ld3(O.pos[chain[n - 1]]), gv = ld3(O.vel[chain[n - 1]]), ga = ld3(O.ang[chain[n - 1]]);
+  DQ gr = ld4(O.rot[chain[n - 1]]);
+  for (int k = n - 2; k >= 0; --k) {
+    const int j = chain[k];
+    const D3 rp = qrot(gr, ld3(O.pos[j]));
+    const D3 nv = gv + qrot(gr, ld3(O.vel[j])) + cross(ga, rp);
+    const D3 na = qrot(gr, ld3(O.ang[j])) + ga;
+    gp = rp + gp; gv = nv; ga = na;
+    gr = qmul(gr, ld4(O.rot[j]));
+  }
+  S.contact_state[f] = 0; S.contact_lock[f] = 0;
+  st3(S.contact_position[f], gp); st3(S.contact_velocity[f], gv);
+  st3(S.contact_point[f], gp); st3(S.contact_target[f], gp);
+  st3(S.contact_offset_position[f], v3<double>(0, 0, 0)); st3(S.contact_offset_velocity[f], v3<double>(0, 0, 0));
+}
+
+// ------------------------------------------------------------------------------------------------
 // per-frame post-process, one WARP per clip: lanes split the 60-frame speed-ratio reduction, the 24
 // joints of the pose assembly, the 25 bones of the blending and the two feet of the contact / IK step;
 // lane 0 integrates the roots. Phases exchange data through the clip's output struct (__syncwarp).
+// start != NULL: clip b runs the frame-0 branch iff start[b] != 0 (per-clip admission; `init` is ignored).
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(128)
 post_frame_kernel(const mocha_post_params P, const float* __restrict__ Y,
                   const float* __restrict__ src_hips_vel, const float* __restrict__ src_rvel,
                   const float* __restrict__ src_rang, const uint8_t* __restrict__ contacts, int B,
-                  int T, int V, int Cin, int init, mocha_clip_state* __restrict__ states,
+                  int T, int V, int Cin, int init, const uint8_t* __restrict__ start, mocha_clip_state* __restrict__ states,
                   mocha_frame_out* __restrict__ outs, int hv_stride, int rv_stride) {
   pdl_trigger();
   pdl_wait();
   const int b = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (b >= B) return;  // warp-uniform
+  if (start) init = start[b] != 0;   // warp-uniform (one warp per clip)
   mocha_clip_state& S = states[b];
   mocha_frame_out& O = outs[b];
   const int J = P.J;
@@ -554,12 +590,7 @@ post_frame_kernel(const mocha_post_params P, const float* __restrict__ Y,
     const V3<float> rv = v3<float>(src_rvel[(long long)b * rv_stride + 0], src_rvel[(long long)b * rv_stride + 1], src_rvel[(long long)b * rv_stride + 2]);
     const V3<float> ra = v3<float>(src_rang[(long long)b * rv_stride + 0], src_rang[(long long)b * rv_stride + 1], src_rang[(long long)b * rv_stride + 2]);
     if (init) {
-      const D3 p0 = dt * v3<double>((double)rv.x, (double)rv.y, (double)rv.z);
-      const DQ r0 = q_from_scaled_angle_axis(dt * v3<double>((double)ra.x, (double)ra.y, (double)ra.z));
-      st3(O.src_root_vel, v3<double>((double)rv.x, (double)rv.y, (double)rv.z));
-      st3(O.src_root_ang, v3<double>((double)ra.x, (double)ra.y, (double)ra.z));
-      st3(O.src_root_pos, v3<double>((double)(float)p0.x, (double)(float)p0.y, (double)(float)p0.z));
-      st4(O.src_root_rot, q4<double>((double)(float)r0.w, (double)(float)r0.x, (double)(float)r0.y, (double)(float)r0.z));
+      src_root_init_dev(O, rv, ra, dt);
     } else {
       const Q4<float> pr = q4<float>((float)S.src_root_rot[0], (float)S.src_root_rot[1], (float)S.src_root_rot[2],
                                      (float)S.src_root_rot[3]);
@@ -598,24 +629,9 @@ post_frame_kernel(const mocha_post_params P, const float* __restrict__ Y,
       for (int c = 0; c < 4; ++c) O.ik_rot[j][c] = O.rot[j][c];
     }
     if (lane < 2) {
-      const int f = lane;
-      // quat.fk_vel_bone (motion/quat.py:207-237) along the ancestor chain of the toe
       int chain[MAXJ]; int n = 0;
-      for (int j = P.contact_bones[f]; j >= 0; j = P.parents[j]) chain[n++] = j;
-      D3 gp = ld3(O.pos[chain[n - 1]]), gv = ld3(O.vel[chain[n - 1]]), ga = ld3(O.ang[chain[n - 1]]);
-      DQ gr = ld4(O.rot[chain[n - 1]]);
-      for (int k = n - 2; k >= 0; --k) {
-        const int j = chain[k];
-        const D3 rp = qrot(gr, ld3(O.pos[j]));
-        const D3 nv = gv + qrot(gr, ld3(O.vel[j])) + cross(ga, rp);
-        const D3 na = qrot(gr, ld3(O.ang[j])) + ga;
-        gp = rp + gp; gv = nv; ga = na;
-        gr = qmul(gr, ld4(O.rot[j]));
-      }
-      S.contact_state[f] = 0; S.contact_lock[f] = 0;
-      st3(S.contact_position[f], gp); st3(S.contact_velocity[f], gv);
-      st3(S.contact_point[f], gp); st3(S.contact_target[f], gp);
-      st3(S.contact_offset_position[f], v3<double>(0, 0, 0)); st3(S.contact_offset_velocity[f], v3<double>(0, 0, 0));
+      for (int j = P.contact_bones[lane]; j >= 0; j = P.parents[j]) chain[n++] = j;
+      contact_init_dev(S, O, chain, n, lane);
     }
     if (lane == 0) { st3(S.root_pos, rootpos); st4(S.root_rot, rootrot); }
     return;
@@ -686,17 +702,21 @@ post_frame_kernel(const mocha_post_params P, const float* __restrict__ Y,
 // round of independent loads, runs the phases on shared-memory copies of the two structs (same expressions, same order:
 // fp64 results as above), and writes both structs back with 16-byte stores. The ancestor chains of the two contact bones
 // depend only on the parameters and are built before the grid dependency resolves.
+// MASKED: start[b] != 0 runs clip b's frame 0 instead (the general kernel's init branch: root from the identity, lists
+// from the raw pose, contacts reset from the toe FK), so clips can start on any frame of a batch. The flag is one byte per
+// block, read with the frame's other loads; the unmasked instantiation is the steady-state kernel alone.
 // ------------------------------------------------------------------------------------------------
 static_assert(sizeof(mocha_clip_state) % 16 == 0 && sizeof(mocha_frame_out) % 16 == 0, "struct copies use 16-byte vectors");
 constexpr int PF_S16 = (int)(sizeof(mocha_clip_state) / 16), PF_O16 = (int)(sizeof(mocha_frame_out) / 16);
 constexpr int PF_YMAX = 24 * 15;   // last pose row: V <= 24 joints x 15 features
 
+template <bool MASKED>
 __global__ void __launch_bounds__(32)
 post_frame_step_kernel(const __grid_constant__ mocha_post_params P, const float* __restrict__ Y,
                        const float* __restrict__ src_hips_vel, const float* __restrict__ src_rvel,
-                       const float* __restrict__ src_rang, const uint8_t* __restrict__ contacts, int T, int V, int Cin,
-                       mocha_clip_state* __restrict__ states, mocha_frame_out* __restrict__ outs, int hv_stride,
-                       int rv_stride) {
+                       const float* __restrict__ src_rang, const uint8_t* __restrict__ contacts,
+                       const uint8_t* __restrict__ start, int T, int V, int Cin, mocha_clip_state* __restrict__ states,
+                       mocha_frame_out* __restrict__ outs, int hv_stride, int rv_stride) {
   pdl_trigger();
   __shared__ __align__(16) mocha_frame_out Osh;
   __shared__ __align__(16) mocha_clip_state Ssh;
@@ -748,6 +768,7 @@ post_frame_step_kernel(const __grid_constant__ mocha_post_params P, const float*
 #pragma unroll
   for (int c = 0; c < 3; ++c) { rvf[c] = src_rvel[(long long)b * rv_stride + c]; raf[c] = src_rang[(long long)b * rv_stride + c]; }
   const bool contact_in = lane < 2 ? contacts[b * 2 + lane] != 0 : false;
+  const bool init = MASKED && start[b] != 0;   // block-uniform
 
 #pragma unroll
   for (int k = 0; k < (PF_S16 + 31) / 32; ++k) {
@@ -782,11 +803,11 @@ post_frame_step_kernel(const __grid_constant__ mocha_post_params P, const float*
 
   DQ rootrot = q4<double>(1.0, 0.0, 0.0, 0.0);
   if (lane == 0) {
-    // root integration (:500-503)
+    // root integration (:500-503 / :345-348)
     const D3 yrvel = v3<double>((double)(rvf[0] * ratio), (double)(rvf[1] * ratio), (double)(rvf[2] * ratio));
     const D3 yrang = v3<double>((double)raf[0], (double)raf[1], (double)raf[2]);
-    const DQ prev_rot = ld4(S.root_rot);
-    const D3 prev_pos = ld3(S.root_pos);
+    const DQ prev_rot = init ? q4<double>(1.0, 0.0, 0.0, 0.0) : ld4(S.root_rot);
+    const D3 prev_pos = init ? v3<double>(0.0, 0.0, 0.0) : ld3(S.root_pos);
     const D3 rootvel = qrot(prev_rot, yrvel);
     const D3 rootang = qrot(prev_rot, yrang);
     const D3 rootpos = prev_pos + dt * rootvel;
@@ -796,17 +817,21 @@ post_frame_step_kernel(const __grid_constant__ mocha_post_params P, const float*
     // source root (:476-483): float32 arrays in the reference, so fp32 integration
     const V3<float> rv = v3<float>(rvf[0], rvf[1], rvf[2]);
     const V3<float> ra = v3<float>(raf[0], raf[1], raf[2]);
-    const Q4<float> pr = q4<float>((float)S.src_root_rot[0], (float)S.src_root_rot[1], (float)S.src_root_rot[2],
-                                   (float)S.src_root_rot[3]);
-    const V3<float> pp = v3<float>((float)S.src_root_pos[0], (float)S.src_root_pos[1], (float)S.src_root_pos[2]);
-    const float dtf = (float)dt;
-    const V3<float> wv = qrot(pr, rv), wa = qrot(pr, ra);
-    const V3<float> np_ = pp + dtf * wv;
-    const Q4<float> nr = qmul(pr, q_from_scaled_angle_axis(dtf * wa));
-    st3(O.src_root_vel, v3<double>((double)wv.x, (double)wv.y, (double)wv.z));
-    st3(O.src_root_ang, v3<double>((double)wa.x, (double)wa.y, (double)wa.z));
-    st3(O.src_root_pos, v3<double>((double)np_.x, (double)np_.y, (double)np_.z));
-    st4(O.src_root_rot, q4<double>((double)nr.w, (double)nr.x, (double)nr.y, (double)nr.z));
+    if (init) {
+      src_root_init_dev(O, rv, ra, dt);
+    } else {
+      const Q4<float> pr = q4<float>((float)S.src_root_rot[0], (float)S.src_root_rot[1], (float)S.src_root_rot[2],
+                                     (float)S.src_root_rot[3]);
+      const V3<float> pp = v3<float>((float)S.src_root_pos[0], (float)S.src_root_pos[1], (float)S.src_root_pos[2]);
+      const float dtf = (float)dt;
+      const V3<float> wv = qrot(pr, rv), wa = qrot(pr, ra);
+      const V3<float> np_ = pp + dtf * wv;
+      const Q4<float> nr = qmul(pr, q_from_scaled_angle_axis(dtf * wa));
+      st3(O.src_root_vel, v3<double>((double)wv.x, (double)wv.y, (double)wv.z));
+      st3(O.src_root_ang, v3<double>((double)wa.x, (double)wa.y, (double)wa.z));
+      st3(O.src_root_pos, v3<double>((double)np_.x, (double)np_.y, (double)np_.z));
+      st4(O.src_root_rot, q4<double>((double)nr.w, (double)nr.x, (double)nr.y, (double)nr.z));
+    }
     for (int c = 0; c < 3; ++c) S.src_root_pos[c] = O.src_root_pos[c];
     for (int c = 0; c < 4; ++c) S.src_root_rot[c] = O.src_root_rot[c];
   }
@@ -821,17 +846,28 @@ post_frame_step_kernel(const __grid_constant__ mocha_post_params P, const float*
   }
   __syncwarp();
 
-  // position blending (:532-536, :626); lane = bone
-  for (int j = lane; j < J; j += 32) {
-    for (int c = 0; c < 3; ++c) {
-      O.ik_pos[j][c] = (S.prev_ik_pos[j][c] + O.vel[j][c] * dt) * 0.5 + O.pos[j][c] * 0.5;
-      O.blend_pos[j][c] = (S.prev_pos[j][c] + O.vel[j][c] * dt) * 0.5 + O.pos[j][c] * 0.5;
+  if (init) {
+    // frame 0 (:375-434): the lists start from the raw pose (the carry step below copies them into the state, and
+    // blend_pos[0] is the identity-integrated root)
+    for (int j = lane; j < J; j += 32) {
+      for (int c = 0; c < 3; ++c) { O.blend_pos[j][c] = O.pos[j][c]; O.ik_pos[j][c] = O.pos[j][c]; }
+      for (int c = 0; c < 4; ++c) O.ik_rot[j][c] = O.rot[j][c];
     }
-    for (int c = 0; c < 4; ++c) O.ik_rot[j][c] = O.rot[j][c];
+  } else {
+    // position blending (:532-536, :626); lane = bone
+    for (int j = lane; j < J; j += 32) {
+      for (int c = 0; c < 3; ++c) {
+        O.ik_pos[j][c] = (S.prev_ik_pos[j][c] + O.vel[j][c] * dt) * 0.5 + O.pos[j][c] * 0.5;
+        O.blend_pos[j][c] = (S.prev_pos[j][c] + O.vel[j][c] * dt) * 0.5 + O.pos[j][c] * 0.5;
+      }
+      for (int c = 0; c < 4; ++c) O.ik_rot[j][c] = O.rot[j][c];
+    }
   }
   __syncwarp();
 
-  if (P.ik_enabled && lane < 2) {
+  if (init) {
+    if (lane < 2) contact_init_dev(S, O, chain_s[lane], chain_n[lane], lane);
+  } else if (P.ik_enabled && lane < 2) {
     const int f = lane;
     const int* ch = chain_s[f];
     const int n = chain_n[f];
@@ -1097,7 +1133,8 @@ extern "C" int mocha_ik(const float* grot, const float* gpos, const int32_t* par
 namespace {
 int post_frame_launch(const mocha_post_params* params, const float* Y, const float* src_hips_vel, const float* src_rvel,
                       const float* src_rang, int hv_stride, int rv_stride, const uint8_t* contacts, int B, int T, int V,
-                      int Cin, int init, mocha_clip_state* state, mocha_frame_out* out, mocha_stream_t stream) {
+                      int Cin, int init, const uint8_t* start, mocha_clip_state* state, mocha_frame_out* out,
+                      mocha_stream_t stream) {
   MOCHA_CHECK_ARG(params && Y && src_hips_vel && src_rvel && src_rang && contacts && state && out && B > 0,
                   "mocha_post_frame: null/empty argument");
   MOCHA_CHECK_ARG(params->J == V + 1 && params->J <= 25, "mocha_post_frame: J=%d must equal V+1=%d and be <= 25",
@@ -1113,15 +1150,19 @@ int post_frame_launch(const mocha_post_params* params, const float* Y, const flo
                     "mocha_post_frame: contact bone %d needs 4 ancestors", params->contact_bones[f]);
   }
   // steady state: the latency-shaped kernel (shared-memory structs, one load round); frame 0 and unaligned struct arrays
-  // take the general kernel
+  // take the general kernel. A per-clip start row (start != NULL) takes the masked step kernel under the same rule.
   static const bool no_step_kernel = getenv("MOCHA_NO_POST_STEP_KERNEL") != nullptr;
   const bool aligned = ((reinterpret_cast<uintptr_t>(state) | reinterpret_cast<uintptr_t>(out)) & 15) == 0;
-  if (!init && aligned && !no_step_kernel && V * Cin <= PF_YMAX)
-    launch_k(post_frame_step_kernel, B, 32, 0, (cudaStream_t)stream, *params, Y, src_hips_vel, src_rvel, src_rang, contacts, T, V,
-             Cin, state, out, hv_stride, rv_stride);
+  const bool step_kernel = aligned && !no_step_kernel && V * Cin <= PF_YMAX;
+  if (start && step_kernel)
+    launch_k(post_frame_step_kernel<true>, B, 32, 0, (cudaStream_t)stream, *params, Y, src_hips_vel, src_rvel, src_rang, contacts,
+             start, T, V, Cin, state, out, hv_stride, rv_stride);
+  else if (!start && !init && step_kernel)
+    launch_k(post_frame_step_kernel<false>, B, 32, 0, (cudaStream_t)stream, *params, Y, src_hips_vel, src_rvel, src_rang, contacts,
+             nullptr, T, V, Cin, state, out, hv_stride, rv_stride);
   else
     launch_k(post_frame_kernel, nblk((long long)B * 32, 128), 128, 0, (cudaStream_t)stream, *params, Y, src_hips_vel, src_rvel, src_rang,
-                                                                   contacts, B, T, V, Cin, init, state, out, hv_stride, rv_stride);
+                                                                   contacts, B, T, V, Cin, init, start, state, out, hv_stride, rv_stride);
   count_launch();
   MOCHA_LAUNCH_CHECK("post_frame_kernel");
   return MOCHA_OK;
@@ -1132,8 +1173,8 @@ extern "C" int mocha_post_frame(const mocha_post_params* params, const float* Y,
                                 const float* src_rvel, const float* src_rang, const uint8_t* contacts, int B, int T,
                                 int V, int Cin, int init, mocha_clip_state* state, mocha_frame_out* out,
                                 mocha_stream_t stream) {
-  return post_frame_launch(params, Y, src_hips_vel, src_rvel, src_rang, T * 3, 3, contacts, B, T, V, Cin, init, state, out,
-                           stream);
+  return post_frame_launch(params, Y, src_hips_vel, src_rvel, src_rang, T * 3, 3, contacts, B, T, V, Cin, init, nullptr, state,
+                           out, stream);
 }
 
 // Same with the three per-clip source-motion inputs packed in ONE row per clip, [hips vel T*3 | rvel 3 | rang 3]
@@ -1143,7 +1184,19 @@ extern "C" int mocha_post_frame_packed(const mocha_post_params* params, const fl
                                        mocha_clip_state* state, mocha_frame_out* out, mocha_stream_t stream) {
   MOCHA_CHECK_ARG(side && side_stride >= T * 3 + 6, "mocha_post_frame_packed: side rows need T*3+6 floats");
   return post_frame_launch(params, Y, side, side + T * 3, side + T * 3 + 3, side_stride, side_stride, contacts, B, T, V,
-                           Cin, init, state, out, stream);
+                           Cin, init, nullptr, state, out, stream);
+}
+
+// Per-clip frame 0 (clip admission): clip b runs the init frame iff d_start[b] != 0, every other clip a steady-state step,
+// in one launch that a captured graph can replay with a different start row every frame.
+extern "C" int mocha_post_frame_packed_masked(const mocha_post_params* params, const float* Y, const float* side,
+                                              int side_stride, const uint8_t* contacts, const uint8_t* start, int B, int T,
+                                              int V, int Cin, mocha_clip_state* state, mocha_frame_out* out,
+                                              mocha_stream_t stream) {
+  MOCHA_CHECK_ARG(start, "mocha_post_frame_packed_masked: null start row");
+  MOCHA_CHECK_ARG(side && side_stride >= T * 3 + 6, "mocha_post_frame_packed_masked: side rows need T*3+6 floats");
+  return post_frame_launch(params, Y, side, side + T * 3, side + T * 3 + 3, side_stride, side_stride, contacts, B, T, V,
+                           Cin, 0, start, state, out, stream);
 }
 
 extern "C" int mocha_contact_update(int32_t* state, int32_t* lock, double* position, double* velocity, double* point,

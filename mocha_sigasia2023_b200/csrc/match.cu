@@ -558,6 +558,38 @@ extern "C" int mocha_topk_merge(const double* dist, const int64_t* idx, int nsha
   return MOCHA_OK;
 }
 
+// Seed of a started clip (clip admission): dst[b] = table[idx[b * idx_stride]] for the rows whose start byte is set,
+// one block per row, 16-byte copies; rows that do not start exit after the grid dependency, and an index outside [0, N)
+// leaves the row as it is.
+__global__ void __launch_bounds__(256) seed_rows_kernel(const uint8_t* __restrict__ start, const int64_t* __restrict__ idx,
+                                                        int idx_stride, const float4* __restrict__ table, long long N,
+                                                        long long row4, float4* __restrict__ dst) {
+  pdl_trigger();
+  pdl_wait();
+  const int b = blockIdx.x;
+  if (!start[b]) return;
+  const long long r = idx[(long long)b * idx_stride];
+  if (r < 0 || r >= N) return;
+  const float4* src = table + r * row4;
+  float4* out = dst + (long long)b * row4;
+#pragma unroll 4
+  for (long long i = threadIdx.x; i < row4; i += 256) out[i] = src[i];
+}
+
+extern "C" int mocha_seed_rows(const uint8_t* start, const int64_t* idx, int idx_stride, const float* table, long long N,
+                               long long row_elems, float* dst, int B, mocha_stream_t stream) {
+  MOCHA_CHECK_ARG(start && idx && table && dst, "mocha_seed_rows: null argument");
+  MOCHA_CHECK_ARG(B > 0 && N > 0 && row_elems > 0 && idx_stride >= 1, "mocha_seed_rows: bad sizes (B=%d, N=%lld, row=%lld)",
+                  B, N, row_elems);
+  MOCHA_CHECK_ARG(row_elems % 4 == 0 && ((reinterpret_cast<uintptr_t>(table) | reinterpret_cast<uintptr_t>(dst)) & 15) == 0,
+                  "mocha_seed_rows: rows must be 16 B aligned multiples of 4 floats");
+  launch_k(seed_rows_kernel, (unsigned)B, 256, 0, (cudaStream_t)stream, start, idx, idx_stride,
+           reinterpret_cast<const float4*>(table), N, row_elems / 4, reinterpret_cast<float4*>(dst));
+  count_launch();
+  MOCHA_LAUNCH_CHECK("seed_rows_kernel");
+  return MOCHA_OK;
+}
+
 // ------------------------------------------------------------------------------------------------
 // Peer-memory exchange + merge of the DB-sharded matcher (see include/mocha_b200.h)
 // ------------------------------------------------------------------------------------------------

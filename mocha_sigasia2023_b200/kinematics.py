@@ -213,10 +213,12 @@ class PostProcessor:
             "mocha_post_frame")
         self.started = True
 
-    def step_packed(self, Y, side, contacts, lo: int = 0, init=None):
+    def step_packed(self, Y, side, contacts, lo: int = 0, init=None, start=None):
         """Same as step() with the source-motion inputs packed one row per clip:
         side [B', T*3+6] = [src_hips_vel | src_rvel | src_rang] (mocha_post_frame_packed). The B' clips are clips
-        lo .. lo+B'-1 of this processor's state / output arrays (sub-batch lanes); init overrides `started`."""
+        lo .. lo+B'-1 of this processor's state / output arrays (sub-batch lanes); init overrides `started`.
+        start (uint8 [B'] CUDA tensor): clip b runs its frame 0 iff start[b] != 0, the others a steady-state step
+        (mocha_post_frame_packed_masked); `init` and `started` are then ignored."""
         _f32(Y)
         _f32(side)
         _lib.require_cuda(contacts)
@@ -225,12 +227,20 @@ class PostProcessor:
             raise _lib.MochaError(f"side must be [B, >= T*3+6] with unit column stride, got {tuple(side.shape)}")
         if lo < 0 or lo + B > self.B:
             raise _lib.MochaError("step_packed: clip range outside this processor's state")
+        state = C.c_void_p(self.state.data_ptr() + lo * C.sizeof(_lib.ClipState))
+        out = C.c_void_p(self.out.data_ptr() + lo * C.sizeof(_lib.FrameOut))
+        if start is not None:
+            _lib.require_cuda(start)
+            if start.dtype != torch.uint8 or start.shape != (B,):
+                raise _lib.MochaError(f"start must be a uint8 [{B}] CUDA tensor, got {start.dtype} {tuple(start.shape)}")
+            _lib.check(_lib.load().mocha_post_frame_packed_masked(
+                C.byref(self.params), _lib.ptr(Y), _lib.ptr(side), side.stride(0), _lib.ptr(contacts), _lib.ptr(start),
+                B, T, V, Cin, state, out, _lib.stream_ptr()), "mocha_post_frame_packed_masked")
+            return
         init = (0 if self.started else 1) if init is None else int(bool(init))
         _lib.check(_lib.load().mocha_post_frame_packed(
             C.byref(self.params), _lib.ptr(Y), _lib.ptr(side), side.stride(0), _lib.ptr(contacts), B, T, V, Cin, init,
-            C.c_void_p(self.state.data_ptr() + lo * C.sizeof(_lib.ClipState)),
-            C.c_void_p(self.out.data_ptr() + lo * C.sizeof(_lib.FrameOut)),
-            _lib.stream_ptr()), "mocha_post_frame_packed")
+            state, out, _lib.stream_ptr()), "mocha_post_frame_packed")
         if lo == 0 and B == self.B:
             self.started = True
 

@@ -36,9 +36,19 @@ class NormStats:
 class CharacterizationSession:
     def __init__(self, gen_sd, cvae_sd, cfg, stats: NormStats, cha_encoded, cha_cnt_nm, batch: int,
                  device="cuda", precision="fp32", with_cm_path=False, match_tensor_cores=None, post_params=None,
-                 lanes: int = 1):
+                 lanes: int = 1, admission: bool = False):
         """gen_sd / cvae_sd: reference-layout state dicts. cha_encoded [N,90,256] and cha_cnt_nm [N,23040]
-        (already (cnt-mean)/std scaled): the target character's feature DB, CUDA or CPU tensors."""
+        (already (cnt-mean)/std scaled): the target character's feature DB, CUDA or CPU tensors.
+
+        admission=True: clips start in any slot on any frame. Every frame takes one more input, the uint8 [B] row
+        `start` (step_host(start=...), or a "start" entry of pinned_inputs()); a slot whose byte is 1 runs that frame as
+        frame 0 of a new clip: its matched DB row seeds the autoregression (its CVAE output is not used) and its
+        post-process state starts from the raw pose. All other slots run a steady-state frame in the same launches, so
+        one captured graph serves every frame, and capture() may run before the first one. Everything a clip carries
+        from frame to frame (prev_cha, the post-process states) is per slot and rewritten by a start, so a reused slot
+        behaves exactly like a fresh one. A slot whose clip has ended keeps computing on whatever finite inputs the
+        caller leaves in its rows; its outputs are meaningless until it is started again, and nothing of an idle or
+        previous occupant reaches a started clip. Slots that never started compute on the zero-initialised buffers."""
         self.lib = _lib.load()
         _lib.check(self.lib.mocha_check_device(), "mocha_check_device")
         dev = torch.device(device)
@@ -84,6 +94,10 @@ class CharacterizationSession:
         self.src_rang = torch.zeros((B, 3), **f32)
         self.contacts = torch.zeros((B, 2), dtype=torch.uint8, device=dev)
         self.eps = torch.zeros((B, D), **f32)
+        self.admission = bool(admission)
+        if self.admission:
+            self.start = torch.zeros((B,), dtype=torch.uint8, device=dev)     # 1 = the slot starts a new clip this frame
+        self._input_names = ("X", "side", "contacts", "eps") + (("start",) if self.admission else ())
         # intermediates
         self.tokens = torch.empty((B, n, D), **f32)
         self.encoded = torch.empty((B, n, D), **f32)
@@ -134,6 +148,8 @@ class CharacterizationSession:
         self.h_side = torch.zeros((B, d.T * 3 + 3 + 3), dtype=torch.float32).pin_memory()
         self.h_contacts = torch.zeros((B, 2), dtype=torch.uint8).pin_memory()
         self.h_eps = torch.zeros((B, D), dtype=torch.float32).pin_memory()
+        if self.admission:
+            self.h_start = torch.zeros((B,), dtype=torch.uint8).pin_memory()
         self.h_out = torch.zeros(self.post.out.shape, dtype=torch.uint8).pin_memory()
         self.side = torch.zeros((B, d.T * 3 + 3 + 3), **f32)
 
@@ -183,11 +199,55 @@ class CharacterizationSession:
                                              _lib.ptr(idx), _lib.ptr(dist), wp, wn, self._s()),
                        "match_exact")
 
-    def _frame_part(self, init: bool, lo: int, hi: int, ws):
-        """One lane: clips [lo, hi) from the input buffers to the FrameOut buffer, on the current stream."""
+    def _cvae_step(self, lo: int, hi: int, ws):
+        """condition + CVAE sample of clips [lo, hi): prev_cha becomes this frame's de-normalised character feature."""
         lib = self.lib
         sl = slice(lo, hi)
         Bp = hi - lo
+        _lib.check(lib.mocha_cvae_condition(_lib.ptr(self.cnt[sl]), _lib.ptr(self.prev_cha[sl]), _lib.ptr(self.m0),
+                                            _lib.ptr(self.s0), _lib.ptr(self.m1), _lib.ptr(self.s1),
+                                            _lib.ptr(self.cond[sl]), Bp, self.ntok, self.D, self._s()), "condition")
+        wp, wn = self._ws(ws)
+        _lib.check(lib.mocha_cvae_sample(C.byref(self.cvae.struct), _lib.ptr(self.cond[sl]), Bp, 2 * self.ntok,
+                                         None if self.deterministic else _lib.ptr(self.eps[sl]),
+                                         _lib.ptr(self.cvae_out[sl]), None, None, _lib.ptr(self.m1), _lib.ptr(self.s1),
+                                         _lib.ptr(self.prev_cha[sl]), self.prec, wp, wn, self._s()), "cvae_sample")
+
+    def _admission_part(self, lo: int, hi: int, ws):
+        """One lane of an admission-mode frame: every clip runs a steady-state frame, and the clips whose start byte is
+        set run their frame 0 inside the same launches (seeded prev_cha, masked post-process)."""
+        sl = slice(lo, hi)
+        self.encode(self.X[sl], self.tokens[sl], self.encoded[sl], self.cnt[sl], self.cnt_nm[sl], self.cnt_nm16[sl], ws)
+        side = None
+        if self.match_async:
+            k = next(i for i, pr in enumerate(self.parts) if pr[0] == lo)
+            side = self.match_streams[k]
+            side.wait_stream(torch.cuda.current_stream())
+            with torch.cuda.stream(side):
+                self._match(lo, hi, self.match_ws[k])
+        else:
+            self._match(lo, hi, ws)
+        self._cvae_step(lo, hi, ws)
+        if side is not None:
+            torch.cuda.current_stream().wait_stream(side)       # join: a started clip's decoder needs its match
+        # started clips: the matched DB row replaces the CVAE output (test_fullframework.py:298, :437)
+        _lib.check(self.lib.mocha_seed_rows(_lib.ptr(self.start[sl]), _lib.ptr(self.match_idx[sl]), 1,
+                                            _lib.ptr(self.cha_encoded), self.cha_encoded.shape[0], self.ntok * self.D,
+                                            _lib.ptr(self.prev_cha[sl]), hi - lo, self._s()), "seed_rows")
+        if self.with_cm_path:
+            torch.index_select(self.cha_encoded, 0, self.match_idx[sl, 0], out=self.cm_cha[sl])
+        self._decode(self.encoded[sl], self.prev_cha[sl], self.decoded[sl], self.Y[sl], ws)
+        self.post.step_packed(self.Y[sl], self.side[sl], self.contacts[sl], lo=lo, start=self.start[sl])
+        if self.with_cm_path:
+            self._decode(self.encoded[sl], self.cm_cha[sl], self.decoded[sl], self.cm_Y[sl], ws)
+            self.cm_post.step_packed(self.cm_Y[sl], self.side[sl], self.contacts[sl], lo=lo, start=self.start[sl])
+
+    def _frame_part(self, init: bool, lo: int, hi: int, ws):
+        """One lane: clips [lo, hi) from the input buffers to the FrameOut buffer, on the current stream."""
+        if self.admission:
+            self._admission_part(lo, hi, ws)
+            return
+        sl = slice(lo, hi)
         self.encode(self.X[sl], self.tokens[sl], self.encoded[sl], self.cnt[sl], self.cnt_nm[sl], self.cnt_nm16[sl], ws)
         side = None
         if self.match_async and not init and not self.with_cm_path:
@@ -204,14 +264,7 @@ class CharacterizationSession:
             # frame 0: the NN result seeds the autoregression (test_fullframework.py:298, :437)
             self.prev_cha[sl].copy_(self.cm_cha[sl])
         else:
-            _lib.check(lib.mocha_cvae_condition(_lib.ptr(self.cnt[sl]), _lib.ptr(self.prev_cha[sl]), _lib.ptr(self.m0),
-                                                _lib.ptr(self.s0), _lib.ptr(self.m1), _lib.ptr(self.s1),
-                                                _lib.ptr(self.cond[sl]), Bp, self.ntok, self.D, self._s()), "condition")
-            wp, wn = self._ws(ws)
-            _lib.check(lib.mocha_cvae_sample(C.byref(self.cvae.struct), _lib.ptr(self.cond[sl]), Bp, 2 * self.ntok,
-                                             None if self.deterministic else _lib.ptr(self.eps[sl]),
-                                             _lib.ptr(self.cvae_out[sl]), None, None, _lib.ptr(self.m1), _lib.ptr(self.s1),
-                                             _lib.ptr(self.prev_cha[sl]), self.prec, wp, wn, self._s()), "cvae_sample")
+            self._cvae_step(lo, hi, ws)
         self._decode(self.encoded[sl], self.prev_cha[sl], self.decoded[sl], self.Y[sl], ws)
         # the kernel reads the packed `side` rows in place (no slicing copies inside the captured frame)
         self.post.step_packed(self.Y[sl], self.side[sl], self.contacts[sl], lo=lo, init=init)
@@ -240,8 +293,9 @@ class CharacterizationSession:
             self.cm_post.started = True
 
     def capture(self):
-        """Capture the steady-state frame (i >= 1) into a CUDA graph. Call after the first frame."""
-        if self.frame == 0:
+        """Capture the steady-state frame (i >= 1) into a CUDA graph. Call after the first frame; in admission mode the
+        captured frame is the only frame body (starts are per slot, from the `start` row), so any time will do."""
+        if self.frame == 0 and not self.admission:
             raise _lib.MochaError("capture() needs the init frame to have run (state must exist)")
         state_backup = (self.prev_cha.clone(), self.post.state.clone(),
                         self.cm_post.state.clone() if self.cm_post else None)
@@ -262,18 +316,25 @@ class CharacterizationSession:
 
     # ---------------------------------------------------------------------------------------------
     def step_device(self):
-        """Advance one frame from the static device input buffers (X, side, contacts, eps)."""
-        init = self.frame == 0
+        """Advance one frame from the static device input buffers (X, side, contacts, eps; and start in admission
+        mode)."""
+        init = self.frame == 0 and not self.admission
         if self.graph is not None and not init:
             self.graph.replay()
         else:
             self._frame_body(init)
         self.frame += 1
 
-    def step_host(self, X, src_hips_vel, src_rvel, src_rang, contacts, eps=None):
+    def step_host(self, X, src_hips_vel, src_rvel, src_rang, contacts, eps=None, start=None):
         """End-to-end call with HOST (numpy) inputs: pinned staging -> H2D -> frame -> D2H.
+        start (admission mode only): uint8 [B], 1 = the slot starts a new clip on this frame; None = no slot starts.
         Returns the frame outputs as a dict of float64 numpy arrays [B, ...]."""
         B, T = self.B, self.T
+        if self.admission:
+            self.h_start.numpy()[...] = 0 if start is None else np.asarray(start, dtype=np.uint8)
+            self.start.copy_(self.h_start, non_blocking=True)
+        elif start is not None:
+            raise _lib.MochaError("a start row needs CharacterizationSession(admission=True)")
         self.h_X.numpy()[...] = X
         hs = self.h_side.numpy()
         hs[:, :T * 3] = np.asarray(src_hips_vel, dtype=np.float32).reshape(B, T * 3)
@@ -298,22 +359,20 @@ class CharacterizationSession:
     # ---------------------------------------------------------------------------------------------
     def pinned_inputs(self):
         """A set of pinned host tensors a caller fills for one frame (shapes of step_host's arguments,
-        with src_hips_vel/src_rvel/src_rang packed as `side` [B, T*3+6])."""
-        return {"X": torch.zeros(self.X.shape, dtype=torch.float32).pin_memory(),
-                "side": torch.zeros(self.side.shape, dtype=torch.float32).pin_memory(),
-                "contacts": torch.zeros(self.contacts.shape, dtype=torch.uint8).pin_memory(),
-                "eps": torch.zeros(self.eps.shape, dtype=torch.float32).pin_memory()}
+        with src_hips_vel/src_rvel/src_rang packed as `side` [B, T*3+6]; admission mode adds the uint8 [B] `start` row)."""
+        return {k: torch.zeros(getattr(self, k).shape, dtype=getattr(self, k).dtype).pin_memory()
+                for k in self._input_names}
 
     def _pipe_init(self):
         dev = self.dev
         self._copy_stream = torch.cuda.Stream(device=dev)
         self._slots = []
         for _ in range(2):
-            self._slots.append({
-                "X": torch.empty_like(self.X), "side": torch.empty_like(self.side),
-                "contacts": torch.empty_like(self.contacts), "eps": torch.empty_like(self.eps),
-                "h_out": torch.zeros(self.post.out.shape, dtype=torch.uint8).pin_memory(),
-                "h2d": torch.cuda.Event(), "consumed": torch.cuda.Event(), "done": torch.cuda.Event(), "used": False})
+            slot = {k: torch.empty_like(getattr(self, k)) for k in self._input_names}
+            slot.update({"h_out": torch.zeros(self.post.out.shape, dtype=torch.uint8).pin_memory(),
+                         "h2d": torch.cuda.Event(), "consumed": torch.cuda.Event(), "done": torch.cuda.Event(),
+                         "used": False})
+            self._slots.append(slot)
         self._ticket = 0
 
     def submit(self, pinned: dict) -> int:
@@ -327,11 +386,12 @@ class CharacterizationSession:
         if s["used"]:
             self._copy_stream.wait_event(s["consumed"])
         with torch.cuda.stream(self._copy_stream):
-            for k in ("X", "side", "contacts", "eps"):
+            for k in self._input_names:
                 s[k].copy_(pinned[k], non_blocking=True)
             s["h2d"].record(self._copy_stream)
         main.wait_event(s["h2d"])
-        self.X.copy_(s["X"]); self.side.copy_(s["side"]); self.contacts.copy_(s["contacts"]); self.eps.copy_(s["eps"])
+        for k in self._input_names:
+            getattr(self, k).copy_(s[k])
         s["consumed"].record(main)
         self.step_device()
         s["h_out"].copy_(self.post.out, non_blocking=True)
@@ -347,7 +407,8 @@ class CharacterizationSession:
         return self._decode_out(s["h_out"].numpy())
 
     def h2d_bytes(self):
-        return self.h_X.numel() * 4 + self.h_side.numel() * 4 + self.h_contacts.numel() + self.h_eps.numel() * 4
+        return (self.h_X.numel() * 4 + self.h_side.numel() * 4 + self.h_contacts.numel() + self.h_eps.numel() * 4
+                + (self.h_start.numel() if self.admission else 0))
 
     def d2h_bytes(self):
         return self.h_out.numel()
