@@ -433,6 +433,25 @@ int mocha_window_features(const float* d_grot, const float* d_gpos, const float*
                           int T, int J, const float* d_X_mean, const float* d_X_std, float* d_X, float* d_xrot,
                           float* d_xpos, mocha_stream_t stream);
 
+/* ---- source windows: every slot's pose window built on the device from a bank of source clips (DESIGN §5b) ----
+ * Bank: per-frame preprocess.process_frames arrays of many clips back to back, d_rot [n_frames,J,4], d_pos / d_vel /
+ * d_ang [n_frames,J,3] fp32 (d_rot 16 B aligned), d_bank_contacts uint8 [n_frames,2]; clip c is frames
+ * d_clip_first[c] .. + d_clip_frames[c] (int64 / int32 tables of n_clips entries; a frame count below T/4 + 1 marks an
+ * unused entry). d_parents [J], d_X_mean / d_X_std [J,15] as for mocha_window_features.
+ * Per slot b, each call: if d_start[b], d_slot_clip[b] = d_clip[b] and d_slot_cursor[b] = 0 (d_clip is read only there).
+ * The slot then serves window w = min(cursor, nwin - 1) of its clip, nwin = F - T/4 (preprocess.sliding_windows' count
+ * and edge padding), and the cursor becomes w + 1 (so it saturates at nwin: a finished clip repeats its last window).
+ * Outputs are what features.extract computes for that window, bit for bit: d_X[b] [T,J-1,15]; d_side row b (stride
+ * side_stride >= T*3+6 floats) = [velocity of joint 1 after ik, T*3 | root velocity 3 | root angular velocity 3] of the
+ * last frame's body frame; d_contacts[b] [2] = contacts of the last frame. A slot whose clip id is outside
+ * [0, n_clips), or names an unused entry, is idle (d_slot_clip[b] = -1): it writes zeros. One launch, graph-capturable. */
+int mocha_source_windows(const float* d_rot, const float* d_pos, const float* d_vel, const float* d_ang,
+                         const uint8_t* d_bank_contacts, long long n_frames, const int64_t* d_clip_first,
+                         const int32_t* d_clip_frames, int n_clips, const int32_t* d_parents, int T, int J,
+                         const float* d_X_mean, const float* d_X_std, const uint8_t* d_start, const int32_t* d_clip,
+                         int32_t* d_slot_clip, int32_t* d_slot_cursor, int B, float* d_X, float* d_side, int side_stride,
+                         uint8_t* d_contacts, mocha_stream_t stream);
+
 /* ---- element-wise quaternion algebra of motion/quat.py in the caller's precision ------------- */
 /* out[i] = op(a[i], b[i]) for i < n; dense [n, width] arrays, float32 (is_f64 == 0) or float64. Ops and widths
  * (a, b, out): 0 mul (4,4,4) quat.py:112 | 1 inv_mul :122 | 2 mul_inv :125 | 3 mul_vec (4,3,3) :128 |

@@ -45,6 +45,13 @@ template <typename T> __device__ __forceinline__ V3<T> qrot(Q4<T> q, V3<T> x) {
   const V3<T> t = (T)2 * cross(qvec(q), x);
   return x + q.w * t + cross(qvec(q), t);
 }
+// quat.mul_vec / quat.inv_mul_vec (motion/quat.py:128-133): mocha_quat_op's ops 3 and 4, and the source windows' root
+// velocities
+template <typename T> __device__ __forceinline__ V3<T> q_mul_vec(const T* q4p, const T* x, bool inv) {
+  Q4<T> q = q4<T>(q4p[0], q4p[1], q4p[2], q4p[3]);
+  if (inv) q = qinv(q);
+  return qrot(q, v3<T>(x[0], x[1], x[2]));
+}
 template <typename T> __device__ __forceinline__ Q4<T> qnormalize(Q4<T> q) {
   const T d = sqrt(q.w * q.w + q.x * q.x + q.y * q.y + q.z * q.z) + (T)1e-8;
   return q4<T>(q.w / d, q.x / d, q.y / d, q.z / d);
@@ -151,6 +158,28 @@ __device__ __forceinline__ void warp_copy_in(T* dst, const T* __restrict__ src, 
 template <typename T>
 __device__ __forceinline__ void warp_copy_out(T* __restrict__ dst, const T* src, int n, int lane) {
   for (int i = lane; i < n; i += 32) dst[i] = src[i];
+}
+
+// Joint steps shared by the batch kernels and source_windows_kernel, which must reproduce their results bit for bit.
+// quat.fk / quat.fk_vel (motion/quat.py:166-204): global transform of a joint from its parent's (pr, pp); rp is the
+// parent-rotated offset the velocity step needs.
+__device__ __forceinline__ void fk_joint_pose(Q4<float> pr, V3<float> pp, Q4<float> lr, V3<float> lp, V3<float>& rp,
+                                              V3<float>& gp, Q4<float>& gr) {
+  rp = qrot(pr, lp);
+  gp = rp + pp;
+  gr = qmul(pr, lr);
+}
+__device__ __forceinline__ void fk_joint_vel(Q4<float> pr, V3<float> rp, V3<float> pv, V3<float> pa, V3<float> lv,
+                                             V3<float> la, V3<float>& gv, V3<float>& ga) {
+  gv = qrot(pr, lv) + cross(pa, rp) + pv;
+  ga = qrot(pr, la) + pa;
+}
+// quat.ik (motion/quat.py:175-187) of a non-root joint
+template <typename T>
+__device__ __forceinline__ void ik_joint(Q4<T> pr, V3<T> pp, Q4<T> gr, V3<T> gp, Q4<T>& lr, V3<T>& lp) {
+  const Q4<T> pinv = qinv(pr);
+  lr = qmul(pinv, gr);
+  lp = qrot(pinv, gp - pp);
 }
 
 // depth of joint `lane` in the hierarchy (parents[i] < i)
@@ -321,9 +350,9 @@ fk_rows_kernel(const float* __restrict__ lrot, const float* __restrict__ lpos, c
         const Q4<float> pr = q4<float>(pr4.x, pr4.y, pr4.z, pr4.w);
         const V3<float> lp = v3<float>(x[3 * j], x[3 * j + 1], x[3 * j + 2]);
         const V3<float> pp = v3<float>(x[3 * p], x[3 * p + 1], x[3 * p + 2]);
-        const V3<float> rp = qrot(pr, lp);
-        const V3<float> gp = rp + pp;
-        const Q4<float> gr = qmul(pr, lr);
+        V3<float> rp, gp;
+        Q4<float> gr;
+        fk_joint_pose(pr, pp, lr, lp, rp, gp, gr);
         x[3 * j] = gp.x; x[3 * j + 1] = gp.y; x[3 * j + 2] = gp.z;
         r[j] = make_float4(gr.w, gr.x, gr.y, gr.z);
         if (WITH_VEL) {
@@ -331,8 +360,8 @@ fk_rows_kernel(const float* __restrict__ lrot, const float* __restrict__ lpos, c
           const V3<float> la = v3<float>(a[3 * j], a[3 * j + 1], a[3 * j + 2]);
           const V3<float> pv = v3<float>(v[3 * p], v[3 * p + 1], v[3 * p + 2]);
           const V3<float> pa = v3<float>(a[3 * p], a[3 * p + 1], a[3 * p + 2]);
-          const V3<float> gv = qrot(pr, lv) + cross(pa, rp) + pv;
-          const V3<float> ga = qrot(pr, la) + pa;
+          V3<float> gv, ga;
+          fk_joint_vel(pr, rp, pv, pa, lv, la, gv, ga);
           v[3 * j] = gv.x; v[3 * j + 1] = gv.y; v[3 * j + 2] = gv.z;
           a[3 * j] = ga.x; a[3 * j + 1] = ga.y; a[3 * j + 2] = ga.z;
         }
@@ -390,10 +419,11 @@ ik_kernel(const T* __restrict__ grot, const T* __restrict__ gpos, const int32_t*
         s.pos[j][0] = gp.x; s.pos[j][1] = gp.y; s.pos[j][2] = gp.z;
       } else {
         const int p = par[j];
-        const Q4<T> pinv = qinv(q4<T>(s.grot[p][0], s.grot[p][1], s.grot[p][2], s.grot[p][3]));
+        const Q4<T> pr = q4<T>(s.grot[p][0], s.grot[p][1], s.grot[p][2], s.grot[p][3]);
         const V3<T> pp = v3<T>(s.gpos[p][0], s.gpos[p][1], s.gpos[p][2]);
-        const Q4<T> lr = qmul(pinv, gr);
-        const V3<T> lp = qrot(pinv, gp - pp);
+        Q4<T> lr;
+        V3<T> lp;
+        ik_joint(pr, pp, gr, gp, lr, lp);
         s.rot[j][0] = lr.w; s.rot[j][1] = lr.x; s.rot[j][2] = lr.y; s.rot[j][3] = lr.z;
         s.pos[j][0] = lp.x; s.pos[j][1] = lp.y; s.pos[j][2] = lp.z;
       }
@@ -1379,9 +1409,7 @@ __global__ void quat_op_kernel(int op, const T* __restrict__ a, const T* __restr
       break;
     }
     case QOP_MUL_VEC: case QOP_INV_MUL_VEC: {
-      Q4<T> q = q4<T>(pa[0], pa[1], pa[2], pa[3]);
-      if (op == QOP_INV_MUL_VEC) q = qinv(q);
-      const V3<T> r = qrot(q, v3<T>(pb[0], pb[1], pb[2]));
+      const V3<T> r = q_mul_vec(pa, pb, op == QOP_INV_MUL_VEC);
       po[0] = r.x; po[1] = r.y; po[2] = r.z;
       break;
     }
@@ -1559,6 +1587,33 @@ extern "C" int mocha_fk_chain(int is_f64, const void* start_pos, const void* sta
 // rotations / positions the following quat.ik (:160) needs.
 // ------------------------------------------------------------------------------------------------
 namespace {
+// per-joint body of the re-rooting, shared with source_windows_kernel: a joint's global transform relative to the root
+// (r0i = inverse root rotation, p0 = root position)
+__device__ __forceinline__ void reroot_joint(Q4<float> r0i, V3<float> p0, Q4<float> gr, V3<float> gp, V3<float> gv,
+                                             V3<float> ga, V3<float>& xp, Q4<float>& xr, V3<float>& xv, V3<float>& xa) {
+  xp = qrot(r0i, gp - p0);
+  xr = qmul(r0i, gr);
+  xv = qrot(r0i, gv);
+  xa = qrot(r0i, ga);
+}
+// the 15 channels of a joint row: position, first two columns of the rotation matrix (6-D encoding), velocity, angular
+// velocity
+__device__ __forceinline__ void feature_row(V3<float> xp, Q4<float> xr, V3<float> xv, V3<float> xa, float (&f)[15]) {
+  const float qw = xr.w, qx = xr.x, qy = xr.y, qz = xr.z;
+  const float x2 = qx + qx, y2 = qy + qy, z2 = qz + qz;
+  const float xx = qx * x2, yy = qy * y2, wx = qw * x2;
+  const float xy = qx * y2, yz = qy * z2, wy = qw * y2;
+  const float xz = qx * z2, zz = qz * z2, wz = qw * z2;
+  f[0] = xp.x; f[1] = xp.y; f[2] = xp.z;
+  f[3] = 1.0f - (yy + zz); f[4] = xy - wz; f[5] = xy + wz; f[6] = 1.0f - (xx + zz); f[7] = xz - wy; f[8] = yz + wx;
+  f[9] = xv.x; f[10] = xv.y; f[11] = xv.z; f[12] = xa.x; f[13] = xa.y; f[14] = xa.z;
+}
+__device__ __forceinline__ void store_normalised_row(float* __restrict__ o, const float (&f)[15], const float* __restrict__ mu,
+                                                     const float* __restrict__ sd) {
+#pragma unroll
+  for (int c = 0; c < 15; ++c) o[c] = (f[c] - mu[c]) / sd[c];
+}
+
 __global__ void __launch_bounds__(256)
 window_reroot_kernel(const float* __restrict__ grot, const float* __restrict__ gpos, const float* __restrict__ gvel,
                      const float* __restrict__ gang, long long W, int T, int J, const float* __restrict__ X_mean,
@@ -1582,32 +1637,222 @@ window_reroot_kernel(const float* __restrict__ grot, const float* __restrict__ g
   const V3<float> gp = v3<float>(gpos[src * 3], gpos[src * 3 + 1], gpos[src * 3 + 2]);
   const V3<float> gv = v3<float>(gvel[src * 3], gvel[src * 3 + 1], gvel[src * 3 + 2]);
   const V3<float> ga = v3<float>(gang[src * 3], gang[src * 3 + 1], gang[src * 3 + 2]);
-  const V3<float> xp = qrot(r0i, gp - p0);
-  const Q4<float> xr = qmul(r0i, gr);
-  const V3<float> xv = qrot(r0i, gv);
-  const V3<float> xa = qrot(r0i, ga);
+  V3<float> xp, xv, xa;
+  Q4<float> xr;
+  reroot_joint(r0i, p0, gr, gp, gv, ga, xp, xr, xv, xa);
   if (xrot) { xrot[i * 4] = xr.w; xrot[i * 4 + 1] = xr.x; xrot[i * 4 + 2] = xr.y; xrot[i * 4 + 3] = xr.z; }
   if (xpos) { xpos[i * 3] = xp.x; xpos[i * 3 + 1] = xp.y; xpos[i * 3 + 2] = xp.z; }
   if (j == 0 && !per_frame_root) return;                  // X drops the simulation root (:186)
-  const float qw = xr.w, qx = xr.x, qy = xr.y, qz = xr.z;
-  const float x2 = qx + qx, y2 = qy + qy, z2 = qz + qz;
-  const float xx = qx * x2, yy = qy * y2, wx = qw * x2;
-  const float xy = qx * y2, yz = qy * z2, wy = qw * y2;
-  const float xz = qx * z2, zz = qz * z2, wz = qw * z2;
-  const float f[15] = {xp.x, xp.y, xp.z,
-                       1.0f - (yy + zz), xy - wz, xy + wz, 1.0f - (xx + zz), xz - wy, yz + wx,
-                       xv.x, xv.y, xv.z, xa.x, xa.y, xa.z};
+  float f[15];
+  feature_row(xp, xr, xv, xa, f);
   if (per_frame_root) {                                   // all J joints, not normalised (trainer.py:364-372)
     float* o = X + i * 15;
 #pragma unroll
     for (int c = 0; c < 15; ++c) o[c] = f[c];
     return;
   }
-  float* o = X + (wt * (J - 1) + (j - 1)) * 15;
-  const float* mu = X_mean + j * 15;
-  const float* sd = X_std + j * 15;
-#pragma unroll
-  for (int c = 0; c < 15; ++c) o[c] = (f[c] - mu[c]) / sd[c];
+  store_normalised_row(X + (wt * (J - 1) + (j - 1)) * 15, f, X_mean + j * 15, X_std + j * 15);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Source windows (DESIGN §5b): every slot's pose window built from a bank of preprocessed per-frame clip arrays, with
+// the results of features.extract (fk_vel -> re-rooting -> ik -> central differences, quat_op inv_mul_vec) bit for bit.
+// One CTA per slot. Window frames are staged SW_CHUNK at a time in shared memory (local transforms, edge-padded the way
+// preprocess.sliding_windows pads: pose of the edge frame, zero velocities), the next chunk's loads in flight while the
+// current one is processed; the hierarchy is walked level by level with one thread per (frame, joint), in place, through
+// the same joint steps as fk_rows_kernel. Each joint row is then
+// re-rooted on the last frame's root, encoded and normalised into X; the hips' local positions (ik of joint 1) collect
+// in shared memory for the central difference once all frames are done.
+// ------------------------------------------------------------------------------------------------
+constexpr int SW_CHUNK = 15;
+constexpr int SW_THREADS = SW_CHUNK * MAXJ;            // one (frame, joint) item of a chunk per thread
+
+__host__ __device__ inline size_t source_windows_smem(int T, int J) {
+  return (size_t)SW_CHUNK * J * (4 + 3 + 3 + 3) * sizeof(float) + (size_t)T * 3 * sizeof(float);
+}
+
+// sliding_windows' index map: clip frame of window w's frame t (F frames in the clip), and whether t is padding
+__device__ __forceinline__ int window_frame(int t, int w, int F, int T, bool& pad) {
+  const int L = min(T, F - w), sh = T - L, left = (sh + 1) / 2;
+  const int k = t - left;
+  pad = k < 0 || k >= L;
+  return w + min(max(k, 0), L - 1);
+}
+
+// torch's (0.5 * (x[t+1] - x[t]) * 60.0 + 0.5 * (x[t] - x[t-1]) * 60.0), every op rounded on its own (no FMA)
+__device__ __forceinline__ float central_diff(float xm, float x0, float xp) {
+  return __fadd_rn(__fmul_rn(__fmul_rn(0.5f, __fsub_rn(xp, x0)), 60.0f), __fmul_rn(__fmul_rn(0.5f, __fsub_rn(x0, xm)), 60.0f));
+}
+
+__global__ void __launch_bounds__(SW_THREADS)
+source_windows_kernel(const float* __restrict__ brot, const float* __restrict__ bpos, const float* __restrict__ bvel,
+                      const float* __restrict__ bang, const uint8_t* __restrict__ bcontacts, long long n_frames,
+                      const long long* __restrict__ clip_first, const int32_t* __restrict__ clip_frames, int n_clips,
+                      const int32_t* __restrict__ parents, int T, int J, const float* __restrict__ X_mean,
+                      const float* __restrict__ X_std, const uint8_t* __restrict__ start, const int32_t* __restrict__ clip,
+                      int32_t* __restrict__ slot_clip, int32_t* __restrict__ slot_cursor, float* __restrict__ X,
+                      float* __restrict__ side, int side_stride, uint8_t* __restrict__ contacts) {
+  pdl_trigger();
+  extern __shared__ __align__(16) float sw_sm[];
+  __shared__ int32_t par[MAXJ];
+  __shared__ int32_t depth[MAXJ];
+  __shared__ int s_maxd, s_w, s_F;
+  __shared__ long long s_first;
+  const int b = blockIdx.x, tid = threadIdx.x;
+  const int V = J - 1;
+  float* out_X = X + (long long)b * T * V * 15;
+  float* out_side = side + (long long)b * side_stride;
+  pdl_wait();
+  if (tid < J) par[tid] = parents[tid];
+  if (tid == 0) {
+    int c = slot_clip[b], cur = slot_cursor[b];
+    if (start[b]) { c = clip[b]; cur = 0; }
+    int w = -1, F = 0;
+    long long first = 0;
+    if (c >= 0 && c < n_clips) {
+      F = clip_frames[c];
+      first = clip_first[c];
+      const int nwin = F - T / 4;                        // sliding_windows' count: range(0, F - T // 4)
+      if (nwin >= 1 && first >= 0 && first + F <= n_frames) {
+        w = min(cur, nwin - 1);
+        cur = w + 1;                                     // saturates at nwin: a finished clip repeats its last window
+      }
+    }
+    if (w < 0) { c = -1; cur = 0; }                      // idle: never started, bad id or empty table entry
+    if (start[b] || c >= 0) { slot_clip[b] = c; slot_cursor[b] = cur; }
+    s_w = w; s_F = F; s_first = first; s_maxd = 0;
+  }
+  __syncthreads();
+  const int w = s_w;
+  if (w < 0) {                                           // idle slot: finite (zero) inputs
+    for (int i = tid; i < T * V * 15; i += blockDim.x) out_X[i] = 0.0f;
+    for (int i = tid; i < T * 3 + 6; i += blockDim.x) out_side[i] = 0.0f;
+    if (tid < 2) contacts[b * 2 + tid] = 0;
+    return;
+  }
+  if (tid < J) {
+    int d = 0;
+    for (int p = par[tid]; p >= 0 && p < J && d < J; p = par[p]) ++d;
+    depth[tid] = d;
+    atomicMax(&s_maxd, d);
+  }
+  const int F = s_F;
+  const long long first = s_first;
+  float* rot = sw_sm;                                    // [SW_CHUNK][J][4]: local, then global transforms
+  float* pos = rot + SW_CHUNK * J * 4;                   // [SW_CHUNK][J][3]
+  float* vel = pos + SW_CHUNK * J * 3;
+  float* ang = vel + SW_CHUNK * J * 3;
+  float* hips = ang + SW_CHUNK * J * 3;                  // [T][3]: ik local position of joint 1
+  // the window's last frame: its root (re-rooting), root velocities and contacts
+  bool pad_last;
+  const long long fl = first + window_frame(T - 1, w, F, T, pad_last);
+  const Q4<float> r0 = q4<float>(brot[fl * J * 4], brot[fl * J * 4 + 1], brot[fl * J * 4 + 2], brot[fl * J * 4 + 3]);
+  const V3<float> p0 = v3<float>(bpos[fl * J * 3], bpos[fl * J * 3 + 1], bpos[fl * J * 3 + 2]);
+  const Q4<float> r0i = qinv(r0);
+  const V3<float> zero3 = v3<float>(0.0f, 0.0f, 0.0f);
+  if (tid == 0) {
+    const float zeros[3] = {0.0f, 0.0f, 0.0f};           // padded frames have zero velocities
+    const V3<float> rv = q_mul_vec(brot + fl * J * 4, pad_last ? zeros : bvel + fl * J * 3, true);
+    const V3<float> ra = q_mul_vec(brot + fl * J * 4, pad_last ? zeros : bang + fl * J * 3, true);
+    float* o = out_side + T * 3;
+    o[0] = rv.x; o[1] = rv.y; o[2] = rv.z; o[3] = ra.x; o[4] = ra.y; o[5] = ra.z;
+    contacts[b * 2] = bcontacts[fl * 2];
+    contacts[b * 2 + 1] = bcontacts[fl * 2 + 1];
+  }
+  __syncthreads();
+  const int maxd = s_maxd;
+  // this thread's item of a chunk: frame t0 + tid / J, joint tid % J; its local transform is loaded one chunk ahead
+  const int jt = tid % J, ft = tid / J;
+  float4 nr = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+  float np_[3], nv[3], na[3];
+  auto fetch = [&](int t0) {
+    if (ft < SW_CHUNK && t0 + ft < T) {
+      bool pad;
+      const long long f = (first + window_frame(t0 + ft, w, F, T, pad)) * J + jt;
+      nr = make_float4(brot[f * 4], brot[f * 4 + 1], brot[f * 4 + 2], brot[f * 4 + 3]);
+      for (int c = 0; c < 3; ++c) {
+        np_[c] = bpos[f * 3 + c];
+        nv[c] = pad ? 0.0f : bvel[f * 3 + c];
+        na[c] = pad ? 0.0f : bang[f * 3 + c];
+      }
+    }
+  };
+  fetch(0);
+  for (int t0 = 0; t0 < T; t0 += SW_CHUNK) {
+    const int n = min(SW_CHUNK, T - t0) * J;
+    if (tid < n) {                                       // stage the local transforms of the chunk
+      reinterpret_cast<float4*>(rot)[tid] = nr;
+      for (int c = 0; c < 3; ++c) { pos[tid * 3 + c] = np_[c]; vel[tid * 3 + c] = nv[c]; ang[tid * 3 + c] = na[c]; }
+    }
+    __syncthreads();
+    fetch(t0 + SW_CHUNK);
+    for (int lvl = 1; lvl <= maxd; ++lvl) {              // quat.fk_vel, one hierarchy level at a time
+      for (int i = tid; i < n; i += blockDim.x) {
+        const int j = i % J;
+        if (depth[j] != lvl) continue;
+        const int q = i - j + par[j];                    // the parent joint of the same frame
+        const float4 lr4 = reinterpret_cast<const float4*>(rot)[i], pr4 = reinterpret_cast<const float4*>(rot)[q];
+        const Q4<float> pr = q4<float>(pr4.x, pr4.y, pr4.z, pr4.w);
+        V3<float> rp, gp, gv, ga;
+        Q4<float> gr;
+        fk_joint_pose(pr, v3<float>(pos[q * 3], pos[q * 3 + 1], pos[q * 3 + 2]), q4<float>(lr4.x, lr4.y, lr4.z, lr4.w),
+                      v3<float>(pos[i * 3], pos[i * 3 + 1], pos[i * 3 + 2]), rp, gp, gr);
+        fk_joint_vel(pr, rp, v3<float>(vel[q * 3], vel[q * 3 + 1], vel[q * 3 + 2]),
+                     v3<float>(ang[q * 3], ang[q * 3 + 1], ang[q * 3 + 2]), v3<float>(vel[i * 3], vel[i * 3 + 1], vel[i * 3 + 2]),
+                     v3<float>(ang[i * 3], ang[i * 3 + 1], ang[i * 3 + 2]), gv, ga);
+        reinterpret_cast<float4*>(rot)[i] = make_float4(gr.w, gr.x, gr.y, gr.z);
+        pos[i * 3] = gp.x; pos[i * 3 + 1] = gp.y; pos[i * 3 + 2] = gp.z;
+        vel[i * 3] = gv.x; vel[i * 3 + 1] = gv.y; vel[i * 3 + 2] = gv.z;
+        ang[i * 3] = ga.x; ang[i * 3 + 1] = ga.y; ang[i * 3 + 2] = ga.z;
+      }
+      __syncthreads();
+    }
+    for (int i = tid; i < n; i += blockDim.x) {          // re-root, encode, normalise; ik of the hips
+      const int j = i % J, t = t0 + i / J;
+      if (j == 0) continue;                              // X drops the simulation root
+      const float4 g4 = reinterpret_cast<const float4*>(rot)[i];
+      V3<float> xp, xv, xa;
+      Q4<float> xr;
+      reroot_joint(r0i, p0, q4<float>(g4.x, g4.y, g4.z, g4.w), v3<float>(pos[i * 3], pos[i * 3 + 1], pos[i * 3 + 2]),
+                   v3<float>(vel[i * 3], vel[i * 3 + 1], vel[i * 3 + 2]), v3<float>(ang[i * 3], ang[i * 3 + 1], ang[i * 3 + 2]),
+                   xp, xr, xv, xa);
+      float fr[15];
+      feature_row(xp, xr, xv, xa, fr);
+      store_normalised_row(out_X + ((long long)t * V + (j - 1)) * 15, fr, X_mean + j * 15, X_std + j * 15);
+      if (j != 1) continue;
+      V3<float> lp = xp;                                 // a root joint's local transform is its global one
+      const int pj = par[1];
+      if (pj >= 0) {
+        // the parent's re-rooted transform; every frame's joint 0 row is the last frame's root
+        const int q = i - 1 + pj;
+        const float4 q4v = reinterpret_cast<const float4*>(rot)[q];
+        const Q4<float> qg = pj == 0 ? r0 : q4<float>(q4v.x, q4v.y, q4v.z, q4v.w);
+        const V3<float> qp = pj == 0 ? p0 : v3<float>(pos[q * 3], pos[q * 3 + 1], pos[q * 3 + 2]);
+        V3<float> pxp, pxv, pxa;
+        Q4<float> pxr, lr;
+        reroot_joint(r0i, p0, qg, qp, zero3, zero3, pxp, pxr, pxv, pxa);
+        ik_joint(pxr, pxp, xr, xp, lr, lp);
+      }
+      hips[t * 3] = lp.x; hips[t * 3 + 1] = lp.y; hips[t * 3 + 2] = lp.z;
+    }
+    __syncthreads();
+  }
+  // hips velocity: features._central_diff_time, linear extrapolation at both ends
+  for (int i = tid; i < T * 3; i += blockDim.x) {
+    const int t = i / 3, c = i % 3;
+    const float* x = hips + c;
+    float v;
+    if (t == 0) {
+      v = __fsub_rn(central_diff(x[0], x[3], x[6]), __fsub_rn(central_diff(x[6], x[9], x[12]), central_diff(x[3], x[6], x[9])));
+    } else if (t == T - 1) {
+      const float a = central_diff(x[(T - 3) * 3], x[(T - 2) * 3], x[(T - 1) * 3]);
+      const float bb = central_diff(x[(T - 4) * 3], x[(T - 3) * 3], x[(T - 2) * 3]);
+      v = __fadd_rn(a, __fsub_rn(a, bb));
+    } else {
+      v = central_diff(x[(t - 1) * 3], x[t * 3], x[(t + 1) * 3]);
+    }
+    out_side[i] = v;
+  }
 }
 }  // namespace
 
@@ -1624,5 +1869,34 @@ extern "C" int mocha_window_features(const float* grot, const float* gpos, const
            T, J, X_mean, X_std, X, xrot, xpos, per_frame);
   count_launch();
   MOCHA_LAUNCH_CHECK("window_reroot_kernel");
+  return MOCHA_OK;
+}
+
+extern "C" int mocha_source_windows(const float* rot, const float* pos, const float* vel, const float* ang,
+                                    const uint8_t* bank_contacts, long long n_frames, const int64_t* clip_first,
+                                    const int32_t* clip_frames, int n_clips, const int32_t* parents, int T, int J,
+                                    const float* X_mean, const float* X_std, const uint8_t* start, const int32_t* clip,
+                                    int32_t* slot_clip, int32_t* slot_cursor, int B, float* X, float* side, int side_stride,
+                                    uint8_t* contacts, mocha_stream_t stream) {
+  MOCHA_CHECK_ARG(rot && pos && vel && ang && bank_contacts && clip_first && clip_frames && parents && X_mean && X_std,
+                  "mocha_source_windows: null bank argument");
+  MOCHA_CHECK_ARG(start && clip && slot_clip && slot_cursor && X && side && contacts, "mocha_source_windows: null slot argument");
+  MOCHA_CHECK_ARG(B > 0 && n_frames > 0 && n_clips > 0, "mocha_source_windows: bad sizes B=%d n_frames=%lld n_clips=%d", B,
+                  n_frames, n_clips);
+  MOCHA_CHECK_ARG(J >= 2 && J <= MAXJ && T >= 5 && T <= 1024, "mocha_source_windows: need 2 <= J <= %d and 5 <= T <= 1024, "
+                  "got J=%d T=%d", MAXJ, J, T);
+  MOCHA_CHECK_ARG(side_stride >= T * 3 + 6, "mocha_source_windows: side rows need T*3+6 floats, stride %d", side_stride);
+  MOCHA_CHECK_ARG((reinterpret_cast<uintptr_t>(rot) & 15) == 0, "mocha_source_windows: rotations not 16 B aligned");
+  const size_t smem = source_windows_smem(T, J);
+  static size_t configured = 0;
+  if (smem > 48 * 1024 && smem > configured) {
+    MOCHA_CUDA(cudaFuncSetAttribute(source_windows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    configured = smem;
+  }
+  launch_k(source_windows_kernel, B, SW_THREADS, smem, (cudaStream_t)stream, rot, pos, vel, ang, bank_contacts, n_frames,
+           reinterpret_cast<const long long*>(clip_first), clip_frames, n_clips, parents, T, J, X_mean, X_std, start, clip,
+           slot_clip, slot_cursor, X, side, side_stride, contacts);
+  count_launch();
+  MOCHA_LAUNCH_CHECK("source_windows_kernel");
   return MOCHA_OK;
 }

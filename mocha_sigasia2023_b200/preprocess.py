@@ -117,9 +117,10 @@ def sliding_windows(x, window, step, zero_pad=False):
     return np.stack(out)
 
 
-def process_clip(clip: dict, window: int = 60, window_step: int = 1) -> dict:
-    """Returns float32 window arrays pos/vel/rot/ang [nwin, window, 25, 3|4] and uint8 contacts
-    [nwin, window, 2], exactly what the driver builds at test_fullframework.py:126-139."""
+def process_frames(clip: dict) -> dict:
+    """The per-frame half of process_clip: float32 pos/vel/rot/ang [F, 25, 3|4], uint8 contacts [F, 2], the bone
+    parents and names. Its arrays are 62x smaller than the windows of a 240-frame clip; SourceBank keeps them on the
+    device and builds the windows there."""
     names = list(clip["names"])
     parents = np.asarray(clip["parents"])
     positions = np.asarray(clip["positions"], dtype=np.float64) * 0.01            # cm -> m (:91)
@@ -154,12 +155,25 @@ def process_clip(clip: dict, window: int = 60, window_step: int = 1) -> dict:
     contacts = np.sqrt((gvel[:, toes] ** 2).sum(-1)) < 0.5                        # :162-171
     for ci in range(contacts.shape[1]):
         contacts[:, ci] = ndimage.median_filter(contacts[:, ci], size=6, mode="nearest")
+    return {"pos": positions.astype(np.float32), "vel": velocities.astype(np.float32), "rot": rotations.astype(np.float32),
+            "ang": angular.astype(np.float32), "contacts": contacts.astype(np.uint8), "parents": bone_parents,
+            "names": bone_names}
+
+
+def frame_windows(frames: dict, window: int = 60, window_step: int = 1) -> dict:
+    """process_frames' arrays cut into process_clip's windows (the float32 cast commutes with the windowing)."""
     return {
-        "pos": sliding_windows(positions, window, window_step).astype(np.float32),
-        "vel": sliding_windows(velocities, window, window_step, zero_pad=True).astype(np.float32),
-        "rot": sliding_windows(rotations, window, window_step).astype(np.float32),
-        "ang": sliding_windows(angular, window, window_step, zero_pad=True).astype(np.float32),
-        "contacts": sliding_windows(contacts, window, window_step).astype(np.uint8),
-        "parents": bone_parents,
-        "names": bone_names,
+        "pos": sliding_windows(frames["pos"], window, window_step),
+        "vel": sliding_windows(frames["vel"], window, window_step, zero_pad=True),
+        "rot": sliding_windows(frames["rot"], window, window_step),
+        "ang": sliding_windows(frames["ang"], window, window_step, zero_pad=True),
+        "contacts": sliding_windows(frames["contacts"], window, window_step),
+        "parents": frames["parents"],
+        "names": frames["names"],
     }
+
+
+def process_clip(clip: dict, window: int = 60, window_step: int = 1) -> dict:
+    """Returns float32 window arrays pos/vel/rot/ang [nwin, window, 25, 3|4] and uint8 contacts
+    [nwin, window, 2], exactly what the driver builds at test_fullframework.py:126-139."""
+    return frame_windows(process_frames(clip), window, window_step)

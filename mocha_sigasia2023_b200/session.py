@@ -36,7 +36,7 @@ class NormStats:
 class CharacterizationSession:
     def __init__(self, gen_sd, cvae_sd, cfg, stats: NormStats, cha_encoded, cha_cnt_nm, batch: int,
                  device="cuda", precision="fp32", with_cm_path=False, match_tensor_cores=None, post_params=None,
-                 lanes: int = 1, admission: bool = False):
+                 lanes: int = 1, admission: bool = False, source_bank=None):
         """gen_sd / cvae_sd: reference-layout state dicts. cha_encoded [N,90,256] and cha_cnt_nm [N,23040]
         (already (cnt-mean)/std scaled): the target character's feature DB, CUDA or CPU tensors.
 
@@ -48,7 +48,16 @@ class CharacterizationSession:
         from frame to frame (prev_cha, the post-process states) is per slot and rewritten by a start, so a reused slot
         behaves exactly like a fresh one. A slot whose clip has ended keeps computing on whatever finite inputs the
         caller leaves in its rows; its outputs are meaningless until it is started again, and nothing of an idle or
-        previous occupant reaches a started clip. Slots that never started compute on the zero-initialised buffers."""
+        previous occupant reaches a started clip. Slots that never started compute on the zero-initialised buffers.
+
+        source_bank (a SourceBank; needs admission=True): every slot's X, side and contacts are built on the device from
+        the bank by mocha_source_windows, the first launch of the frame. The per-frame inputs become the `start` row,
+        an int32 [B] `clip` row (the bank's clip id of each starting slot, read only where start is set) and eps
+        (step_bank(), or pinned_inputs() for submit / collect). A started slot serves its clip's windows one per frame
+        and repeats the last one once the clip has ended; an idle slot (never started, or started with an id the bank
+        does not hold) gets zero inputs."""
+        if source_bank is not None and not admission:
+            raise _lib.MochaError("source_bank needs CharacterizationSession(admission=True)")
         self.lib = _lib.load()
         _lib.check(self.lib.mocha_check_device(), "mocha_check_device")
         dev = torch.device(device)
@@ -98,6 +107,15 @@ class CharacterizationSession:
         if self.admission:
             self.start = torch.zeros((B,), dtype=torch.uint8, device=dev)     # 1 = the slot starts a new clip this frame
         self._input_names = ("X", "side", "contacts", "eps") + (("start",) if self.admission else ())
+        self.bank = source_bank
+        if source_bank is not None:
+            if source_bank.dev != dev or source_bank.T != d.T or source_bank.J != d.V + 1:
+                raise _lib.MochaError(f"source_bank holds windows of {source_bank.T} frames x {source_bank.J} joints on "
+                                      f"{source_bank.dev}; this session needs {d.T} x {d.V + 1} on {dev}")
+            self.clip = torch.zeros((B,), dtype=torch.int32, device=dev)       # bank clip id of each starting slot
+            self.slot_clip = torch.full((B,), -1, dtype=torch.int32, device=dev)
+            self.slot_cursor = torch.zeros((B,), dtype=torch.int32, device=dev)
+            self._input_names = ("start", "clip", "eps")
         # intermediates
         self.tokens = torch.empty((B, n, D), **f32)
         self.encoded = torch.empty((B, n, D), **f32)
@@ -150,6 +168,8 @@ class CharacterizationSession:
         self.h_eps = torch.zeros((B, D), dtype=torch.float32).pin_memory()
         if self.admission:
             self.h_start = torch.zeros((B,), dtype=torch.uint8).pin_memory()
+        if self.bank is not None:
+            self.h_clip = torch.zeros((B,), dtype=torch.int32).pin_memory()
         self.h_out = torch.zeros(self.post.out.shape, dtype=torch.uint8).pin_memory()
         self.side = torch.zeros((B, d.T * 3 + 3 + 3), **f32)
 
@@ -217,6 +237,9 @@ class CharacterizationSession:
         """One lane of an admission-mode frame: every clip runs a steady-state frame, and the clips whose start byte is
         set run their frame 0 inside the same launches (seeded prev_cha, masked post-process)."""
         sl = slice(lo, hi)
+        if self.bank is not None:
+            self.bank.windows(self.start[sl], self.clip[sl], self.slot_clip[sl], self.slot_cursor[sl], self.X[sl],
+                              self.side[sl], self.contacts[sl])
         self.encode(self.X[sl], self.tokens[sl], self.encoded[sl], self.cnt[sl], self.cnt_nm[sl], self.cnt_nm16[sl], ws)
         side = None
         if self.match_async:
@@ -299,6 +322,7 @@ class CharacterizationSession:
             raise _lib.MochaError("capture() needs the init frame to have run (state must exist)")
         state_backup = (self.prev_cha.clone(), self.post.state.clone(),
                         self.cm_post.state.clone() if self.cm_post else None)
+        slots_backup = (self.slot_clip.clone(), self.slot_cursor.clone()) if self.bank is not None else None
         s = torch.cuda.Stream()
         s.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(s):
@@ -312,6 +336,9 @@ class CharacterizationSession:
         self.post.state.copy_(state_backup[1])
         if self.cm_post:
             self.cm_post.state.copy_(state_backup[2])
+        if slots_backup is not None:
+            self.slot_clip.copy_(slots_backup[0])
+            self.slot_cursor.copy_(slots_backup[1])
         self.graph = g
 
     # ---------------------------------------------------------------------------------------------
@@ -330,6 +357,8 @@ class CharacterizationSession:
         start (admission mode only): uint8 [B], 1 = the slot starts a new clip on this frame; None = no slot starts.
         Returns the frame outputs as a dict of float64 numpy arrays [B, ...]."""
         B, T = self.B, self.T
+        if self.bank is not None:
+            raise _lib.MochaError("a session with a source bank takes step_bank(start, clip, eps)")
         if self.admission:
             self.h_start.numpy()[...] = 0 if start is None else np.asarray(start, dtype=np.uint8)
             self.start.copy_(self.h_start, non_blocking=True)
@@ -354,12 +383,33 @@ class CharacterizationSession:
         torch.cuda.current_stream().synchronize()
         return self._decode_out(self.h_out.numpy())
 
+    def step_bank(self, start, clip, eps=None):
+        """End-to-end call of a session with a source bank: host (numpy) start row uint8 [B] (None = no slot starts),
+        clip row int32 [B] (bank clip ids, read where start is set; None = all 0) and optionally eps [B, D].
+        Returns the frame outputs as a dict of float64 numpy arrays [B, ...]."""
+        if self.bank is None:
+            raise _lib.MochaError("step_bank() needs CharacterizationSession(..., source_bank=...)")
+        self.h_start.numpy()[...] = 0 if start is None else np.asarray(start, dtype=np.uint8)
+        self.h_clip.numpy()[...] = 0 if clip is None else np.asarray(clip, dtype=np.int32)
+        self.start.copy_(self.h_start, non_blocking=True)
+        self.clip.copy_(self.h_clip, non_blocking=True)
+        if eps is not None:
+            self.h_eps.numpy()[...] = eps
+            self.eps.copy_(self.h_eps, non_blocking=True)
+        elif not self.deterministic:
+            self.eps.normal_()
+        self.step_device()
+        self.h_out.copy_(self.post.out, non_blocking=True)
+        torch.cuda.current_stream().synchronize()
+        return self._decode_out(self.h_out.numpy())
+
     # ---------------------------------------------------------------------------------------------
     # pipelined end-to-end streaming: the H2D copy of frame i+1 overlaps the kernels of frame i
     # ---------------------------------------------------------------------------------------------
     def pinned_inputs(self):
         """A set of pinned host tensors a caller fills for one frame (shapes of step_host's arguments,
-        with src_hips_vel/src_rvel/src_rang packed as `side` [B, T*3+6]; admission mode adds the uint8 [B] `start` row)."""
+        with src_hips_vel/src_rvel/src_rang packed as `side` [B, T*3+6]; admission mode adds the uint8 [B] `start` row).
+        A session with a source bank takes `start`, `clip` (int32 [B]) and `eps` only."""
         return {k: torch.zeros(getattr(self, k).shape, dtype=getattr(self, k).dtype).pin_memory()
                 for k in self._input_names}
 
@@ -407,6 +457,8 @@ class CharacterizationSession:
         return self._decode_out(s["h_out"].numpy())
 
     def h2d_bytes(self):
+        if self.bank is not None:
+            return self.h_start.numel() + self.h_clip.numel() * 4 + self.h_eps.numel() * 4
         return (self.h_X.numel() * 4 + self.h_side.numel() * 4 + self.h_contacts.numel() + self.h_eps.numel() * 4
                 + (self.h_start.numel() if self.admission else 0))
 
