@@ -452,6 +452,51 @@ int mocha_source_windows(const float* d_rot, const float* d_pos, const float* d_
                          int32_t* d_slot_clip, int32_t* d_slot_cursor, int B, float* d_X, float* d_side, int side_stride,
                          uint8_t* d_contacts, mocha_stream_t stream);
 
+/* ---- result bank: each served clip's motion recorded on the device, its bvh.save payload built per clip (DESIGN §5c)
+ * One record row per (clip, window), at row d_clip_first[c] + w of arrays sized like the source bank's frames (w < nwin
+ * < F keeps it inside the clip's frame range): the fields of mocha_frame_out the reference's final step reads, fp64,
+ * and the matched DB row. 1464 B. */
+typedef struct {
+  double ik_pos[25][3];
+  double ik_rot[25][4];
+  double src_root_pos[3];
+  double src_root_rot[4];
+  int64_t match;
+} mocha_frame_record;
+
+/* Per slot b, the last launch of an admission frame (after mocha_post_frame_packed_masked): the slot's record count
+ * d_slot_count[b] (int32 [B], session state) restarts at 0 if d_start[b]. If d_slot_clip[b] = c >= 0 (as
+ * mocha_source_windows left it for this frame) and count < nwin(c) = d_clip_frames[c] - T/4, d_out[b]'s ik_pos /
+ * ik_rot / src_root_pos / src_root_rot and d_match_idx[b * match_stride] go to d_rec[d_clip_first[c] + count]; then
+ * count += 1, d_clip_done[c] = count and d_clip_built[c] = 0 (int32 [n_clips] each; a new row makes the clip's payload
+ * stale). Idle slots and finished clips (whose last window the source
+ * bank repeats) write nothing. Bank tables as for mocha_source_windows; d_rec has n_rows rows. Copies only; one launch,
+ * graph-capturable. Two slots serving the same clip at once write the same rows: the caller must not do that. */
+int mocha_record_frames(const mocha_frame_out* d_out, const int64_t* d_match_idx, int match_stride,
+                        const uint8_t* d_start, const int32_t* d_slot_clip, int32_t* d_slot_count, int B,
+                        const int64_t* d_clip_first, const int32_t* d_clip_frames, int n_clips, int T,
+                        mocha_frame_record* d_rec, long long n_rows, int32_t* d_clip_done, int32_t* d_clip_built,
+                        mocha_stream_t stream);
+
+/* For the n_ids clip ids d_ids (int32, device), every recorded window w < min(d_clip_done[c], nwin(c)) of clip c: the
+ * payload the reference hands to bvh.save (test_fullframework.py:672-721), at row r = d_clip_first[c] + w of the
+ * outputs, [n_frames, 24, 3] each (joints 1..24; joint 1, the hips, takes its global transform; rotations as Euler 'xyz'
+ * degrees):
+ *   d_ours_pos / d_ours_rot fp64 from the recorded ik_pos / ik_rot;
+ *   d_src_pos / d_src_rot fp32 from the local pose of window w's last frame, as features.extract gives it (fk of the
+ *   bank frame d_rot / d_pos, re-rooting on its root, ik: bit for bit), with the recorded src_root_pos / src_root_rot
+ *   (cast to fp32) as the root;
+ *   d_match [n_frames] int64 the recorded matched DB row.
+ * d_clip_built[c] becomes 1 if clip c was complete (d_clip_done[c] >= nwin), else 0: a reader of the payload rows
+ * checks it, and the next record row of the clip clears it.
+ * J must be 25 (the record's skeleton); max_nwin >= the largest nwin among the ids. Ids outside [0, n_clips) are
+ * skipped. One warp per row, stream-ordered, off the frame. */
+int mocha_clip_payload(const mocha_frame_record* d_rec, long long n_frames, const float* d_rot, const float* d_pos,
+                       const int64_t* d_clip_first, const int32_t* d_clip_frames, int n_clips, const int32_t* d_clip_done,
+                       int32_t* d_clip_built, const int32_t* d_parents, int T, int J, const int32_t* d_ids, int n_ids, int max_nwin,
+                       float* d_src_rot, float* d_src_pos, double* d_ours_rot, double* d_ours_pos, int64_t* d_match,
+                       mocha_stream_t stream);
+
 /* ---- element-wise quaternion algebra of motion/quat.py in the caller's precision ------------- */
 /* out[i] = op(a[i], b[i]) for i < n; dense [n, width] arrays, float32 (is_f64 == 0) or float64. Ops and widths
  * (a, b, out): 0 mul (4,4,4) quat.py:112 | 1 inv_mul :122 | 2 mul_inv :125 | 3 mul_vec (4,3,3) :128 |

@@ -184,6 +184,8 @@ SIGNATURES = {
     "mocha_window_features": (_I, [_P, _P, _P, _P, _L, _I, _I, _P, _P, _P, _P, _P, _P]),
     "mocha_source_windows": (_I, [_P, _P, _P, _P, _P, _L, _P, _P, _I, _P, _I, _I, _P, _P, _P, _P, _P, _P, _I, _P, _P, _I,
                                   _P, _P]),
+    "mocha_record_frames": (_I, [_P, _P, _I, _P, _P, _P, _I, _P, _P, _I, _I, _P, _L, _P, _P, _P]),
+    "mocha_clip_payload": (_I, [_P, _L, _P, _P, _P, _P, _I, _P, _P, _P, _I, _I, _P, _I, _I, _P, _P, _P, _P, _P, _P]),
     "mocha_quat_op": (_I, [_I, _I, _P, _P, _L, C.c_double, _P, _P]),
     "mocha_fk_chain": (_I, [_I, _P, _P, _P, _P, _L, _I, _P, _P, _P]),
     "mocha_post_frame_packed": (_I, [C.POINTER(PostParams), _P, _P, _I, _P, _I, _I, _I, _I, _I, _P, _P, _P]),

@@ -43,20 +43,12 @@ def _final_payload(rot, pos, parents_t):
     return np.degrees(to_euler_xyz(out_rot)), out_pos
 
 
-def characterize(src_clip: dict, cha_clip: dict, raw_stats: dict, gen_sd=None, cvae_sd=None, eps_seq=None,
-                 precision: str = "fp32", encode_batch: int = 32, deterministic: bool = False,
-                 with_cm_path: bool = False) -> dict:
-    """with_cm_path: also run the reference loop's second decode of every frame, the matched DB row's ("cm_trans",
-    :465-472), and return its network output rows (Ytil_cm_rows) and the condition and normalised sample of the first
-    CVAE call (cvae_cond0, cvae_out0, frame 1)."""
+def _character_db(cha_clip: dict, raw_stats: dict, gen_sd, cvae_sd, stats: NormStats, precision: str,
+                  encode_batch: int):
+    """Encode the character clip into the feature DB (:213-279, :293-294): (encoded [N,90,256], cnt_nm [N,23040])."""
     dev = "cuda"
-    gen_sd = gen_sd or weights.generator_state_dict(1777)
-    cvae_sd = cvae_sd or weights.cvae_state_dict(1778)
-    stats = _stats_from_raw(raw_stats)
     Xm, Xs = raw_stats["norm"]["X_mean"], raw_stats["norm"]["X_std"]
-    src = features.extract(preprocess.process_clip(src_clip), Xm, Xs, dev)
     cha = features.extract(preprocess.process_clip(cha_clip), Xm, Xs, dev)
-    # encode the character clip into the feature DB (:271-279, :293-294)
     dummy = torch.zeros((1, 90, 256)), torch.zeros((1, 90 * 256))
     enc_sess = CharacterizationSession(gen_sd, cvae_sd, weights.DEFAULT_MODEL_CFG, stats, dummy[0], dummy[1],
                                        batch=encode_batch, device=dev, precision=precision)
@@ -69,8 +61,24 @@ def characterize(src_clip: dict, cha_clip: dict, raw_stats: dict, gen_sd=None, c
         enc_sess.encode(enc_sess.X, enc_sess.tokens, enc_sess.encoded, enc_sess.cnt, enc_sess.cnt_nm)
         encs.append(enc_sess.encoded[:m].clone())
         nms.append(enc_sess.cnt_nm[:m].clone())
-    del enc_sess
-    sess = CharacterizationSession(gen_sd, cvae_sd, weights.DEFAULT_MODEL_CFG, stats, torch.cat(encs), torch.cat(nms),
+    return torch.cat(encs), torch.cat(nms)
+
+
+def characterize(src_clip: dict, cha_clip: dict, raw_stats: dict, gen_sd=None, cvae_sd=None, eps_seq=None,
+                 precision: str = "fp32", encode_batch: int = 32, deterministic: bool = False,
+                 with_cm_path: bool = False) -> dict:
+    """with_cm_path: also run the reference loop's second decode of every frame, the matched DB row's ("cm_trans",
+    :465-472), and return its network output rows (Ytil_cm_rows) and the condition and normalised sample of the first
+    CVAE call (cvae_cond0, cvae_out0, frame 1)."""
+    dev = "cuda"
+    gen_sd = gen_sd or weights.generator_state_dict(1777)
+    cvae_sd = cvae_sd or weights.cvae_state_dict(1778)
+    stats = _stats_from_raw(raw_stats)
+    Xm, Xs = raw_stats["norm"]["X_mean"], raw_stats["norm"]["X_std"]
+    src = features.extract(preprocess.process_clip(src_clip), Xm, Xs, dev)
+    cha_enc, cha_nm = _character_db(cha_clip, raw_stats, gen_sd, cvae_sd, stats, precision, encode_batch)
+    n_cha = cha_enc.shape[0]
+    sess = CharacterizationSession(gen_sd, cvae_sd, weights.DEFAULT_MODEL_CFG, stats, cha_enc, cha_nm,
                                    batch=1, device=dev, precision=precision, match_tensor_cores=False,
                                    with_cm_path=with_cm_path)
     sess.deterministic = deterministic
@@ -114,3 +122,38 @@ def characterize(src_clip: dict, cha_clip: dict, raw_stats: dict, gen_sd=None, c
             "match": np.array(match), "Ytil_last_rows": np.stack(ytil_rows),
             "trans_pos": np.stack([f["blend_pos"][0] for f in frames]),
             "trans_rot": np.stack([f["rot"][0] for f in frames]), "n_db": int(n_cha)}
+
+
+def characterize_many(src_clips, cha_clip: dict, raw_stats: dict, gen_sd=None, cvae_sd=None, slots: int = 1,
+                      eps_seqs=None, precision: str = "fp32", encode_batch: int = 32, lanes: int = 1,
+                      with_cm_path: bool = False) -> list:
+    """The many-clip counterpart of characterize(): every source clip characterized with one target character through
+    a source bank, a result bank and one captured admission session of `slots` slots (CharacterizationSession.serve).
+    The character DB is built as characterize() builds it, and the session matches with the same fp64 brute-force
+    kernel (match_tensor_cores=False).
+
+    eps_seqs: None (fresh standard-normal draws) or {index into src_clips: array [nwin-1, 256]} in characterize()'s
+    eps_seq layout; clips without an entry draw standard-normal rows. Returns one dict per source clip:
+    {src_rotations, src_positions, ours_rotations, ours_positions, match}."""
+    from .result_bank import ResultBank
+    from .source_bank import SourceBank
+    src_clips = list(src_clips)
+    if not src_clips:
+        return []
+    dev = "cuda"
+    gen_sd = gen_sd or weights.generator_state_dict(1777)
+    cvae_sd = cvae_sd or weights.cvae_state_dict(1778)
+    stats = _stats_from_raw(raw_stats)
+    frames = [preprocess.process_frames(c) for c in src_clips]
+    bank = SourceBank(sum(f["pos"].shape[0] for f in frames), len(frames), raw_stats["norm"]["X_mean"],
+                      raw_stats["norm"]["X_std"], device=dev)
+    ids = [bank.add(f)[0] for f in frames]
+    results = ResultBank(bank)
+    cha_enc, cha_nm = _character_db(cha_clip, raw_stats, gen_sd, cvae_sd, stats, precision, encode_batch)
+    sess = CharacterizationSession(gen_sd, cvae_sd, weights.DEFAULT_MODEL_CFG, stats, cha_enc, cha_nm, batch=slots,
+                                   device=dev, precision=precision, match_tensor_cores=False, lanes=lanes,
+                                   with_cm_path=with_cm_path, admission=True, source_bank=bank, result_bank=results)
+    sess.capture()
+    eps = None if eps_seqs is None else {ids[i]: e for i, e in eps_seqs.items()}
+    out = sess.serve(ids, eps=eps)
+    return [out[c] for c in ids]

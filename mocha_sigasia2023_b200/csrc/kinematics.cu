@@ -1388,6 +1388,13 @@ __host__ __device__ inline QuatOpWidths quat_op_widths(int op) {
 
 template <typename T> __device__ __forceinline__ T clamp1(T x) { return x < (T)-1 ? (T)-1 : x > (T)1 ? (T)1 : x; }
 
+// quat.to_euler(order='xyz') (quat.py:346-358), radians; shared by quat_op_kernel and clip_payload_kernel
+template <typename T> __device__ __forceinline__ void to_euler_xyz(T q0, T q1, T q2, T q3, T* po) {
+  po[0] = atan2((T)2 * (q0 * q1 + q2 * q3), (T)1 - (T)2 * (q1 * q1 + q2 * q2));
+  po[1] = asin(clamp1((T)2 * (q0 * q2 - q3 * q1)));
+  po[2] = atan2((T)2 * (q0 * q3 + q1 * q2), (T)1 - (T)2 * (q2 * q2 + q3 * q3));
+}
+
 template <typename T>
 __global__ void quat_op_kernel(int op, const T* __restrict__ a, const T* __restrict__ b, long long n, T param,
                                T* __restrict__ out) {
@@ -1481,13 +1488,7 @@ __global__ void quat_op_kernel(int op, const T* __restrict__ a, const T* __restr
       po[0] = r.w; po[1] = r.x; po[2] = r.y; po[3] = r.z;
       break;
     }
-    case QOP_TO_EULER_XYZ: {
-      const T q0 = pa[0], q1 = pa[1], q2 = pa[2], q3 = pa[3];
-      po[0] = atan2((T)2 * (q0 * q1 + q2 * q3), (T)1 - (T)2 * (q1 * q1 + q2 * q2));
-      po[1] = asin(clamp1((T)2 * (q0 * q2 - q3 * q1)));
-      po[2] = atan2((T)2 * (q0 * q3 + q1 * q2), (T)1 - (T)2 * (q2 * q2 + q3 * q3));
-      break;
-    }
+    case QOP_TO_EULER_XYZ: to_euler_xyz(pa[0], pa[1], pa[2], pa[3], po); break;
     case QOP_TO_EULER_YZX: {
       const T q0 = pa[0], q1 = pa[1], q2 = pa[2], q3 = pa[3];
       po[0] = atan2((T)2 * (q1 * q0 - q2 * q3), -q1 * q1 + q2 * q2 - q3 * q3 + q0 * q0);
@@ -1854,6 +1855,153 @@ source_windows_kernel(const float* __restrict__ brot, const float* __restrict__ 
     out_side[i] = v;
   }
 }
+
+// ------------------------------------------------------------------------------------------------
+// Result bank (DESIGN §5c). record_frames_kernel is the last launch of a frame: one warp per slot copies the slot's
+// ik_pos / ik_rot / src_root_pos / src_root_rot (one contiguous span of mocha_frame_out) and its matched DB row into
+// record row clip_first[c] + count of the clip c the slot served this frame. Copies only: nothing here lengthens the
+// frame's critical path beyond a ~1.5 KB store per slot.
+// clip_payload_kernel runs off the frame, once per batch of finished clips: one warp per (clip, window) row, one lane
+// per joint, builds what the reference hands to bvh.save (test_fullframework.py:672-721; final_payload).
+// ------------------------------------------------------------------------------------------------
+constexpr int RF_WARPS = 4;
+constexpr int REC_SPAN = 25 * 3 + 25 * 4 + 3 + 4;     // doubles from mocha_frame_out::ik_pos through src_root_rot
+static_assert(offsetof(mocha_frame_out, src_root_rot) + 4 * sizeof(double) ==
+              offsetof(mocha_frame_out, ik_pos) + REC_SPAN * sizeof(double), "frame_out record span is not contiguous");
+static_assert(offsetof(mocha_frame_record, match) == REC_SPAN * sizeof(double) && sizeof(mocha_frame_record) == 1464,
+              "mocha_frame_record layout");
+
+__global__ void __launch_bounds__(RF_WARPS * 32)
+record_frames_kernel(const mocha_frame_out* __restrict__ out, const int64_t* __restrict__ match_idx, int match_stride,
+                     const uint8_t* __restrict__ start, const int32_t* __restrict__ slot_clip,
+                     int32_t* __restrict__ slot_count, int B, const long long* __restrict__ clip_first,
+                     const int32_t* __restrict__ clip_frames, int n_clips, int T, mocha_frame_record* __restrict__ rec,
+                     long long n_rows, int32_t* __restrict__ clip_done, int32_t* __restrict__ clip_built) {
+  pdl_trigger();
+  pdl_wait();
+  const int b = blockIdx.x * RF_WARPS + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (b >= B) return;
+  long long row = -1;
+  if (lane == 0) {
+    int n = start[b] ? 0 : slot_count[b];
+    const int c = slot_clip[b];                          // as mocha_source_windows left it for this frame
+    if (c >= 0 && c < n_clips) {
+      const int nwin = clip_frames[c] - T / 4;
+      const long long r = clip_first[c] + n;
+      if (n < nwin && r >= 0 && r < n_rows) {            // a finished clip's repeated last window writes nothing
+        row = r;
+        clip_done[c] = ++n;
+        clip_built[c] = 0;                               // a new row makes the clip's payload stale
+      }
+    }
+    slot_count[b] = n;
+  }
+  row = __shfl_sync(0xffffffffu, row, 0);
+  if (row < 0) return;
+  const double* src = &out[b].ik_pos[0][0];
+  double* dst = &rec[row].ik_pos[0][0];
+  for (int i = lane; i < REC_SPAN; i += 32) dst[i] = src[i];
+  if (lane == 0) rec[row].match = match_idx[(long long)b * match_stride];
+}
+
+constexpr int CP_WARPS = 4;
+constexpr int REC_J = 25;
+
+__global__ void __launch_bounds__(CP_WARPS * 32)
+clip_payload_kernel(const mocha_frame_record* __restrict__ rec, long long n_frames, const float* __restrict__ brot,
+                    const float* __restrict__ bpos, const long long* __restrict__ clip_first,
+                    const int32_t* __restrict__ clip_frames, int n_clips, const int32_t* __restrict__ clip_done,
+                    int32_t* __restrict__ clip_built,
+                    const int32_t* __restrict__ parents, int T, const int32_t* __restrict__ ids,
+                    float* __restrict__ src_rot, float* __restrict__ src_pos, double* __restrict__ ours_rot,
+                    double* __restrict__ ours_pos, int64_t* __restrict__ match) {
+  pdl_trigger();
+  pdl_wait();
+  constexpr int J = REC_J;
+  constexpr unsigned FULL = 0xffffffffu;
+  const int lane = threadIdx.x & 31, w = blockIdx.x * CP_WARPS + (threadIdx.x >> 5);
+  const int c = ids[blockIdx.y];
+  if (c < 0 || c >= n_clips) return;
+  const int F = clip_frames[c];
+  const long long first = clip_first[c];
+  const int nwin = F - T / 4;
+  if (nwin < 1 || first < 0 || first + F > n_frames) return;
+  const int done = clip_done[c];
+  if (blockIdx.x == 0 && threadIdx.x == 0) clip_built[c] = done >= nwin;   // the payload of a complete clip
+  if (w >= min(done, nwin)) return;                      // warp-uniform
+  const long long row = first + w;
+  const int j = lane;
+  const bool on = j < J;
+  const int pj = on ? parents[j] : -1;
+  const int d = on ? joint_depth(parents, j, J) : 0;
+  const int maxd = __reduce_max_sync(FULL, d);
+  // src: the local pose of window w's last frame as features.extract gives it (Ypos[w, -1] / Yrot[w, -1]): fk of that
+  // frame (sliding_windows' edge padding keeps the edge frame's pose), re-rooted on its own root, then ik
+  bool pad;
+  const long long f = (first + window_frame(T - 1, w, F, T, pad)) * J + (on ? j : 0);
+  const Q4<float> lr = q4<float>(brot[f * 4], brot[f * 4 + 1], brot[f * 4 + 2], brot[f * 4 + 3]);
+  const V3<float> lp = v3<float>(bpos[f * 3], bpos[f * 3 + 1], bpos[f * 3 + 2]);
+  Q4<float> gr = lr;
+  V3<float> gp = lp;
+  const int src_lane = pj >= 0 ? pj : j;
+  for (int lvl = 1; lvl <= maxd; ++lvl) {                // quat.fk, one hierarchy level at a time
+    const Q4<float> pr = q4<float>(__shfl_sync(FULL, gr.w, src_lane), __shfl_sync(FULL, gr.x, src_lane),
+                                   __shfl_sync(FULL, gr.y, src_lane), __shfl_sync(FULL, gr.z, src_lane));
+    const V3<float> pp = v3<float>(__shfl_sync(FULL, gp.x, src_lane), __shfl_sync(FULL, gp.y, src_lane),
+                                   __shfl_sync(FULL, gp.z, src_lane));
+    if (d == lvl) {
+      V3<float> rp;
+      fk_joint_pose(pr, pp, lr, lp, rp, gp, gr);
+    }
+  }
+  const Q4<float> r0 = q4<float>(__shfl_sync(FULL, gr.w, 0), __shfl_sync(FULL, gr.x, 0), __shfl_sync(FULL, gr.y, 0),
+                                 __shfl_sync(FULL, gr.z, 0));
+  const V3<float> p0 = v3<float>(__shfl_sync(FULL, gp.x, 0), __shfl_sync(FULL, gp.y, 0), __shfl_sync(FULL, gp.z, 0));
+  const V3<float> zero3 = v3<float>(0.0f, 0.0f, 0.0f);
+  V3<float> xp, xv, xa;
+  Q4<float> xr;
+  reroot_joint(qinv(r0), p0, gr, gp, zero3, zero3, xp, xr, xv, xa);
+  const Q4<float> pxr = q4<float>(__shfl_sync(FULL, xr.w, src_lane), __shfl_sync(FULL, xr.x, src_lane),
+                                  __shfl_sync(FULL, xr.y, src_lane), __shfl_sync(FULL, xr.z, src_lane));
+  const V3<float> pxp = v3<float>(__shfl_sync(FULL, xp.x, src_lane), __shfl_sync(FULL, xp.y, src_lane),
+                                  __shfl_sync(FULL, xp.z, src_lane));
+  Q4<float> sr = xr;                                     // a root joint's local transform is its global one
+  V3<float> sp = xp;
+  if (pj >= 0) ik_joint(pxr, pxp, xr, xp, sr, sp);
+  if (!on || j == 0) return;                             // the payload drops the simulation root
+  const mocha_frame_record& R = rec[row];
+  // ours (fp64): the recorded post-IK pose
+  DQ orr = ld4(&R.ik_rot[j][0]);
+  D3 op = ld3(&R.ik_pos[j][0]);
+  if (j == 1 && pj == 0) {
+    // hips: global transform under the recorded root; src in fp32 under the integrated source root (:478-488)
+    const DQ r = ld4(&R.ik_rot[0][0]);
+    op = qrot(r, op) + ld3(&R.ik_pos[0][0]);
+    orr = qmul(r, orr);
+    const Q4<float> qr = q4<float>((float)R.src_root_rot[0], (float)R.src_root_rot[1], (float)R.src_root_rot[2],
+                                   (float)R.src_root_rot[3]);
+    const V3<float> qp = v3<float>((float)R.src_root_pos[0], (float)R.src_root_pos[1], (float)R.src_root_pos[2]);
+    V3<float> rp, hp;
+    Q4<float> hr;
+    fk_joint_pose(qr, qp, sr, sp, rp, hp, hr);
+    sr = hr;
+    sp = hp;
+  }
+  const long long o = (row * (J - 1) + (j - 1)) * 3;
+  float fe[3];
+  to_euler_xyz(sr.w, sr.x, sr.y, sr.z, fe);
+  double de[3];
+  to_euler_xyz(orr.w, orr.x, orr.y, orr.z, de);
+  constexpr double DEG = 180.0 / 3.14159265358979323846;          // np.degrees
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    src_rot[o + k] = fe[k] * (float)DEG;
+    ours_rot[o + k] = de[k] * DEG;
+  }
+  src_pos[o] = sp.x; src_pos[o + 1] = sp.y; src_pos[o + 2] = sp.z;
+  ours_pos[o] = op.x; ours_pos[o + 1] = op.y; ours_pos[o + 2] = op.z;
+  if (j == 1) match[row] = R.match;
+}
 }  // namespace
 
 extern "C" int mocha_window_features(const float* grot, const float* gpos, const float* gvel, const float* gang, long long W,
@@ -1898,5 +2046,44 @@ extern "C" int mocha_source_windows(const float* rot, const float* pos, const fl
            slot_clip, slot_cursor, X, side, side_stride, contacts);
   count_launch();
   MOCHA_LAUNCH_CHECK("source_windows_kernel");
+  return MOCHA_OK;
+}
+
+extern "C" int mocha_record_frames(const mocha_frame_out* out, const int64_t* match_idx, int match_stride,
+                                   const uint8_t* start, const int32_t* slot_clip, int32_t* slot_count, int B,
+                                   const int64_t* clip_first, const int32_t* clip_frames, int n_clips, int T,
+                                   mocha_frame_record* rec, long long n_rows, int32_t* clip_done, int32_t* clip_built,
+                                   mocha_stream_t stream) {
+  MOCHA_CHECK_ARG(out && match_idx && start && slot_clip && slot_count, "mocha_record_frames: null slot argument");
+  MOCHA_CHECK_ARG(clip_first && clip_frames && rec && clip_done && clip_built, "mocha_record_frames: null bank argument");
+  MOCHA_CHECK_ARG(B > 0 && n_clips > 0 && n_rows > 0 && match_stride >= 1 && T >= 5,
+                  "mocha_record_frames: bad sizes B=%d n_clips=%d n_rows=%lld match_stride=%d T=%d", B, n_clips, n_rows,
+                  match_stride, T);
+  launch_k(record_frames_kernel, ceil_div(B, RF_WARPS), RF_WARPS * 32, 0, (cudaStream_t)stream, out, match_idx,
+           match_stride, start, slot_clip, slot_count, B, reinterpret_cast<const long long*>(clip_first), clip_frames,
+           n_clips, T, rec, n_rows, clip_done, clip_built);
+  count_launch();
+  MOCHA_LAUNCH_CHECK("record_frames_kernel");
+  return MOCHA_OK;
+}
+
+extern "C" int mocha_clip_payload(const mocha_frame_record* rec, long long n_frames, const float* rot, const float* pos,
+                                  const int64_t* clip_first, const int32_t* clip_frames, int n_clips,
+                                  const int32_t* clip_done, int32_t* clip_built, const int32_t* parents, int T, int J,
+                                  const int32_t* ids,
+                                  int n_ids, int max_nwin, float* src_rot, float* src_pos, double* ours_rot,
+                                  double* ours_pos, int64_t* match, mocha_stream_t stream) {
+  MOCHA_CHECK_ARG(rec && rot && pos && clip_first && clip_frames && clip_done && clip_built && parents,
+                  "mocha_clip_payload: null bank argument");
+  MOCHA_CHECK_ARG(ids && src_rot && src_pos && ours_rot && ours_pos && match, "mocha_clip_payload: null output argument");
+  MOCHA_CHECK_ARG(n_frames > 0 && n_clips > 0 && n_ids > 0 && n_ids <= 65535 && max_nwin > 0,
+                  "mocha_clip_payload: bad sizes n_frames=%lld n_clips=%d n_ids=%d max_nwin=%d", n_frames, n_clips, n_ids,
+                  max_nwin);
+  MOCHA_CHECK_ARG(J == REC_J && T >= 5, "mocha_clip_payload: need J=%d and T >= 5, got J=%d T=%d", REC_J, J, T);
+  launch_k(clip_payload_kernel, dim3((unsigned)ceil_div(max_nwin, CP_WARPS), (unsigned)n_ids), CP_WARPS * 32, 0,
+           (cudaStream_t)stream, rec, n_frames, rot, pos, reinterpret_cast<const long long*>(clip_first), clip_frames,
+           n_clips, clip_done, clip_built, parents, T, ids, src_rot, src_pos, ours_rot, ours_pos, match);
+  count_launch();
+  MOCHA_LAUNCH_CHECK("clip_payload_kernel");
   return MOCHA_OK;
 }

@@ -36,7 +36,7 @@ class NormStats:
 class CharacterizationSession:
     def __init__(self, gen_sd, cvae_sd, cfg, stats: NormStats, cha_encoded, cha_cnt_nm, batch: int,
                  device="cuda", precision="fp32", with_cm_path=False, match_tensor_cores=None, post_params=None,
-                 lanes: int = 1, admission: bool = False, source_bank=None):
+                 lanes: int = 1, admission: bool = False, source_bank=None, result_bank=None):
         """gen_sd / cvae_sd: reference-layout state dicts. cha_encoded [N,90,256] and cha_cnt_nm [N,23040]
         (already (cnt-mean)/std scaled): the target character's feature DB, CUDA or CPU tensors.
 
@@ -55,9 +55,18 @@ class CharacterizationSession:
         an int32 [B] `clip` row (the bank's clip id of each starting slot, read only where start is set) and eps
         (step_bank(), or pinned_inputs() for submit / collect). A started slot serves its clip's windows one per frame
         and repeats the last one once the clip has ended; an idle slot (never started, or started with an id the bank
-        does not hold) gets zero inputs."""
+        does not hold) gets zero inputs.
+
+        result_bank (a ResultBank of the same source_bank): the last launch of each lane's frame, mocha_record_frames,
+        records every serving slot's post-IK pose, integrated source root and matched DB row into the clip's record
+        rows (the `post` path; the reference exports no other). serve() runs a list of bank clips through the slots and
+        returns each clip's bvh.save payload, built on the device."""
         if source_bank is not None and not admission:
             raise _lib.MochaError("source_bank needs CharacterizationSession(admission=True)")
+        if result_bank is not None and source_bank is None:
+            raise _lib.MochaError("result_bank needs CharacterizationSession(..., source_bank=...)")
+        if result_bank is not None and result_bank.bank is not source_bank:
+            raise _lib.MochaError("result_bank records another source bank than this session's source_bank")
         self.lib = _lib.load()
         _lib.check(self.lib.mocha_check_device(), "mocha_check_device")
         dev = torch.device(device)
@@ -116,6 +125,9 @@ class CharacterizationSession:
             self.slot_clip = torch.full((B,), -1, dtype=torch.int32, device=dev)
             self.slot_cursor = torch.zeros((B,), dtype=torch.int32, device=dev)
             self._input_names = ("start", "clip", "eps")
+        self.results = result_bank
+        if result_bank is not None:
+            self.slot_count = torch.zeros((B,), dtype=torch.int32, device=dev)   # windows recorded by each slot's clip
         # intermediates
         self.tokens = torch.empty((B, n, D), **f32)
         self.encoded = torch.empty((B, n, D), **f32)
@@ -261,6 +273,9 @@ class CharacterizationSession:
             torch.index_select(self.cha_encoded, 0, self.match_idx[sl, 0], out=self.cm_cha[sl])
         self._decode(self.encoded[sl], self.prev_cha[sl], self.decoded[sl], self.Y[sl], ws)
         self.post.step_packed(self.Y[sl], self.side[sl], self.contacts[sl], lo=lo, start=self.start[sl])
+        if self.results is not None:
+            self.results.record(self.post.out.view(self.B, -1)[sl].view(-1), self.match_idx[sl], self.start[sl],
+                                self.slot_clip[sl], self.slot_count[sl])
         if self.with_cm_path:
             self._decode(self.encoded[sl], self.cm_cha[sl], self.decoded[sl], self.cm_Y[sl], ws)
             self.cm_post.step_packed(self.cm_Y[sl], self.side[sl], self.contacts[sl], lo=lo, start=self.start[sl])
@@ -323,6 +338,8 @@ class CharacterizationSession:
         state_backup = (self.prev_cha.clone(), self.post.state.clone(),
                         self.cm_post.state.clone() if self.cm_post else None)
         slots_backup = (self.slot_clip.clone(), self.slot_cursor.clone()) if self.bank is not None else None
+        rec_backup = ((self.slot_count.clone(), self.results.clip_done.clone(), self.results.clip_built.clone())
+                      if self.results is not None else None)
         s = torch.cuda.Stream()
         s.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(s):
@@ -339,6 +356,10 @@ class CharacterizationSession:
         if slots_backup is not None:
             self.slot_clip.copy_(slots_backup[0])
             self.slot_cursor.copy_(slots_backup[1])
+        if rec_backup is not None:      # record rows the warm-up wrote are rewritten by the next real frame
+            self.slot_count.copy_(rec_backup[0])
+            self.results.clip_done.copy_(rec_backup[1])
+            self.results.clip_built.copy_(rec_backup[2])
         self.graph = g
 
     # ---------------------------------------------------------------------------------------------
@@ -428,6 +449,15 @@ class CharacterizationSession:
     def submit(self, pinned: dict) -> int:
         """Enqueue one frame from pinned host inputs (see pinned_inputs()); returns a ticket for collect().
         The caller must not modify `pinned` until the next-but-one submit."""
+        t, s = self._enqueue(pinned, self._input_names)
+        main = torch.cuda.current_stream()
+        s["h_out"].copy_(self.post.out, non_blocking=True)
+        s["done"].record(main)
+        return t
+
+    def _enqueue(self, pinned: dict, names):
+        """H2D of the inputs `names` from pinned host tensors on the copy stream (double-buffered device staging), then
+        one frame on the current stream. Returns (ticket, pipeline slot)."""
         if not hasattr(self, "_slots"):
             self._pipe_init()
         t = self._ticket
@@ -436,19 +466,128 @@ class CharacterizationSession:
         if s["used"]:
             self._copy_stream.wait_event(s["consumed"])
         with torch.cuda.stream(self._copy_stream):
-            for k in self._input_names:
+            for k in names:
                 s[k].copy_(pinned[k], non_blocking=True)
             s["h2d"].record(self._copy_stream)
         main.wait_event(s["h2d"])
-        for k in self._input_names:
+        for k in names:
             getattr(self, k).copy_(s[k])
         s["consumed"].record(main)
-        self.step_device()
-        s["h_out"].copy_(self.post.out, non_blocking=True)
-        s["done"].record(main)
-        s["used"] = True
+        s["used"] = True            # the next fill of this staging slot waits until this frame has read it
         self._ticket += 1
-        return t
+        self.step_device()
+        return t, s
+
+    def serve(self, clip_ids, eps=None) -> dict:
+        """Run the source bank's clips `clip_ids` through the slots and return {clip_id: payload}, each payload a dict
+        of numpy arrays {src_rotations, src_positions [nwin,24,3] float32, ours_rotations, ours_positions [nwin,24,3]
+        float64, match [nwin] int64}: what characterize() returns for one clip (test_fullframework.py:672-721).
+
+        Clips are placed by serving_schedule (first free slot, FIFO) and start on the frame their slot frees up. Per
+        frame only the start / clip rows (and eps) go to the device, from pinned double-buffered host rows on a copy
+        stream; the host never waits for a frame, only for the copy of the buffer it refills. Before the first of them,
+        one extra frame starts every slot idle (start = 1, clip = -1), so that no slot keeps recording a clip of an
+        earlier call into the bank's rows; it costs one frame per call and resets every slot's state. After the frame on which
+        clips end, one mocha_clip_payload launch on a side stream converts them, and their rows download into pinned
+        memory while later frames run. The returned arrays are views of one host buffer per call.
+
+        eps None: eps.normal_() every frame, as step_bank does (the draws then depend on the schedule). Otherwise
+        {clip_id: array [nwin-1, D]} in characterize()'s eps_seq layout: window w >= 1 of the clip uses row w-1,
+        wherever and whenever it runs; clips without a table draw standard-normal rows on the host.
+        """
+        from .result_bank import PAYLOAD_KEYS, serving_schedule
+        if self.results is None:
+            raise _lib.MochaError("serve() needs CharacterizationSession(..., result_bank=...)")
+        ids = [int(c) for c in clip_ids]
+        if len(set(ids)) != len(ids):
+            raise _lib.MochaError("serve(): duplicate clip ids (one clip cannot run in two slots at once)")
+        if not ids:
+            return {}
+        self.results._check_ids(ids)
+        bank, B, D = self.bank, self.B, self.D
+        nwins = np.array([bank.clip_nwin[c] for c in ids], dtype=np.int64)
+        tables, rng = None, None
+        if eps is not None:
+            tables = {}
+            for c in ids:
+                if c in eps:
+                    e = np.asarray(eps[c], dtype=np.float32)
+                    if e.shape != (bank.clip_nwin[c] - 1, D):
+                        raise _lib.MochaError(f"serve(): eps of clip {c} must be [{bank.clip_nwin[c] - 1}, {D}], got {e.shape}")
+                    tables[c] = e
+            rng = np.random.default_rng()
+        start_rows, clip_rows, place = serving_schedule(nwins, B)
+        nframes = start_rows.shape[0]
+        ends = place[:, 1] + nwins - 1
+        order = np.argsort(ends, kind="stable")           # clips in the order they end
+        ends_sorted = ends[order]
+        dev = self.dev
+        ids_dev = torch.tensor([ids[k] for k in order], dtype=torch.int32, device=dev)
+        # host payload buffers: clip k at rows off[k] .. + nwin
+        off = np.concatenate([[0], np.cumsum(nwins)[:-1]])
+        total = int(nwins.sum())
+        host = [torch.empty((total,) + tuple(t.shape[1:]), dtype=t.dtype).pin_memory()
+                for t in self.results.payload_arrays()]
+        names = ("start", "clip") + (("eps",) if tables is not None else ())
+        pins = [{k: torch.zeros(getattr(self, k).shape, dtype=getattr(self, k).dtype).pin_memory() for k in names}
+                for _ in range(2)]
+        pin_ready = [None, None]
+        side = torch.cuda.Stream(device=dev)
+        main = torch.cuda.current_stream()
+        ids_np = np.asarray(ids, dtype=np.int32)
+        slot_clip = np.full(B, -1, dtype=np.int64)        # schedule index of each slot's clip
+        slot_first = np.zeros(B, dtype=np.int64)
+        self.start.fill_(1)                              # drop whatever the slots held: start them idle
+        self.clip.fill_(-1)
+        self.step_device()
+        self.start.zero_()
+        j = 0
+        for f in range(nframes):
+            p = pins[f % 2]
+            if pin_ready[f % 2] is not None:
+                pin_ready[f % 2].synchronize()           # the copy of frame f-2 out of this buffer has finished
+            st = start_rows[f]
+            p["start"].numpy()[...] = st
+            p["clip"].numpy()[...] = ids_np[clip_rows[f]]
+            new = np.nonzero(st)[0]
+            slot_clip[new], slot_first[new] = clip_rows[f][new], f
+            if tables is not None:
+                er = p["eps"].numpy()
+                er[...] = 0.0
+                for b in range(B):
+                    k = slot_clip[b]
+                    if k < 0:
+                        continue
+                    w = f - slot_first[b]
+                    if 1 <= w < nwins[k]:
+                        e = tables.get(ids[k])
+                        er[b] = e[w - 1] if e is not None else rng.standard_normal(D, dtype=np.float32)
+            elif not self.deterministic:
+                self.eps.normal_()
+            _, s = self._enqueue(p, names)
+            ev = torch.cuda.Event()
+            ev.record(self._copy_stream)
+            pin_ready[f % 2] = ev
+            if j < len(order) and ends_sorted[j] == f:
+                j1 = j
+                while j1 < len(order) and ends_sorted[j1] == f:
+                    j1 += 1
+                done_ev = torch.cuda.Event()
+                done_ev.record(main)
+                side.wait_event(done_ev)
+                with torch.cuda.stream(side):
+                    ks = order[j:j1]
+                    self.results.payload_device(ids_dev[j:], j1 - j, int(nwins[ks].max()))
+                    for k in ks:
+                        first, n = bank.clip_start[ids[k]], int(nwins[k])
+                        for h, t in zip(host, self.results.payload_arrays()):
+                            h[off[k]:off[k] + n].copy_(t[first:first + n], non_blocking=True)
+                j = j1
+        side.synchronize()
+        main.synchronize()
+        hv = [h.numpy() for h in host]
+        return {ids[k]: {name: a[off[k]:off[k] + int(nwins[k])] for name, a in zip(PAYLOAD_KEYS, hv)}
+                for k in range(len(ids))}
 
     def collect(self, ticket: int) -> dict:
         """Wait for a submitted frame and return its outputs (dict of float64 numpy arrays [B, ...])."""

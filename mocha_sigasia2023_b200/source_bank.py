@@ -39,6 +39,8 @@ class SourceBank:
         self.X_std = torch.from_numpy(xs).to(dev)
         self.n_clips = 0
         self.n_frames = 0
+        self.clip_nwin: list[int] = []      # host copy of each clip's window count
+        self.clip_start: list[int] = []     # host copy of clip_first
 
     def add(self, clip: dict) -> tuple[int, int]:
         """Append one clip: a raw clip dict (motion/bvh.py:load layout; preprocessed with preprocess.process_frames) or
@@ -66,6 +68,8 @@ class SourceBank:
         self.clip_first[c:c + 1].copy_(torch.tensor([a], dtype=torch.int64))
         self.clip_frames[c:c + 1].copy_(torch.tensor([F], dtype=torch.int32))
         self.n_frames, self.n_clips = a + F, c + 1
+        self.clip_nwin.append(nwin)
+        self.clip_start.append(a)
         return c, nwin
 
     def clear(self):
@@ -73,6 +77,7 @@ class SourceBank:
         given that id next from its old cursor: start the slots anew after clear()."""
         self.clip_frames.zero_()
         self.n_clips = self.n_frames = 0
+        self.clip_nwin, self.clip_start = [], []
 
     def nbytes(self) -> int:
         """Device memory of the bank arrays and clip tables."""

@@ -52,7 +52,7 @@ def step_inputs(B: int, seed: int) -> dict:
 def build_session(batch: int, n_db: int = 385, precision: str = "fp32", device="cuda", seed: int = 0,
                   with_cm_path: bool = False, match_tensor_cores=None, gen_seed: int = 1777, cvae_seed: int = 1778,
                   db_precision: str = "fp32", db_batch: int = 64, lanes: int = 1, admission: bool = False,
-                  source_bank=None):
+                  source_bank=None, result_bank=None):
     """Session on random-init weights with a character DB of n_db encoded synthetic windows
     (n_db = 385 is what a 400-frame character clip yields, SURVEY §8d config 1). The DB comes from the
     feature-DB builder (feature_db.build_feature_db: same CUDA encoder, matcher layout)."""
@@ -68,6 +68,6 @@ def build_session(batch: int, n_db: int = 385, precision: str = "fp32", device="
                                    BallTree.from_feature_db(fdb, device=device, use_tensor_cores=match_tensor_cores),
                                    batch=batch, device=device, precision=precision, with_cm_path=with_cm_path,
                                    match_tensor_cores=match_tensor_cores, lanes=lanes, admission=admission,
-                                   source_bank=source_bank)
+                                   source_bank=source_bank, result_bank=result_bank)
     sess.feature_db = fdb
     return sess, gen_sd, cvae_sd, stats

@@ -46,6 +46,7 @@ def main():
     import torch
     from admission_bench import gpu_info
     from mocha_sigasia2023_b200 import _lib, preprocess, synthetic, workload
+    from mocha_sigasia2023_b200.result_bank import serving_schedule
     from mocha_sigasia2023_b200.source_bank import SourceBank
     if not torch.cuda.is_available():
         raise SystemExit("source_bank_bench needs a CUDA device (there is no CPU measurement)")
@@ -171,23 +172,11 @@ def main():
         kernels[arm] = {"kernel_us_per_step_sum": total / 20, "kernels": per}
 
     # ---- serving run: the mixed-length clips through the bank session's slots ----
-    queue, slot_left, start_rows, clip_rows = list(range(args.clips)), np.zeros(B, dtype=np.int64), [], []
-    busy = 0
-    while queue or slot_left.any():
-        row, crow = np.zeros(B, dtype=np.uint8), np.zeros(B, dtype=np.int32)
-        for s in range(B):
-            if slot_left[s] == 0 and queue:
-                c = queue.pop(0)
-                slot_left[s], row[s], crow[s] = nwins[c], 1, c
-        busy += int((slot_left > 0).sum())
-        start_rows.append(row)
-        clip_rows.append(crow)
-        slot_left = np.maximum(slot_left - 1, 0)
+    start_rows, clip_rows, _ = serving_schedule(nwins, B)
     nframes = len(start_rows)
-    starts_dev = torch.from_numpy(np.stack(start_rows)).to(dev)
-    clips_dev = torch.from_numpy(np.stack(clip_rows)).to(dev)
+    starts_dev = torch.from_numpy(start_rows).to(dev)
+    clips_dev = torch.from_numpy(clip_rows).to(dev)
     useful = int(nwins.sum())
-    assert busy == useful
     torch.cuda.synchronize()
     e0.record()
     for f in range(nframes):
