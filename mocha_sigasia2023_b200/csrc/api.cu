@@ -1,5 +1,4 @@
 // Library-level entry points of the C ABI: error channel, version, device check, launch counter.
-#include <cstdlib>
 #include "../../include/mocha_b200.h"
 #include "common.cuh"
 #include "gemm_tc.cuh"
@@ -20,14 +19,6 @@ int set_error(int code, const char* fmt, ...) {
 }
 const char* last_error() { return g_err; }
 void count_launch(int n) { g_launches.fetch_add(n, std::memory_order_relaxed); }
-
-bool pdl_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("MOCHA_PDL");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
 
 }  // namespace mocha
 

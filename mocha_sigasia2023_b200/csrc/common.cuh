@@ -55,11 +55,9 @@ void count_launch(int n = 1);
 //     (griddepcontrol.wait = the previous grid has completed and its memory is visible);
 //   * every kernel executes pdl_wait() before it exits, so completion stays transitive along the stream.
 // A ~110-launch frame captured in a CUDA graph keeps these edges as programmatic dependencies.
-// MOCHA_PDL=0 in the environment launches everything with plain stream serialization (A/B switch).
 // ---------------------------------------------------------------------------------------------
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-bool pdl_enabled();
 
 template <typename... KArgs, typename... Args>
 inline void launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args&&... args) {
@@ -72,7 +70,7 @@ inline void launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t sme
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = 1;
   (void)cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);   // errors surface through MOCHA_LAUNCH_CHECK
 }
 

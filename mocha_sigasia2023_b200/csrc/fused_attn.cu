@@ -15,8 +15,6 @@
 // epilogue (two warps per TMEM lane quarter split the key columns / the head dimension and exchange row maxima and sums).
 #include "fused.cuh"
 
-#include <cstdlib>
-
 #include "gemm_tc.cuh"
 #include "tc_ptx.cuh"
 
@@ -365,9 +363,8 @@ int tc_attn_fused(const __nv_bfloat16* q, int ldq, const __nv_bfloat16* k, int l
   const uint32_t v_bytes = (uint32_t)nkb * (uint32_t)dkb * 8192u;
   // two-group mode: double-buffered scores / outputs in TMEM, two P buffers (each also hosts 4 warps x 2 staging boxes);
   // a second Q / K stage when it still fits
-  static const bool one_group = getenv("MOCHA_ATTN_ONE_GROUP") != nullptr;
   const size_t fixed = 256 + 2048;
-  p.groups = (!one_group && 2 * (p.npad + dh) <= 512 && p.p_bytes >= 32768u &&
+  p.groups = (2 * (p.npad + dh) <= 512 && p.p_bytes >= 32768u &&
               (size_t)p.qk_stride + v_bytes + 2 * (size_t)p.p_bytes + fixed <= 227 * 1024) ? 2 : 1;
   p.qk_stages = (p.groups == 2 && 2 * (size_t)p.qk_stride + v_bytes + 2 * (size_t)p.p_bytes + fixed <= 227 * 1024) ? 2 : 1;
   p.off_v = (uint32_t)p.qk_stages * p.qk_stride;

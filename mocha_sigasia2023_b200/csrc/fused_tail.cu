@@ -75,26 +75,10 @@ struct TailParams {
   int r0_period;     // > 0: the residual is a [period, 256] table shared by every group of `period` rows
 };
 
-__device__ __forceinline__ float gelu_fast_f(float x) {
-  // GELU(x) = x/2 (1 + erf(x / sqrt 2)); erf through Abramowitz & Stegun 7.1.28 (|error| <= 3e-7), see gemm_tc.cu
-  const float t = fabsf(x) * 0.70710678118654752f;
-  float p = fmaf(0.0000430638f, t, 0.0002765672f);
-  p = fmaf(p, t, 0.0001520143f);
-  p = fmaf(p, t, 0.0092705272f);
-  p = fmaf(p, t, 0.0422820123f);
-  p = fmaf(p, t, 0.0705230784f);
-  p = fmaf(p, t, 1.0f);
-  p *= p; p *= p; p *= p; p *= p;
-  float rp;
-  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(rp) : "f"(p));
-  const float e = 1.0f - rp;
-  return 0.5f * x * (1.0f + copysignf(e, x));
-}
-
 // Hidden-layer GELU of the fused path: tanh form on the hardware tanh (MUFU.TANH), ~7 instructions per element instead of
 // ~22 for the erf polynomial - the hidden epilogue is issue-bound (128 x 512 activations per tile on one SM).
 // |gelu_tanh - gelu_erf| <= 5e-4 absolute (at |x| ~ 2), below the bf16 rounding (2^-9 relative) the activation gets anyway;
-// the fp32 parity path keeps erff. MOCHA_TAIL_EXACT_GELU selects the erf polynomial here as well.
+// the fp32 parity path keeps erff.
 __device__ __forceinline__ float gelu_tanh_f(float x) {
   const float x2 = x * x;
   const float u = x * fmaf(0.0356774081f, x2, 0.7978845608f);
@@ -536,11 +520,7 @@ tail_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CU
             for (int i = 0; i < 32; ++i) f[i] = fmaxf(f[i], 0.f);
           } else if (p.act == ACT_GELU) {
 #pragma unroll
-#ifdef MOCHA_TAIL_EXACT_GELU
-            for (int i = 0; i < 32; ++i) f[i] = gelu_fast_f(f[i]);
-#else
             for (int i = 0; i < 32; ++i) f[i] = gelu_tanh_f(f[i]);
-#endif
           } else if (p.act == ACT_LRELU) {
 #pragma unroll
             for (int i = 0; i < 32; ++i) f[i] = lrelu02(f[i]);

@@ -12,7 +12,6 @@
 // Operands are K-major bf16: A tile 128 x 64, B tile BN x 64, both landing in the canonical
 // SWIZZLE_128B layout the UMMA shared-memory descriptors describe (8-row groups 1024 B apart).
 #include <cuda.h>
-#include <cstdlib>
 
 #include "gemm_tc.cuh"
 
@@ -30,14 +29,10 @@ constexpr int BLOCK_M = 128;
 constexpr int BLOCK_K = 64;  // 64 bf16 = 128 B = one swizzle atom row
 constexpr int UMMA_K = 16;
 // Warp roles. Ten warps put three warps on one scheduler partition (16 K registers each), which caps every thread at
-// 168 registers and made the epilogue spill. Default: twelve warps in three warpgroups - warps 0-3 are the producer
-// group (TMA warp, MMA warp, two idle warps) and shrink to TC_REGS_PRODUCER with setmaxnreg, warps 4-11 (the epilogue)
-// grow to TC_REGS_EPI. -DMOCHA_TC_TEN_WARPS restores the ten-warp layout.
-#ifdef MOCHA_TC_TEN_WARPS
-constexpr int TC_EPI_WARP0 = 2;
-#else
+// 168 registers and made the epilogue spill. Twelve warps in three warpgroups: warps 0-3 are the producer group (TMA
+// warp, MMA warp, two idle warps) and shrink to TC_REGS_PRODUCER with setmaxnreg, warps 4-11 (the epilogue) grow to
+// TC_REGS_EPI.
 constexpr int TC_EPI_WARP0 = 4;
-#endif
 constexpr int TC_THREADS = TC_EPI_WARP0 * 32 + 8 * 32;
 constexpr int TC_REGS_PRODUCER = 88, TC_REGS_EPI = 208;   // 4 x 88 + 8 x 208 = 2016 = the 12 x 168 registers per lane slot the launch allocates
 constexpr int A_STAGE_BYTES = BLOCK_M * BLOCK_K * 2;
@@ -155,49 +150,6 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
         "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
         "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
         "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-      : "r"(taddr)
-      : "memory");
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-// Split form for software-pipelined epilogues: issue the load of the NEXT chunk, work on the current one, then wait.
-// tmem_ld32_wait names the destination registers as in/out operands, so no use of them can be scheduled above the wait.
-__device__ __forceinline__ void tmem_ld32_issue(uint32_t taddr, uint32_t (&v)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-        "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]),
-        "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]),
-        "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-      : "r"(taddr)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_ld32_wait(uint32_t (&v)[32]) {
-  asm volatile("tcgen05.wait::ld.sync.aligned;"
-               : "+r"(v[0]), "+r"(v[1]), "+r"(v[2]), "+r"(v[3]), "+r"(v[4]), "+r"(v[5]), "+r"(v[6]), "+r"(v[7]), "+r"(v[8]),
-                 "+r"(v[9]), "+r"(v[10]), "+r"(v[11]), "+r"(v[12]), "+r"(v[13]), "+r"(v[14]), "+r"(v[15]), "+r"(v[16]),
-                 "+r"(v[17]), "+r"(v[18]), "+r"(v[19]), "+r"(v[20]), "+r"(v[21]), "+r"(v[22]), "+r"(v[23]), "+r"(v[24]),
-                 "+r"(v[25]), "+r"(v[26]), "+r"(v[27]), "+r"(v[28]), "+r"(v[29]), "+r"(v[30]), "+r"(v[31])
-               :
-               : "memory");
-}
-// lane = row of the accumulator, 64 consecutive fp32 columns in one instruction (the 64-column epilogue step)
-__device__ __forceinline__ void tmem_ld64(uint32_t taddr, uint32_t (&v)[64]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x64.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, "
-      "%32, %33, %34, %35, %36, %37, %38, %39, %40, %41, %42, %43, %44, %45, %46, %47, "
-      "%48, %49, %50, %51, %52, %53, %54, %55, %56, %57, %58, %59, %60, %61, %62, %63}, [%64];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-        "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]),
-        "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]),
-        "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31]), "=r"(v[32]),
-        "=r"(v[33]), "=r"(v[34]), "=r"(v[35]), "=r"(v[36]), "=r"(v[37]), "=r"(v[38]), "=r"(v[39]), "=r"(v[40]),
-        "=r"(v[41]), "=r"(v[42]), "=r"(v[43]), "=r"(v[44]), "=r"(v[45]), "=r"(v[46]), "=r"(v[47]), "=r"(v[48]),
-        "=r"(v[49]), "=r"(v[50]), "=r"(v[51]), "=r"(v[52]), "=r"(v[53]), "=r"(v[54]), "=r"(v[55]), "=r"(v[56]),
-        "=r"(v[57]), "=r"(v[58]), "=r"(v[59]), "=r"(v[60]), "=r"(v[61]), "=r"(v[62]), "=r"(v[63])
       : "r"(taddr)
       : "memory");
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
@@ -443,7 +395,6 @@ struct LinearEpiT : LinearEpiData {
     uint32_t par;     // MODE 4: which of the two staging boxes the next chunk fills
   };
   static constexpr bool kM1 = MODE == 1 || MODE == 4;   // single-output TMA-store epilogue
-  static constexpr bool kWide64 = MODE == 4;            // has the 64-column step (chunk64) for bf16-only wide boxes
   static constexpr bool kDouble = MODE == 4;
   // per warp: 4 KB fp32 box [32][128 B] (128 B-swizzled, 1 KB aligned) + 2 KB bf16 box [32][64 B]
   // (64 B-swizzled) + 4 KB residual box (128 B-swizzled); the LSU path uses a [32][EPI_LD] float
@@ -789,67 +740,6 @@ struct LinearEpiT : LinearEpiData {
     EPI_DBG(13);
   }
 
-  // -DMOCHA_TC_WIDE64 (opt-in, measured NEGATIVE: 1.127 -> 1.138 ms/step at 128 clips, same-box A/B): 64-column step of the
-  // bf16-only wide-box path (MODE 4, c16_wide): ONE tcgen05.ld.x64 and one dependent chain - bias, activation, eight 16-byte
-  // staging stores, fence, one TMA store of the 128-byte-row box - per 64 columns instead of two chains of 32. Coarser steps
-  // lose more overlap between the warps of a scheduler than the saved load / fence latency gains.
-  __device__ __forceinline__ bool wide64() const { return kWide64 && c16_wide && !C && (bias_period == 0 || !bias); }
-  template <int ACT>
-  __device__ __forceinline__ void drain_tma64(State& st, const EpiCtx& e, int col0, const uint32_t (&v)[64]) const {
-    float f[64];
-#pragma unroll
-    for (int j = 0; j < 64; ++j) f[j] = __uint_as_float(v[j]);
-    if (row_scale) {
-      const float rs = st.rs;
-#pragma unroll
-      for (int j = 0; j < 64; ++j) f[j] *= rs;
-    }
-    if (bias) {
-      const uint32_t bs = e.bias_smem + (uint32_t)(col0 * 4);
-#pragma unroll
-      for (int j = 0; j < 16; ++j) {
-        const float4 b4 = lds128(bs + 16u * j);   // same address in every lane: broadcast
-        f[4 * j] += b4.x; f[4 * j + 1] += b4.y; f[4 * j + 2] += b4.z; f[4 * j + 3] += b4.w;
-      }
-    }
-    if (ACT != ACT_NONE) {
-#pragma unroll
-      for (int j = 0; j < 64; ++j) f[j] = act_fn<ACT>(f[j]);
-    }
-    const uint32_t sbuf = e.stage + (kDouble ? st.par * 4096u : 0u);
-    if (e.lane == 0) { if (kDouble) bulk_wait_read1(); else bulk_wait_read0(); }
-    __syncwarp();
-    const int sw = e.lane & 7;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      uint32_t pk[4];
-#pragma unroll
-      for (int t = 0; t < 4; ++t) {
-        float a = f[8 * j + 2 * t], b = f[8 * j + 2 * t + 1];
-        if (c16_lrelu) { a = lrelu02(a); b = lrelu02(b); }
-        __nv_bfloat162 h2 = __floats2bfloat162_rn(a, b);
-        pk[t] = *reinterpret_cast<uint32_t*>(&h2);
-      }
-      sts128(sbuf + (uint32_t)(e.lane * 128 + ((j ^ sw) << 4)), pk[0], pk[1], pk[2], pk[3]);
-    }
-    fence_async_smem();
-    __syncwarp();
-    if (e.lane == 0) {
-      tma_store_3d(&tmC16w, sbuf, col0 + e.col_off, e.row0_in_img, e.img);
-      bulk_commit();
-    }
-    if (kDouble) st.par ^= 1u;
-  }
-  __device__ __forceinline__ void chunk64(State& st, const EpiCtx& e, int col0, const uint32_t (&v)[64]) const {
-    if (col0 >= N || e.slab_rows <= 0) return;
-    switch (act) {
-      case ACT_RELU: drain_tma64<ACT_RELU>(st, e, col0, v); break;
-      case ACT_GELU: drain_tma64<ACT_GELU>(st, e, col0, v); break;
-      case ACT_LRELU: drain_tma64<ACT_LRELU>(st, e, col0, v); break;
-      default: drain_tma64<ACT_NONE>(st, e, col0, v); break;
-    }
-  }
-
   // Residual GEMMs (x + f(x) feeding both an fp32 stream and a bf16 operand): the residual box is
   // TMA-prefetched one chunk ahead into a 128 B-swizzled buffer, so everything stays in the lane = row
   // layout of tcgen05.ld: v = act(v + bias) + res, fp32 box and 64 B-swizzled bf16 box, TMA stores.
@@ -1031,7 +921,6 @@ struct SoftmaxEpi {
   static constexpr uint64_t kHintA = 0, kHintB = 0;
   static constexpr bool kTf32 = false;
   static constexpr bool kWholeTile = true;
-  static constexpr bool kWide64 = false;
   __device__ __forceinline__ void unit_begin(State&) const {}
   __device__ __forceinline__ void kernel_begin(State&, const EpiCtx&) const {}
   __device__ __forceinline__ void tile_begin(State&, const EpiCtx&, int, int) const {}
@@ -1114,7 +1003,6 @@ struct MatchEpi {
   static constexpr int kWarpStageBytes = 0;
   static constexpr int kStageBytes = 0;
   static constexpr bool kWholeTile = false;
-  static constexpr bool kWide64 = false;
   // query tiles are re-read for every DB tile: keep them in L2; DB rows stream through once per group
   static constexpr uint64_t kHintA = L2_EVICT_LAST, kHintB = L2_EVICT_FIRST;
   struct State {
@@ -1202,14 +1090,10 @@ struct HaloSmem {
 // Register re-partition between the producer warpgroup and the two epilogue warpgroups (see TC_EPI_WARP0): warpgroup-
 // uniform, executed by every warp of the CTA once the prologue is done.
 __device__ __forceinline__ void tc_regs_producer() {
-#ifndef MOCHA_TC_TEN_WARPS
   asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(TC_REGS_PRODUCER));
-#endif
 }
 __device__ __forceinline__ void tc_regs_epilogue() {
-#ifndef MOCHA_TC_TEN_WARPS
   asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(TC_REGS_EPI));
-#endif
 }
 
 template <int BN, class Epi, bool HALO = false>
@@ -1508,22 +1392,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 #else
         const int c_stop = c_end;
 #endif
-#if defined(MOCHA_TC_WIDE64) && !defined(MOCHA_TC_TEN_WARPS) && !defined(MOCHA_TRACE)
-        bool done64 = false;
-        if constexpr (Epi::kWide64 && !HALO && BN >= 128) {
-          if (epi.wide64()) {   // bf16-only wide boxes: the warp's share (BN / 2 columns) goes out in 64-column steps
-#pragma unroll 1
-            for (int c0 = c_begin; c0 < c_stop; c0 += 64) {
-              uint32_t v64[64];
-              tmem_ld64(taddr + (uint32_t)c0, v64);
-              epi.chunk64(st, ectx, nt * BN + c0, v64);
-            }
-            done64 = true;
-          }
-        }
-        if (!done64)
-#endif
-#if !defined(MOCHA_TC_LD_PIPELINE) || defined(MOCHA_TC_TEN_WARPS) || defined(MOCHA_TRACE)
 #pragma unroll 1
         for (int c0 = c_begin; c0 < (Epi::kWholeTile ? c_begin : c_stop); c0 += 32) {
           uint32_t v[32];
@@ -1537,24 +1405,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           if (warp == TC_EPI_WARP0 && lane == 0 && trace_tile == 0 && c0 == c_begin + 32) TC_TRACE(28, (unsigned long long)clock64());
 #endif
         }
-#else
-        // -DMOCHA_TC_LD_PIPELINE (opt-in, measured NEGATIVE: 1.140 -> 1.156 ms/step at 128 clips, same-box A/B): two chunks in
-        // registers, the TMEM load of chunk i + 1 in flight while chunk i goes through bias / activation / staging / TMA
-        // store. The 260-cycle load was already covered by the lane quarter's partner warp; the extra live chunk costs more.
-        if (!Epi::kWholeTile && c_begin < c_stop) {
-          uint32_t vn[32];
-          tmem_ld32_issue(taddr + (uint32_t)c_begin, vn);
-#pragma unroll 1
-          for (int c0 = c_begin; c0 < c_stop; c0 += 32) {
-            tmem_ld32_wait(vn);
-            uint32_t v[32];
-#pragma unroll
-            for (int j = 0; j < 32; ++j) v[j] = vn[j];
-            if (c0 + 32 < c_stop) tmem_ld32_issue(taddr + (uint32_t)(c0 + 32), vn);
-            epi.chunk(st, ectx, row, row_ok, nt * BN + c0, v, c0 + 32 < c_end ? nt * BN + c0 + 32 : -1);
-          }
-        }
-#endif
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(&tempty_bar[as]);
@@ -1582,8 +1432,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 }
 
 // ------------------------------------------------------------------------------------------------
-// 2-CTA matcher kernel: a thread-block cluster of two CTAs (one TPC) computes a 256 x 256 tile with
-// tcgen05.mma.cta_group::2. Each CTA stages its own 128 query rows (A) and HALF of the DB rows (B)
+// CTA-pair GEMM kernel: a thread-block cluster of two CTAs (one TPC) computes a 256 x 256 tile with
+// tcgen05.mma.cta_group::2. Each CTA stages its own 128 activation rows (A) and HALF of the weight rows (B)
 // per k-block, so the shared-memory fill and operand-read traffic per SM drop by 1/3 and 1/3 vs the
 // 1-CTA kernel; the leader CTA's single MMA thread issues for the pair, tcgen05.commit multicasts the
 // "slot free" / "accumulator ready" signals to both CTAs, and each CTA's epilogue warps drain their
@@ -1663,8 +1513,6 @@ tc_gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   using SM = PairSmem<Epi::kStageBytes>;
   constexpr int STAGES = SM::STAGES;
   constexpr int BN = M2_BN;
-  constexpr uint64_t kPolA = Epi::kHintA ? Epi::kHintA : L2_EVICT_NORMAL;
-  constexpr uint64_t kPolB = Epi::kHintB ? Epi::kHintB : L2_EVICT_NORMAL;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   uint8_t* epi_stage = smem + STAGES * M2_STAGE_BYTES;
@@ -1722,8 +1570,8 @@ tc_gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
             uint8_t* sb = sa + A_STAGE_BYTES;
             if (rank == 0) mbar_expect_tx(&full_bar[stage], 2 * M2_STAGE_BYTES);
             const int tap = kb / sh.kb_per_tap, kc = kb - tap * sh.kb_per_tap;
-            tma_load_2d_pair(sa, &tmA, &full_bar[stage], kc * BLOCK_K, (int)(a_row0 + (long long)tap * sh.tap_row_stride), kPolA);
-            tma_load_2d_pair(sb, &tmB, &full_bar[stage], kb * BLOCK_K, b_row0, kPolB);
+            tma_load_2d_pair(sa, &tmA, &full_bar[stage], kc * BLOCK_K, (int)(a_row0 + (long long)tap * sh.tap_row_stride), L2_EVICT_NORMAL);
+            tma_load_2d_pair(sb, &tmB, &full_bar[stage], kb * BLOCK_K, b_row0, L2_EVICT_NORMAL);
             if (rank != 0) mbar_arrive_remote(&full_bar[stage], 0);
             if (++stage == STAGES) { stage = 0; phase ^= 1; }
           }
@@ -1922,8 +1770,6 @@ int setup_out_tma(LinearEpi& epi, unsigned long long rows_per_img, unsigned long
                   unsigned long long img_pitch_rows = 0) {
   epi.tma = 0;
   if (cols == 0) cols = (unsigned long long)epi.N;
-  static const bool off = getenv("MOCHA_NO_TMA_STORE") != nullptr;  // debugging aid: force the LSU epilogue
-  if (off) return MOCHA_OK;
   const bool ok = (epi.N % 4) == 0 && (epi.ldc % 8) == 0 && (epi.N <= 2048 || !epi.bias || epi.bias_period > 0) &&
                   ((reinterpret_cast<uintptr_t>(epi.C) | reinterpret_cast<uintptr_t>(epi.C16) |
                     reinterpret_cast<uintptr_t>(epi.res) | reinterpret_cast<uintptr_t>(epi.bias)) & 15) == 0;
@@ -2005,11 +1851,6 @@ int launch_pair(const CUtensorMap& tmA, const CUtensorMap& tmB, const TcShape& s
   count_launch();
   MOCHA_LAUNCH_CHECK("tc_gemm2_kernel");
   return MOCHA_OK;
-}
-template <int KC>
-int launch_match2(const CUtensorMap& tmA, const CUtensorMap& tmB, const TcShape& sh, int num_kb, const MatchEpi<KC>& epi,
-                  cudaStream_t s) {
-  return launch_pair(tmA, tmB, sh, num_kb, epi, s);
 }
 
 __global__ void cast_act_bf16_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ y, long long n,
@@ -2096,8 +1937,6 @@ std::mutex g_blob_mutex;
 // k_blocks > 0 lets long-K problems keep 256-wide tiles below one wave: a 128-wide tile needs twice the
 // shared-memory fill per MMA (fill-bound at ~64 B/clk/SM), measured 16.3 -> 12.0 us on 11520 x 256 x 1024
 int pick_bn(long long tiles_m, int N, int k_blocks = 0) {
-  static const int forced = getenv("MOCHA_FORCE_BN") ? atoi(getenv("MOCHA_FORCE_BN")) : 0;  // tuning aid
-  if (forced == 32 || forced == 64 || forced == 128 || forced == 256) return forced;
   // largest BN that still gives about one wave of CTAs; tiles that would be mostly padding are skipped
   if (k_blocks >= 8 && N >= 256 && tiles_m * ((N + 255) / 256) * 2 >= num_sms()) return 256;
   const int cands[4] = {256, 128, 64, 32};
@@ -2209,11 +2048,8 @@ const __nv_bfloat16* tc_lookup_bf16(const float* W) {
 
 namespace {
 // plain / image-batched linear layers on the CTA-pair kernel: single TMA-stored output, whole 256-wide n-tiles
-bool pair_linear_wanted(const LinearEpi& epi, int rows_per_img, int nb, int N, int bias_period) {
-  static const bool off = getenv("MOCHA_NO_PAIR_LINEAR") != nullptr;
-  static const bool no_periodic = getenv("MOCHA_NO_PAIR_PERIODIC_BIAS") != nullptr;   // A/B switch: bias tables [period, N] (-7 us)
-  return !off && epi.tma == 1 && N % 256 == 0 && (bias_period == 0 || !no_periodic) &&
-         (long long)ceil_div(rows_per_img, 256) * nb * (N / 256) >= num_sms() / 4;
+bool pair_linear_wanted(const LinearEpi& epi, int rows_per_img, int nb, int N) {
+  return epi.tma == 1 && N % 256 == 0 && (long long)ceil_div(rows_per_img, 256) * nb * (N / 256) >= num_sms() / 4;
 }
 TcShape pair_shape(const TcShape& sh, int rows_per_img, int nb, int N) {
   TcShape sp = sh;
@@ -2248,8 +2084,7 @@ int tc_linear_bf16(const __nv_bfloat16* A16, int lda, const __nv_bfloat16* W16, 
   // CTA pairs (256 x 256 pair tiles, each CTA stages half of the weight rows) for the plain projections too: a 128 x 256 tile
   // of a K = 256 layer pulls 192 KB of operands per CTA from L2, a pair tile 128 KB, and these short-K launches turned out to
   // be sensitive to exactly that (same-box A/B: -15 us per step; 128-wide tiles, which re-read A twice as often: +28 us).
-  // MOCHA_NO_PAIR_LINEAR=1 keeps the 1-CTA kernel.
-  if (pair_linear_wanted(epi, M, 1, N, bias_period)) {
+  if (pair_linear_wanted(epi, M, 1, N)) {
     CUtensorMap tmB;
     MOCHA_TRY(make_tmap(&tmB, W16, (unsigned long long)N, (unsigned long long)K, 128));
     return launch_pair(tmA, tmB, pair_shape(sh, M, 1, N), ceil_div(K, BLOCK_K), LinearEpiT<1>{epi}, s);
@@ -2279,8 +2114,7 @@ int tc_linear_bf16_img(const __nv_bfloat16* A16, int lda, const __nv_bfloat16* W
   LinearEpi epi{out.f32, N, N, bias, 0, nullptr, act, out.bf16, out.lrelu};
   MOCHA_TRY(setup_out_tma(epi, (unsigned long long)rows_per_img, (unsigned long long)nb, 0, (unsigned long long)out_img_pitch_rows));
   if (epi.tma != 1) return set_error(MOCHA_ERR_ARG, "tc_linear_img: output is not TMA-storable");
-  static const bool no_pair_img = getenv("MOCHA_NO_PAIR_IMG") != nullptr;   // A/B switch (-9.5 us per step with the pair kernel)
-  if (!no_pair_img && pair_linear_wanted(epi, rows_per_img, nb, N, 0)) {
+  if (pair_linear_wanted(epi, rows_per_img, nb, N)) {
     CUtensorMap tmB;
     MOCHA_TRY(make_tmap(&tmB, W16, (unsigned long long)N, (unsigned long long)K, 128));
     return launch_pair(tmA, tmB, pair_shape(sh, rows_per_img, nb, N), ceil_div(K, BLOCK_K), LinearEpiT<1>{epi}, s);
@@ -2311,8 +2145,7 @@ int tc_linear_bf16_grouped(const __nv_bfloat16* A16, const __nv_bfloat16* W16, _
   LinearEpi epi{nullptr, N, N, nullptr, 0, nullptr, ACT_NONE, out16, 0};
   MOCHA_TRY(setup_out_tma(epi, (unsigned long long)R, (unsigned long long)nb));
   if (epi.tma != 1) return set_error(MOCHA_ERR_ARG, "tc_linear_grouped: output is not TMA-storable");
-  static const bool no_pair_grp = getenv("MOCHA_NO_PAIR_GROUPED") != nullptr;   // A/B switch (-6.7 us per step with the pair kernel)
-  if (!no_pair_grp && pair_linear_wanted(epi, R, nb, N, 0)) {
+  if (pair_linear_wanted(epi, R, nb, N)) {
     CUtensorMap tmB;
     MOCHA_TRY(make_tmap(&tmB, W16, (unsigned long long)nb * N, (unsigned long long)K, 128));
     return launch_pair(tmA, tmB, pair_shape(sh, R, nb, N), ceil_div(K, BLOCK_K), LinearEpiT<1>{epi}, s);   // sh.H = 1: per-image weights
@@ -2583,13 +2416,11 @@ int tc_tconv_ex(const float* X, const __nv_bfloat16* Xh, const float* W, const f
   int rc = MOCHA_OK;
   // long-K, wide-N convolutions are bound by the shared-memory fill rate (~64 B/clk/SM) with 128 x 256
   // tiles: a CTA pair (cta_group::2) stages half of the weight rows each and runs 256 x 256 tiles
-  static const bool no_pair = getenv("MOCHA_NO_PAIR_GEMM") != nullptr;
   const int pair_tiles = ceil_div(T * V, 256) * B;
   // images shorter than a pair tile (BodyBlock convs: 90 rows per clip) would run 256-row tiles that are mostly padding:
-  // those keep the 1-CTA kernel's 128-row tiles (MOCHA_PAIR_SHORT_IMAGES=1 restores the pair kernel for them)
-  static const bool pair_short = getenv("MOCHA_PAIR_SHORT_IMAGES") != nullptr;
-  const bool pair_fill_ok = pair_short || ceil_div(T * V, 256) * 256 <= ceil_div(T * V, BLOCK_M) * BLOCK_M;
-  if (!no_pair && pair_fill_ok && epi.tma == 1 && Cout % 256 == 0 && taps * sh.kb_per_tap >= 8 && pair_tiles >= num_sms() / 2) {
+  // those keep the 1-CTA kernel's 128-row tiles
+  const bool pair_fill_ok = ceil_div(T * V, 256) * 256 <= ceil_div(T * V, BLOCK_M) * BLOCK_M;
+  if (pair_fill_ok && epi.tma == 1 && Cout % 256 == 0 && taps * sh.kb_per_tap >= 8 && pair_tiles >= num_sms() / 2) {
     CUtensorMap tmB;
     MOCHA_TRY(make_tmap(&tmB, W16, (unsigned long long)Cout, (unsigned long long)taps * Cin, 128));
     TcShape sp = sh;
@@ -2606,9 +2437,8 @@ int tc_tconv_ex(const float* X, const __nv_bfloat16* Xh, const float* W, const f
     return rc;
   }
   // 64 -> 64 channels, 5 taps, 24 rows per frame (to_mot's JointBlock conv): one 224-row box per tile serves all taps and the
-  // weights stay resident (halo variant; MOCHA_NO_HALO_TCONV=1 keeps the general kernel)
-  static const bool no_halo = getenv("MOCHA_NO_HALO_TCONV") != nullptr;
-  if (!no_halo && epi.tma == 1 && !epi.C && epi.C16 && Cin == BLOCK_K && Cout == 64 && taps == HALO_TAPS && V == HALO_SHIFT &&
+  // weights stay resident (halo variant)
+  if (epi.tma == 1 && !epi.C && epi.C16 && Cin == BLOCK_K && Cout == 64 && taps == HALO_TAPS && V == HALO_SHIFT &&
       bias_period == 0 && sh.tiles_m_total >= num_sms()) {
     CUtensorMap tmAh, tmB;
     MOCHA_TRY(make_tmap(&tmAh, X16c, (unsigned long long)B * Tp * V, (unsigned long long)Cin, HALO_ROWS));
@@ -2964,39 +2794,6 @@ int tc_match_splits(int nq, long long N) {
   return (int)splits * 2;  // x2: the two column halves of a tile keep separate lists
 }
 
-// 2-CTA (cta_group::2) variant of the coarse pass: 256 x 256 pair tiles
-int tc_match_coarse_pair(const __nv_bfloat16* Q16, int nq, const __nv_bfloat16* DB16, const float* dbnorm, long long N,
-                         int D, int kc, float* cand_score, int32_t* cand_idx, cudaStream_t s) {
-  CUtensorMap tmA, tmB;
-  MOCHA_TRY(make_tmap(&tmA, Q16, (unsigned long long)nq, (unsigned long long)D, 128));
-  MOCHA_TRY(make_tmap(&tmB, DB16, (unsigned long long)N, (unsigned long long)D, 128));
-  TcShape sh{};
-  sh.nb = 1;
-  sh.rows_out_per_b = nq;
-  sh.tiles_m_per_b = ceil_div(nq, 256);
-  sh.tiles_m_total = sh.tiles_m_per_b;
-  sh.src_rows_per_b = nq;
-  sh.taps = 1;
-  sh.kb_per_tap = ceil_div(D, BLOCK_K);
-  sh.tiles_n = (int)((N + M2_BN - 1) / M2_BN);
-  const int splits = tc_match_splits(nq, N) / 2;
-  sh.tiles_per_unit = ceil_div(sh.tiles_n, splits);
-  sh.units = sh.tiles_m_total * splits;
-  sh.splits = splits;
-  {
-    long long gm = (64LL << 20) / (256LL * D * 2);
-    if (gm < 1) gm = 1;
-    for (long long d = gm; d >= 1; --d)
-      if (sh.tiles_m_total % d == 0) { if (2 * d > gm) gm = d; break; }
-    if (const char* e = getenv("MOCHA_MATCH_GROUP_M")) gm = atoll(e);
-    sh.group_m = (int)(gm < 1 ? 1 : gm);
-  }
-  const int num_kb = ceil_div(D, BLOCK_K);
-  if (kc == 4) return launch_match2<4>(tmA, tmB, sh, num_kb, MatchEpi<4>{dbnorm, N, cand_score, cand_idx, 2 * splits}, s);
-  if (kc == 8) return launch_match2<8>(tmA, tmB, sh, num_kb, MatchEpi<8>{dbnorm, N, cand_score, cand_idx, 2 * splits}, s);
-  return launch_match2<16>(tmA, tmB, sh, num_kb, MatchEpi<16>{dbnorm, N, cand_score, cand_idx, 2 * splits}, s);
-}
-
 // fp32-storage variant: queries and DB rows stay fp32 in HBM and are consumed as TF32 by tcgen05
 // (kind::tf32, K = 8 per instruction; 32 elements per 128-byte k-block row)
 int tc_match_coarse_tf32(const float* Q, int nq, const float* DB, const float* dbnorm, long long N, int D, int kc,
@@ -3042,12 +2839,6 @@ int tc_match_coarse(const __nv_bfloat16* Q16, int nq, const __nv_bfloat16* DB16,
   MOCHA_CHECK_ARG(D >= BLOCK_K && D % 8 == 0, "tc_match_coarse: D=%d must be >= 64 and a multiple of 8", D);
   MOCHA_CHECK_ARG(kc == 4 || kc == 8 || kc == 16, "tc_match_coarse: kc must be 4, 8 or 16");
   constexpr int BN = 256;
-  static int use_pair = -1;
-  if (use_pair < 0) {
-    const char* e = getenv("MOCHA_MATCH_2CTA");
-    use_pair = e ? atoi(e) : 0;
-  }
-  if (use_pair && nq > BLOCK_M) return tc_match_coarse_pair(Q16, nq, DB16, dbnorm, N, D, kc, cand_score, cand_idx, s);
   CUtensorMap tmA, tmB;
   MOCHA_TRY(make_tmap(&tmA, Q16, (unsigned long long)nq, (unsigned long long)D, BLOCK_M));
   MOCHA_TRY(make_tmap(&tmB, DB16, (unsigned long long)N, (unsigned long long)D, BN));
@@ -3072,8 +2863,7 @@ int tc_match_coarse(const __nv_bfloat16* Q16, int nq, const __nv_bfloat16* DB16,
     // prefer a group size that divides the m-tile count (balanced groups measured ~10 % faster)
     for (long long d = gm; d >= 1; --d)
       if (sh.tiles_m_total % d == 0) { if (2 * d > gm) gm = d; break; }
-    if (const char* e = getenv("MOCHA_MATCH_GROUP_M")) gm = atoll(e);
-    sh.group_m = (int)(gm < 1 ? 1 : gm);
+    sh.group_m = (int)gm;
   }
   const int num_kb = ceil_div(D, BLOCK_K);
   if (kc == 4) return launch_tc<BN, MatchEpi<4>>(tmA, tmB, sh, num_kb, MatchEpi<4>{dbnorm, N, cand_score, cand_idx, 2 * splits}, s);
@@ -3107,8 +2897,7 @@ __global__ void splitk_reduce_kernel(const float* __restrict__ partial, int slic
 }  // namespace
 
 int tc_match_splitk_slices(int nq, long long N, int D) {
-  static const bool off = getenv("MOCHA_NO_SPLITK") != nullptr;
-  if (off || N > 8192 || D % 8 != 0) return 0;
+  if (N > 8192 || D % 8 != 0) return 0;
   const int num_kb = ceil_div(D, BLOCK_K);
   const long long units0 = (long long)ceil_div(nq, BLOCK_M) * ((N + 127) / 128);
   if (num_kb < 16 || units0 * 2 > num_sms()) return 0;

@@ -1091,15 +1091,14 @@ static unsigned fk_grid(long long F) {
 }
 
 // thread-per-skeleton streaming kernel for batches that fill the GPU (>= 4096 skeletons); the warp-per-skeleton kernel keeps
-// the small calls (a frame's clips), where parallelism inside the skeleton is all there is. MOCHA_NO_FK_ROWS=1 disables it.
+// the small calls (a frame's clips), where parallelism inside the skeleton is all there is.
 static bool fk_rows_wanted(long long F, int J, const void* a = nullptr, const void* b = nullptr, const void* c = nullptr,
                            const void* d = nullptr, const void* e = nullptr, const void* f = nullptr, const void* g = nullptr,
                            const void* h = nullptr) {
-  static const bool off = getenv("MOCHA_NO_FK_ROWS") != nullptr;
   const uintptr_t all = reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b) | reinterpret_cast<uintptr_t>(c) |
                         reinterpret_cast<uintptr_t>(d) | reinterpret_cast<uintptr_t>(e) | reinterpret_cast<uintptr_t>(f) |
                         reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(h);
-  return !off && F >= 4096 && J >= 1 && J <= MAXJ && (all & 15) == 0;   // bulk copies move 16-byte aligned slabs
+  return F >= 4096 && J >= 1 && J <= MAXJ && (all & 15) == 0;   // bulk copies move 16-byte aligned slabs
 }
 template <bool WITH_VEL, int WARPS>
 static int fk_rows_launch(const float* lrot, const float* lpos, const float* lvel, const float* lang, const int32_t* parents,
@@ -1181,9 +1180,8 @@ int post_frame_launch(const mocha_post_params* params, const float* Y, const flo
   }
   // steady state: the latency-shaped kernel (shared-memory structs, one load round); frame 0 and unaligned struct arrays
   // take the general kernel. A per-clip start row (start != NULL) takes the masked step kernel under the same rule.
-  static const bool no_step_kernel = getenv("MOCHA_NO_POST_STEP_KERNEL") != nullptr;
   const bool aligned = ((reinterpret_cast<uintptr_t>(state) | reinterpret_cast<uintptr_t>(out)) & 15) == 0;
-  const bool step_kernel = aligned && !no_step_kernel && V * Cin <= PF_YMAX;
+  const bool step_kernel = aligned && V * Cin <= PF_YMAX;
   if (start && step_kernel)
     launch_k(post_frame_step_kernel<true>, B, 32, 0, (cudaStream_t)stream, *params, Y, src_hips_vel, src_rvel, src_rang, contacts,
              start, T, V, Cin, state, out, hv_stride, rv_stride);

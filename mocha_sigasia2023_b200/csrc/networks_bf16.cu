@@ -5,8 +5,6 @@
 // a residual add, a normalisation or a SIMT kernel reads them. Same math as networks.cu (fp32 mode).
 #include "networks_bf16.cuh"
 
-#include <cstdlib>
-
 #include "fused.cuh"
 #include "gemm_f32.cuh"
 #include "gemm_tc.cuh"
@@ -35,7 +33,6 @@ struct Tc {
 struct SideStream {
   cudaStream_t stream = nullptr;
   cudaEvent_t fork = nullptr, join = nullptr;
-  cudaEvent_t ev[MOCHA_MAX_DEPTH] = {nullptr, nullptr, nullptr, nullptr};   // per-layer "ready" marks of side work
 };
 SideStream* side_stream() {
   // one set per (host thread, device): a stream belongs to the device that was current when it was created
@@ -49,7 +46,6 @@ SideStream* side_stream() {
     bool ok = cudaStreamCreateWithFlags(&ss.stream, cudaStreamNonBlocking) == cudaSuccess &&
               cudaEventCreateWithFlags(&ss.fork, cudaEventDisableTiming) == cudaSuccess &&
               cudaEventCreateWithFlags(&ss.join, cudaEventDisableTiming) == cudaSuccess;
-    for (int i = 0; i < MOCHA_MAX_DEPTH && ok; ++i) ok = cudaEventCreateWithFlags(&ss.ev[i], cudaEventDisableTiming) == cudaSuccess;
     if (!ok) {
       failed[dev] = true;
       (void)cudaGetLastError();
@@ -71,22 +67,15 @@ inline TcOut both(float* p, bf16* q) { return TcOut{p, q, 0}; }
 
 inline int ntok(const mocha_dims& d) { return (d.T / d.tp) * d.P; }
 
-// MOCHA_NO_FUSED_TAIL=1 keeps the unfused launch sequence (out-projection, LayerNorm, FFN GEMMs) for A/B runs
-inline bool use_fused_tail(int D) {
-  static const bool off = getenv("MOCHA_NO_FUSED_TAIL") != nullptr;
-  return !off && D == 256;
-}
+// the fused block tail (fused_tail.cu) is built for D = 256; other widths run the unfused launch sequence
+// (out-projection, LayerNorm, FFN GEMMs)
+inline bool use_fused_tail(int D) { return D == 256; }
 
 // Attention of the bf16 path: one fused launch (fused_attn.cu) when the geometry fits, else the two-launch sequence
-// (scores + softmax epilogue, P V) of gemm_tc.cu. MOCHA_NO_FUSED_ATTN=1 forces the latter (A/B runs).
-inline bool fused_attn_on() {
-  static const bool off = getenv("MOCHA_NO_FUSED_ATTN") != nullptr;
-  return !off;
-}
+// (scores + softmax epilogue, P V) of gemm_tc.cu.
 int attn(cudaStream_t s, Workspace& ws, const bf16* q, int ldq, const bf16* k, int ldk, const bf16* v, int ldv, int B, int H, int nq,
          int nkv, int dh, bf16* out, int ldo) {
-  const bool off = !fused_attn_on();
-  if (!off && tc_attn_fused_supported(nq, nkv, dh) && ldo == H * dh)
+  if (tc_attn_fused_supported(nq, nkv, dh) && ldo == H * dh)
     return tc_attn_fused(q, ldq, k, ldk, v, ldv, B, H, nq, nkv, dh, out, ldo, s);
   return tc_attention_ex(nullptr, q, ldq, nullptr, k, ldk, nullptr, v, ldv, B, H, nq, nkv, dh, nullptr, h16(out), ldo, ws, s);
 }
@@ -222,8 +211,7 @@ int decoder_bf16(const mocha_generator_weights* w, const float* src, const float
   WS_OK(ws, "mocha_decoder_fwd(bf16)");
   // layer-independent functions of the style tokens
   // AdaIN parameters of every layer depend on the style only: one launch for the token mean and all MLPs
-  static const bool no_style_mlp = getenv("MOCHA_NO_STYLE_MLP") != nullptr;
-  bool fused_style = !no_style_mlp && style_mlp_supported(d.D, d.dec_depth);
+  bool fused_style = style_mlp_supported(d.D, d.dec_depth);
   const bf16 *w1[MOCHA_MAX_DEPTH], *w2[MOCHA_MAX_DEPTH];
   const float *b1[MOCHA_MAX_DEPTH], *b2[MOCHA_MAX_DEPTH];
   for (int l = 0; l < d.dec_depth && fused_style; ++l) {
@@ -234,9 +222,8 @@ int decoder_bf16(const mocha_generator_weights* w, const float* src, const float
   }
   // The style MLP (128 blocks, L2-latency-bound) and the two token-wise passes over the style (instance norm, bf16 copy)
   // are independent: the latter run on a side stream that forks from and joins the caller's stream through events, so the
-  // fork is captured into a CUDA graph like any other dependency. MOCHA_NO_DECODER_FORK=1 keeps one stream.
-  static const bool no_fork = getenv("MOCHA_NO_DECODER_FORK") != nullptr;
-  SideStream* side = (!no_fork && fused_style) ? side_stream() : nullptr;
+  // fork is captured into a CUDA graph like any other dependency.
+  SideStream* side = fused_style ? side_stream() : nullptr;
   cudaStream_t s2 = s;
   if (side) {
     MOCHA_CUDA(cudaEventRecord(side->fork, s));
@@ -251,37 +238,7 @@ int decoder_bf16(const mocha_generator_weights* w, const float* src, const float
   }
   MOCHA_TRY(instance_norm_tokens(cha, B, n, d.D, eps, nullptr, nullptr, nullptr, nullptr, nullptr, s2, sty_in));
   MOCHA_TRY(tc_cast(cha, cha16, (long long)R * d.D, 0, s2));
-  // Keys and values of every layer are functions of the style only (k = to_k(IN(style)), v = to_v(style)), so the later
-  // layers' projections CAN run on the side stream while layer 0 is busy. Measured negative (same-box A/B at 128 clips:
-  // +4.5 us with layer 1 ahead, +6 us with both layers ahead): a second 148-CTA persistent GEMM competes with the
-  // critical path's GEMMs for whole SMs instead of filling the block tails' idle ones. Opt-in: MOCHA_DECODER_KV_AHEAD=1.
-  static const bool want_kv_ahead = getenv("MOCHA_DECODER_KV_AHEAD") != nullptr;
-  bool kv_ahead = side != nullptr && want_kv_ahead && inner % 64 == 0;
-  for (int l = 0; l < d.dec_depth && kv_ahead; ++l) {
-    const mocha_dec_layer& L = w->dec[l];
-    kv_ahead = L.wq && L.wk && L.wv && L.wk == L.wq + (size_t)inner * d.D && L.wv == L.wk + (size_t)inner * d.D &&
-               tc_lookup_bf16(L.wk) != nullptr;
-  }
-  bf16* kv_l[MOCHA_MAX_DEPTH] = {nullptr, nullptr, nullptr, nullptr};
-  if (kv_ahead) {
-    const size_t mark = ws.off;
-    for (int l = 0; l < d.dec_depth; ++l) {
-      kv_l[l] = l == 0 ? k : ws.take<bf16>((size_t)2 * R * inner);     // layer 0 uses the k | v part of qkv3
-      if (!kv_l[l]) { kv_ahead = false; break; }
-    }
-    if (!kv_ahead) { ws.off = mark; ws.overflow = false; }   // no room: fall back to the in-line grouped projection
-  }
-  if (kv_ahead) {
-    // layer 0 keeps its grouped q / k / v launch on the main stream (projecting its k / v on the side stream as well put two
-    // 148-CTA GEMMs in competition right on the critical path: +6 us); ev[0] marks the style operands as ready
-    MOCHA_CUDA(cudaEventRecord(side->ev[0], side->stream));
-    for (int l = 1; l < d.dec_depth; ++l) {
-      MOCHA_TRY(tc_linear_bf16_grouped(sty_in, tc_lookup_bf16(w->dec[l].wk), kv_l[l], 2, R, inner, d.D, s2));
-      MOCHA_CUDA(cudaEventRecord(side->ev[l], side->stream));
-    }
-    if (d.dec_depth == 1) kv_ahead = false;   // nothing to project ahead: plain fork / join
-    MOCHA_CUDA(cudaStreamWaitEvent(s, side->ev[0], 0));
-  } else if (side) {
+  if (side) {
     MOCHA_CUDA(cudaEventRecord(side->join, side->stream));
     MOCHA_CUDA(cudaStreamWaitEvent(s, side->join, 0));
   }
@@ -301,15 +258,8 @@ int decoder_bf16(const mocha_generator_weights* w, const float* src, const float
       MOCHA_TRY(instance_norm_tokens(x, B, n, d.D, eps, gb, x1, nullptr, nullptr, nullptr, s));
       MOCHA_TRY(instance_norm_tokens(x1, B, n, d.D, eps, nullptr, nullptr, nullptr, nullptr, nullptr, s, qin));
     }
-    static const bool no_group = getenv("MOCHA_NO_GROUPED_QKV") != nullptr;
     const bf16* wq16 = tc_lookup_bf16(L.wq);
-    const bf16 *kk = k, *vv = v;
-    if (kv_ahead && l >= 1) {
-      MOCHA_TRY(tc.lin(qin, d.D, L.wq, nullptr, 0, nullptr, h16(q), R, inner, d.D, ACT_NONE));
-      MOCHA_CUDA(cudaStreamWaitEvent(s, side->ev[l], 0));
-      kk = kv_l[l];
-      vv = kv_l[l] + (size_t)R * inner;
-    } else if (!no_group && wq16 && L.wk == L.wq + (size_t)inner * d.D && L.wv == L.wk + (size_t)inner * d.D && inner % 64 == 0) {
+    if (wq16 && L.wk == L.wq + (size_t)inner * d.D && L.wv == L.wk + (size_t)inner * d.D && inner % 64 == 0) {
       // to_q / to_k / to_v sit back to back in the packed blob: three inputs x three weights in one launch
       MOCHA_TRY(tc_linear_bf16_grouped(in3, wq16, qkv3, 3, R, inner, d.D, s));
     } else {
@@ -317,7 +267,7 @@ int decoder_bf16(const mocha_generator_weights* w, const float* src, const float
       MOCHA_TRY(tc.lin(sty_in, d.D, L.wk, nullptr, 0, nullptr, h16(k), R, inner, d.D, ACT_NONE));
       MOCHA_TRY(tc.lin(cha16, d.D, L.wv, nullptr, 0, nullptr, h16(v), R, inner, d.D, ACT_NONE));
     }
-    MOCHA_TRY(attn(s, ws, q, inner, kk, inner, vv, inner, B, d.heads, n, n, d.dec_dh, att, inner));
+    MOCHA_TRY(attn(s, ws, q, inner, k, inner, v, inner, B, d.heads, n, n, d.dec_dh, att, inner));
     float* dst = (l == d.dec_depth - 1) ? decoded : xb;
     if (use_fused_tail(d.D) && tc_tail_supported(R, inner, d.mlp)) {
       MOCHA_TRY(tail(s, att, inner, L.wo, L.bo, x1, nullptr, nullptr, d.mlp, ACT_GELU, L.w1, L.b1, L.w2, L.b2, nullptr, nullptr,
@@ -358,8 +308,7 @@ int to_mot_bf16(const mocha_generator_weights* w, const float* tokens, int B, fl
   MOCHA_TRY(graph_agg_kv_pad16(y3, w->tm_A2, gp16, B, Tp, d.tp, padj, d.P, d.V, d.C0, d.Kj, s));
   MOCHA_TRY(tc_tconv_ex(nullptr, gp16, w->tm_jb_tcn_w, w->tm_jb_tcn_b, 0, h16(y4, 1), B, d.T, d.V, d.C0, d.C0, d.taps_j, 1, ws, s, 1,
                         true));
-  static const bool no_out_conv = getenv("MOCHA_NO_OUT_CONV_KERNEL") != nullptr;
-  if (!no_out_conv && out_conv_affine_supported(d.C0, d.Cin) && (Y || Ytil))
+  if (out_conv_affine_supported(d.C0, d.Cin) && (Y || Ytil))
     return out_conv_affine(y4, w->tm_out_w, w->tm_out_b, Y_mean, Y_std, Ytil, Y, R, d.C0, d.Cin, d.V, s);
   MOCHA_TRY(tc.lin(y4, d.C0, w->tm_out_w, w->tm_out_b, 0, nullptr, f32(ytp), R, Cp, d.C0, ACT_NONE));
   if (Y || Ytil) MOCHA_TRY(affine_rows(ytp, Y_mean, Y_std, Y, R, d.Cin, d.V, s, Cp, Ytil));
@@ -385,11 +334,9 @@ int cvae_bf16(const mocha_cvae_weights* w, const float* cond, int B, int ncond, 
   bf16* mem = ws.take<bf16>((size_t)Rm * D);
   bf16* memkv = ws.take<bf16>((size_t)Rm * 2 * D);
   // memory K | V of the decoder layers after the first depend on `mem` only: they are projected on a side stream while
-  // layer 0 runs (its 90-CTA block tails leave 58 SMs idle) - MOCHA_NO_CVAE_FORK=1 keeps them in line
-  static const bool no_cvae_fork = getenv("MOCHA_NO_CVAE_FORK") != nullptr;
+  // layer 0 runs (its 90-CTA block tails leave 58 SMs idle)
   bf16* memkv_ahead[MOCHA_MAX_DEPTH] = {nullptr, nullptr, nullptr, nullptr};
-  if (!no_cvae_fork)
-    for (int l = 1; l < w->depth; ++l) memkv_ahead[l] = ws.take<bf16>((size_t)Rm * 2 * D);
+  for (int l = 1; l < w->depth; ++l) memkv_ahead[l] = ws.take<bf16>((size_t)Rm * 2 * D);
   bf16* dq = ws.take<bf16>((size_t)Rq * D);
   WS_OK(ws, "mocha_cvae_sample(bf16)");
 
@@ -409,10 +356,9 @@ int cvae_bf16(const mocha_cvae_weights* w, const float* cond, int B, int ncond, 
       float* xq = y;          // [2B, D] gathered rows of x (residual)
       bf16* xq16 = y16;
       bf16* kv = qkv;         // [Rp, 2D]
-      static const bool no_rows_kernel = getenv("MOCHA_NO_PRIOR_LAST_KERNEL") != nullptr;
       const bf16 *wq16 = tc_lookup_bf16(L.in_w), *wo16 = tc_lookup_bf16(L.out_w), *w116 = tc_lookup_bf16(L.l1_w),
                  *w216 = tc_lookup_bf16(L.l2_w);
-      if (!no_rows_kernel && cvae_prior_last_supported(D, H, w->dff, np) && wq16 && wo16 && w116 && w216 && L.n1_b && L.n2_b) {
+      if (cvae_prior_last_supported(D, H, w->dff, np) && wq16 && wo16 && w116 && w216 && L.n1_b && L.n2_b) {
         // everything after the K / V projection acts on 2 rows per clip: one SIMT launch (ops.cu)
         MOCHA_TRY(tc.lin(x16, D, L.in_w + (size_t)D * D, L.in_b + D, 0, nullptr, h16(kv), Rp, 2 * D, D, ACT_NONE));
         MOCHA_TRY(cvae_prior_last(x, B, np, kv, wq16, L.in_b, wo16, L.out_b, L.n1_g, L.n1_b, w116, L.l1_b, w216, L.l2_b, L.n2_g,
@@ -459,7 +405,7 @@ int cvae_bf16(const mocha_cvae_weights* w, const float* cond, int B, int ncond, 
     }
   }
   MOCHA_TRY(cvae_memory(x, prior_rows, eps, cond, nullptr, mu, logvar, B, ncond, D, s, mem));
-  SideStream* side = (!no_cvae_fork && w->depth > 1) ? side_stream() : nullptr;
+  SideStream* side = w->depth > 1 ? side_stream() : nullptr;
   bool ahead_pending = false;
   if (side) {
     MOCHA_CUDA(cudaEventRecord(side->fork, s));
@@ -487,9 +433,7 @@ int cvae_bf16(const mocha_cvae_weights* w, const float* cond, int B, int ncond, 
     // Layer 0 with both cached tables: the query rows are the same for every clip, so neither the broadcast [B, nq, D]
     // tensor nor its per-clip projection is materialised - the attention kernel reads the shared bf16 query table and the
     // block tail reads the fp32 table as a periodic residual.
-    static const bool no_shared_q = getenv("MOCHA_NO_SHARED_Q") != nullptr;
-    const bool shared_q = !no_shared_q && l == 0 && w->dec0_sa && w->dec0_q16 && fused && fused_attn_on() &&
-                          tc_attn_fused_supported(nq, nm, dh);
+    const bool shared_q = l == 0 && w->dec0_sa && w->dec0_q16 && fused && tc_attn_fused_supported(nq, nm, dh);
     const float* res_cross = dy;
     int res_period = 0;
     if (shared_q) {

@@ -1057,46 +1057,9 @@ __device__ __forceinline__ void warp_matvec2(const __nv_bfloat16* __restrict__ W
   }
 }
 
-// Two clips per block (opt-in: MOCHA_STYLE_MLP_TWO_CLIPS=1). With one clip per block the 128 blocks pull the same 1.5 MB of
-// weights from L2 each (197 MB in 26 us = 7.5 TB/s), so a weight row loaded once here serves two clips and the traffic halves.
-// Measured NEGATIVE in the frame (+2.8 us at 128 clips, same-box A/B): 64 blocks pull 1.5 MB each at the per-SM rate, which
-// takes as long as 128 blocks sharing the aggregate rate, and the launch overlaps the side stream's work either way.
-constexpr int STYLE2_THREADS = 512;
-__global__ void __launch_bounds__(STYLE2_THREADS, 1)
-style_mlp2_kernel(const float* __restrict__ cha, int n, const StyleMlpLayers L, int nlayers, float* __restrict__ gb, int B) {
-  constexpr int D = 256, NW = STYLE2_THREADS / 32;
-  pdl_trigger();
-  pdl_wait();
-  __shared__ __align__(16) float smean[2][D];
-  __shared__ __align__(16) float hid[2][2 * D];
-  const int b0 = 2 * blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  {
-    // token means: one thread per (clip, column), four independent partial sums (same pairing as style_mlp_kernel)
-    const int c = threadIdx.x & (D - 1), v = threadIdx.x >> 8;
-    const float* xb = cha + (long long)(b0 + v) * n * D + c;
-    float part[4];
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-      float s0 = 0.f, s1 = 0.f;
-      int i = q;
-      for (; i + 4 < n; i += 8) { s0 += xb[(long long)i * D]; s1 += xb[(long long)(i + 4) * D]; }
-      for (; i < n; i += 4) s0 += xb[(long long)i * D];
-      part[q] = s0 + s1;
-    }
-    smean[v][c] = ((part[0] + part[1]) + (part[2] + part[3])) / (float)n;
-  }
-  __syncthreads();
-  for (int l = 0; l < nlayers; ++l) {
-    warp_matvec2<1, 8, 2>(L.w1[l], L.b1[l], &smean[0][0], D, &hid[0][0], 2 * D, nullptr, 2 * D, 2, 1.f, warp, NW, lane);
-    __syncthreads();
-    warp_matvec2<2, 4, 2>(L.w2[l], L.b2[l], &hid[0][0], 2 * D, gb + ((long long)l * B + b0) * 2 * D, 2 * D, nullptr, 2 * D, 0, 1.f,
-                          warp, NW, lane);
-    __syncthreads();
-  }
-}
-
-// Two clips per CLUSTER of two CTAs (default for even batches >= 64): the launch above is bound by the aggregate L2 -> SM
-// bandwidth (128 blocks x 1.5 MB of the same weights), and two clips per block only moved the bound to the per-SM load rate.
+// Two clips per CLUSTER of two CTAs (for even batches >= 64): one clip per block (style_mlp_kernel) is bound by the aggregate
+// L2 -> SM bandwidth (128 blocks x 1.5 MB of the same weights), and two clips per block only moved the bound to the per-SM
+// load rate (measured slower in the frame).
 // Here CTA r of the pair owns HALF of every layer's output features for both clips: it reads half of each weight matrix
 // (768 KB per CTA, 98 MB per launch), writes its half of the hidden vector into both CTAs' shared memory (DSMEM stores) and,
 // after a cluster barrier, produces its half of gamma | beta. Same summation order per output as style_mlp_kernel.
@@ -1165,8 +1128,7 @@ __device__ __forceinline__ void ln2_rows256(const float* in, int ldi, const floa
 
 constexpr int PL_THREADS = 512;
 constexpr int PL_MAXKEYS = 256;
-constexpr int PL_SMEM_KEYS = 192;   // a clip's K | V rows (1 KB per key) are staged in shared memory up to this many keys
-template <int KCH2, bool KVS>   // dff / 256; K / V staged in shared memory
+template <int KCH2>   // dff / 256
 __global__ void __launch_bounds__(PL_THREADS, 1)
 cvae_prior_last_kernel(const float* __restrict__ x, int np, const __nv_bfloat16* __restrict__ kv, const PriorLastW W, int H,
                        float eps, float* __restrict__ out) {
@@ -1180,37 +1142,14 @@ cvae_prior_last_kernel(const float* __restrict__ x, int np, const __nv_bfloat16*
   float* hid = t1 + 2 * D;               // [2][DFF]
   float* part = hid + 2 * DFF;           // [4][2][D] partial P V sums
   float* sc = part + 8 * D;              // [2][H][PL_MAXKEYS] scores / probabilities
-  __nv_bfloat16* kvs = reinterpret_cast<__nv_bfloat16*>(sc + 2 * H * PL_MAXKEYS);   // [np][2D] (KVS only; 16 B aligned)
-  __shared__ __align__(8) unsigned long long kv_bar;
   const int b = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int dh = D / H, lph = dh / 8;    // lanes per head when a lane owns 8 consecutive columns
   const __nv_bfloat16* kb = kv + (long long)b * np * 2 * D;
-  const uint32_t bar_s = (uint32_t)__cvta_generic_to_shared(&kv_bar);
-  if (KVS && threadIdx.x == 0) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_s) : "memory");
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
   pdl_wait();
-  if (KVS && threadIdx.x == 0) {
-    // the clip's keys and values are one contiguous block: a single bulk copy, in flight during the q projection
-    const uint32_t bytes = (uint32_t)np * 2u * D * 2u;
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_s), "r"(bytes) : "memory");
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                     (uint32_t)__cvta_generic_to_shared(kvs)),
-                 "l"(kb), "r"(bytes), "r"(bar_s)
-                 : "memory");
-  }
   for (int i = threadIdx.x; i < 2 * D; i += PL_THREADS) xs[i] = x[(long long)b * np * D + i];   // tokens 0 and 1 are adjacent
   __syncthreads();
   warp_matvec2<1, 8, 2>(W.wq, W.bq, xs, D, qs, D, nullptr, D, 0, rsqrtf((float)dh), warp, NW, lane);
   __syncthreads();
-  if (KVS) {
-    uint32_t done = 0;
-    while (!done)
-      asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], 0;\nselp.u32 %0, 1, 0, p;\n}"
-                   : "=r"(done) : "r"(bar_s) : "memory");
-  }
-  const __nv_bfloat16* ksrc = KVS ? kvs : kb;
   {
     // scores: a warp per key, lane = 8 consecutive columns of the key row (one 512-byte row per load)
     float q0[8], q1[8];
@@ -1218,9 +1157,9 @@ cvae_prior_last_kernel(const float* __restrict__ x, int np, const __nv_bfloat16*
     for (int j = 0; j < 8; ++j) { q0[j] = qs[lane * 8 + j]; q1[j] = qs[D + lane * 8 + j]; }
     for (int j0 = warp; j0 < np; j0 += 2 * NW) {
       const int j1 = j0 + NW;
-      const uint4 k0 = *reinterpret_cast<const uint4*>(ksrc + (long long)j0 * 2 * D + lane * 8);
+      const uint4 k0 = *reinterpret_cast<const uint4*>(kb + (long long)j0 * 2 * D + lane * 8);
       uint4 k1 = make_uint4(0, 0, 0, 0);
-      if (j1 < np) k1 = *reinterpret_cast<const uint4*>(ksrc + (long long)j1 * 2 * D + lane * 8);
+      if (j1 < np) k1 = *reinterpret_cast<const uint4*>(kb + (long long)j1 * 2 * D + lane * 8);
       const uint32_t u0[4] = {k0.x, k0.y, k0.z, k0.w}, u1[4] = {k1.x, k1.y, k1.z, k1.w};
       float s00 = 0.f, s01 = 0.f, s10 = 0.f, s11 = 0.f;   // s[key][row]
 #pragma unroll
@@ -1262,7 +1201,7 @@ cvae_prior_last_kernel(const float* __restrict__ x, int np, const __nv_bfloat16*
   {
     // a = p v: thread = 2 columns x one of 4 key groups
     const int c2 = (threadIdx.x & 127) * 2, kg = threadIdx.x >> 7, h = c2 / dh;
-    const __nv_bfloat16* vb = ksrc + D + c2;
+    const __nv_bfloat16* vb = kb + D + c2;
     const float* p0 = sc + (0 * H + h) * PL_MAXKEYS;
     const float* p1 = sc + (1 * H + h) * PL_MAXKEYS;
     float a00 = 0.f, a01 = 0.f, a10 = 0.f, a11 = 0.f;   // a[row][column]
@@ -1745,8 +1684,7 @@ int embed_graph_agg(const float* X, const float* Wemb, const float* bemb, const 
   MOCHA_CHECK_ARG(Cin <= EMB_MAXCIN, "embed_graph_agg: Cin=%d > %d unsupported", Cin, EMB_MAXCIN);
   MOCHA_CHECK_ARG(V % 4 == 0 && V <= 32, "embed_graph_agg: V=%d must be a multiple of 4, at most 32", V);
   constexpr int G = 4;
-  static const bool no_mma = getenv("MOCHA_NO_MMA_EMBED") != nullptr;   // A/B switch: the sparse SIMT kernel below
-  if (!no_mma && V == 24 && Kk == 3 && C == 64 && ldo % 8 == 0 && ldo <= 512 &&
+  if (V == 24 && Kk == 3 && C == 64 && ldo % 8 == 0 && ldo <= 512 &&
       ((reinterpret_cast<uintptr_t>(out16) | reinterpret_cast<uintptr_t>(X)) & 15) == 0) {
     constexpr int XT = (G * 24 + 15) / 16;
     const size_t smem_mma = (size_t)(XT * 16 * EMB_XLD + G * 24 * EMB_HLD) * sizeof(float) + (size_t)G * 24 * (ldo + 8) * 2;
@@ -1949,8 +1887,7 @@ int graph_agg_kv_pad16(const float* in, const float* A2, __nv_bfloat16* out16, i
                       (C & 3) == 0 && Kk > 0 && (reinterpret_cast<uintptr_t>(in) & 15) == 0,
                   "graph_agg_kv_pad16: bad args");
   MOCHA_CHECK_ARG(tdiv + 2 * pad <= 16 && pad < Ts * tdiv, "graph_agg_kv_pad16: tdiv / pad too large");
-  static const bool no_stream = getenv("MOCHA_NO_STREAM_AGG") != nullptr;   // A/B switch: the list kernel below
-  if (!no_stream && Kk * U <= GKP_TERMS && Wn % 4 == 0 && Wn <= 32 && (reinterpret_cast<uintptr_t>(out16) & 7) == 0) {
+  if (Kk * U <= GKP_TERMS && Wn % 4 == 0 && Wn <= 32 && (reinterpret_cast<uintptr_t>(out16) & 7) == 0) {
     const long long total = (long long)B * Ts * (Wn / 4) * (C / 4);
     launch_k(graph_agg_kv_pad16_stream_kernel, blocks_for(total, 256), 256, 0, s, in, A2, out16, total, Ts, tdiv, pad, U, Wn, C / 4, Kk);
     count_launch();
@@ -1982,8 +1919,7 @@ int pool_graph_agg(const __nv_bfloat16* in, const float* Wp, const float* A, __n
   MOCHA_CHECK_ARG(P > 0 && P <= POOL_MAXP, "pool_graph_agg: P=%d unsupported (max %d)", P, POOL_MAXP);
   MOCHA_CHECK_ARG(tp > 0 && T % tp == 0, "pool_graph_agg: T=%d not a multiple of tp=%d", T, tp);
   const size_t smem = (size_t)(Kk * P * P + 2 * P * V + P) * sizeof(float);
-  static const bool no_v4 = getenv("MOCHA_NO_POOL_V4") != nullptr;   // A/B switch: the bf162 kernel below
-  if (!no_v4 && C % 4 == 0 && C / 4 <= 128 && 128 % (C / 4) == 0 && (reinterpret_cast<uintptr_t>(in) & 7) == 0 &&
+  if (C % 4 == 0 && C / 4 <= 128 && 128 % (C / 4) == 0 && (reinterpret_cast<uintptr_t>(in) & 7) == 0 &&
       (reinterpret_cast<uintptr_t>(out16) & 7) == 0) {
     const int groups = B * (T / tp), gpb = 128 / (C / 4);
     launch_k(pool_graph_agg_v4_kernel, (groups + gpb - 1) / gpb, 128, smem, s, in, Wp, A, out16, groups, T, V, P, C, tp, Kk);
@@ -2049,12 +1985,8 @@ int style_mlp(const float* cha, int B, int n, int D, int nlayers, const __nv_bfl
     MOCHA_CHECK_ARG(w1[l] && w2[l] && aligned16(w1[l]) && aligned16(w2[l]), "style_mlp: layer %d weights missing / unaligned", l);
     L.w1[l] = w1[l]; L.b1[l] = b1[l]; L.w2[l] = w2[l]; L.b2[l] = b2[l];
   }
-  static const bool two_clips = getenv("MOCHA_STYLE_MLP_TWO_CLIPS") != nullptr;   // opt-in (measured negative, see the kernel)
-  static const bool no_cluster = getenv("MOCHA_NO_STYLE_MLP_CLUSTER") != nullptr;  // A/B switch
-  if (!two_clips && !no_cluster && (B & 1) == 0 && B >= 64)
+  if ((B & 1) == 0 && B >= 64)
     launch_k(style_mlp_cluster_kernel, B, STYLEC_THREADS, 0, s, cha, n, L, nlayers, gb, B);
-  else if (two_clips && (B & 1) == 0 && B >= 64)
-    launch_k(style_mlp2_kernel, B / 2, STYLE2_THREADS, 0, s, cha, n, L, nlayers, gb, B);
   else
     launch_k(style_mlp_kernel, B, STYLE_THREADS, 0, s, cha, n, L, nlayers, gb, B);
   count_launch();
@@ -2077,13 +2009,7 @@ int cvae_prior_last(const float* x, int B, int np, const __nv_bfloat16* kv, cons
   MOCHA_CHECK_ARG(cvae_prior_last_supported(256, H, dff, np), "cvae_prior_last: unsupported geometry");
   MOCHA_CHECK_ARG(aligned16(kv) && aligned16(wq) && aligned16(wo) && aligned16(w1) && aligned16(w2), "cvae_prior_last: unaligned operand");
   PriorLastW W{wq, wo, w1, w2, bq, bo, b1, b2, g1, be1, g2, be2};
-  const size_t base = (size_t)(8 * 256 + 2 * dff + 8 * 256 + 2 * H * PL_MAXKEYS) * sizeof(float);
-  // staging the clip's K | V block in shared memory (one bulk copy) makes the kernel itself faster but costs more than it
-  // gains inside the frame: with ~215 KB of shared memory the block cannot become resident next to the previous GEMM's
-  // CTAs, so the programmatic-launch overlap of its prologue (and of the next kernel's) is lost. Opt-in for A/B runs.
-  static const bool want_kvs = getenv("MOCHA_PRIOR_LAST_KVS") != nullptr;
-  const bool kvs = want_kvs && np <= PL_SMEM_KEYS && base + (size_t)np * 1024 + 256 <= 220 * 1024;
-  const size_t smem = base + (kvs ? (size_t)np * 1024 : 0) + 128;
+  const size_t smem = (size_t)(8 * 256 + 2 * dff + 8 * 256 + 2 * H * PL_MAXKEYS) * sizeof(float) + 128;
   MOCHA_CHECK_ARG(smem <= 227 * 1024, "cvae_prior_last: too many heads");
   auto go = [&](auto kern) -> int {
     // (no cached flag: the variants share one function-pointer type, so a static here would be shared between them)
@@ -2091,15 +2017,9 @@ int cvae_prior_last(const float* x, int B, int np, const __nv_bfloat16* kv, cons
     launch_k(kern, B, PL_THREADS, smem, s, x, np, kv, W, H, eps, out);
     return MOCHA_OK;
   };
-  if (kvs) {
-    if (dff == 256) MOCHA_TRY(go(cvae_prior_last_kernel<1, true>));
-    else if (dff == 512) MOCHA_TRY(go(cvae_prior_last_kernel<2, true>));
-    else MOCHA_TRY(go(cvae_prior_last_kernel<4, true>));
-  } else {
-    if (dff == 256) MOCHA_TRY(go(cvae_prior_last_kernel<1, false>));
-    else if (dff == 512) MOCHA_TRY(go(cvae_prior_last_kernel<2, false>));
-    else MOCHA_TRY(go(cvae_prior_last_kernel<4, false>));
-  }
+  if (dff == 256) MOCHA_TRY(go(cvae_prior_last_kernel<1>));
+  else if (dff == 512) MOCHA_TRY(go(cvae_prior_last_kernel<2>));
+  else MOCHA_TRY(go(cvae_prior_last_kernel<4>));
   count_launch();
   MOCHA_LAUNCH_CHECK("cvae_prior_last");
   return MOCHA_OK;

@@ -9,8 +9,6 @@ from __future__ import annotations
 
 import ctypes as C
 
-import os
-
 import torch
 
 from . import _lib
@@ -80,12 +78,11 @@ def _gcn_first_aug(w: torch.Tensor, b: torch.Tensor, A: torch.Tensor) -> torch.T
     """W' of _gcn_first with K extra columns holding the per-partition biases b[k*Cout+co] (they multiply the
     adjacency column sums that the aggregation kernel appends to its rows), zero-padded to a multiple of 16 (one
     tcgen05 K step; the GEMM's 64-wide TMA boxes read past the last column and are zero-filled by the engine, so the
-    padding up to 64 costs no HBM traffic). MOCHA_GCN_KAUG_PAD=64 restores the dense multiple-of-64 layout."""
+    padding up to 64 costs no HBM traffic)."""
     K = A.shape[0]
     wp, _ = _gcn_first(w, b, A)
     co = wp.shape[0]
-    pad = int(os.environ.get("MOCHA_GCN_KAUG_PAD", "16"))
-    kaug = (wp.shape[1] + K + pad - 1) // pad * pad
+    kaug = (wp.shape[1] + K + 15) // 16 * 16
     out = torch.zeros((co, kaug), dtype=torch.float32)
     out[:, :wp.shape[1]] = wp
     out[:, wp.shape[1]:wp.shape[1] + K] = b.reshape(K, co).t()

@@ -9,7 +9,6 @@ whole step can be captured once into a CUDA graph (`capture()`) and replayed per
 from __future__ import annotations
 
 import ctypes as C
-import os
 from dataclasses import dataclass
 
 import numpy as np
@@ -165,7 +164,6 @@ class CharacterizationSession:
         # decode; in the steady state it is a side branch of the frame, so it runs on its own stream (own workspace)
         # concurrently with the CVAE / decoder chain and is joined at the end of the frame. Its kernels are small
         # (split-K coarse pass, re-rank) and fit next to the 90-CTA block tails.
-        self.match_async = os.environ.get("MOCHA_MATCH_ASYNC", "1") != "0"
         mbytes = max(self.lib.mocha_match_exact_workspace_bytes(B, self.tree.N, 1),
                      self.lib.mocha_match_tc_workspace_bytes(B, self.tree.N, self.tree.D, self.tree.kc))
         self.match_ws = [torch.empty(mbytes + 4096, dtype=torch.uint8, device=dev) for _ in self.parts]
@@ -253,18 +251,13 @@ class CharacterizationSession:
             self.bank.windows(self.start[sl], self.clip[sl], self.slot_clip[sl], self.slot_cursor[sl], self.X[sl],
                               self.side[sl], self.contacts[sl])
         self.encode(self.X[sl], self.tokens[sl], self.encoded[sl], self.cnt[sl], self.cnt_nm[sl], self.cnt_nm16[sl], ws)
-        side = None
-        if self.match_async:
-            k = next(i for i, pr in enumerate(self.parts) if pr[0] == lo)
-            side = self.match_streams[k]
-            side.wait_stream(torch.cuda.current_stream())
-            with torch.cuda.stream(side):
-                self._match(lo, hi, self.match_ws[k])
-        else:
-            self._match(lo, hi, ws)
+        k = next(i for i, pr in enumerate(self.parts) if pr[0] == lo)
+        side = self.match_streams[k]
+        side.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(side):
+            self._match(lo, hi, self.match_ws[k])
         self._cvae_step(lo, hi, ws)
-        if side is not None:
-            torch.cuda.current_stream().wait_stream(side)       # join: a started clip's decoder needs its match
+        torch.cuda.current_stream().wait_stream(side)       # join: a started clip's decoder needs its match
         # started clips: the matched DB row replaces the CVAE output (test_fullframework.py:298, :437)
         _lib.check(self.lib.mocha_seed_rows(_lib.ptr(self.start[sl]), _lib.ptr(self.match_idx[sl]), 1,
                                             _lib.ptr(self.cha_encoded), self.cha_encoded.shape[0], self.ntok * self.D,
@@ -288,7 +281,7 @@ class CharacterizationSession:
         sl = slice(lo, hi)
         self.encode(self.X[sl], self.tokens[sl], self.encoded[sl], self.cnt[sl], self.cnt_nm[sl], self.cnt_nm16[sl], ws)
         side = None
-        if self.match_async and not init and not self.with_cm_path:
+        if not init and not self.with_cm_path:
             k = next(i for i, pr in enumerate(self.parts) if pr[0] == lo)
             side = self.match_streams[k]
             side.wait_stream(torch.cuda.current_stream())

@@ -16,17 +16,19 @@ def _spatial_conv_ref(x, w, b, A):
     return np.einsum("nkctv,kvw->nctw", y, A)
 
 
-def test_augmented_weight_padding_switch(monkeypatch):
-    """MOCHA_GCN_KAUG_PAD picks the K padding of the augmented gcn weight: 16 by default (the GEMM's TMA boxes zero-fill
-    the rest of the last 64-column k-block), 64 = the dense layout; the payload columns are the same either way."""
+def test_augmented_weight_layout():
+    """The augmented gcn weight is [_gcn_first's weight | the K per-partition biases | zeros], its width padded to the
+    next multiple of 16 (one tcgen05 K step; the GEMM's TMA boxes zero-fill the rest of the last 64-column k-block)."""
     sd = {k: v.detach().to(torch.float32) for k, v in weights.generator_state_dict(1777).items()}
     w4, b, A = sd["mot_embedding.2.blk.gcn.conv.weight"], sd["mot_embedding.2.blk.gcn.conv.bias"], sd["mot_embedding.2.A_j"]
-    monkeypatch.delenv("MOCHA_GCN_KAUG_PAD", raising=False)
+    K = A.shape[0]
+    wp, _ = packing._gcn_first(w4, b, A)
+    co, kp = wp.shape
     w16 = packing._gcn_first_aug(w4, b, A)
-    monkeypatch.setenv("MOCHA_GCN_KAUG_PAD", "64")
-    w64 = packing._gcn_first_aug(w4, b, A)
-    assert w16.shape[1] % 16 == 0 and w64.shape[1] % 64 == 0 and w16.shape[1] <= w64.shape[1]
-    assert torch.equal(w64[:, :w16.shape[1]], w16) and not w64[:, w16.shape[1]:].any()
+    assert w16.shape == (co, (kp + K + 15) // 16 * 16) and w16.shape[1] % 16 == 0
+    assert torch.equal(w16[:, :kp], wp)
+    assert torch.equal(w16[:, kp:kp + K], b.reshape(K, co).t())
+    assert not w16[:, kp + K:].any()
 
 
 def test_gcn_first_and_augmented_weights_reproduce_spatial_conv():

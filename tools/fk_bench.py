@@ -1,5 +1,4 @@
-"""GB/s of the batched FK kernels at the window-feature-extraction size (16 clips x 225 windows x 60 frames skeletons).
-MOCHA_NO_FK_ROWS=1 selects the warp-per-skeleton kernel for the same call (A/B of the thread-per-skeleton streaming kernel)."""
+"""GB/s of the batched FK kernels at the window-feature-extraction size (16 clips x 225 windows x 60 frames skeletons)."""
 import json
 import os
 import sys
@@ -26,7 +25,7 @@ def main():
     par = kin.parents_tensor(skeleton.BONE_PARENTS, dev)
     lrot = torch.randn((F, 25, 4), device=dev); lpos = torch.randn((F, 25, 3), device=dev)
     lvel = torch.randn((F, 25, 3), device=dev); lang = torch.randn((F, 25, 3), device=dev)
-    out = {"skeletons": F, "kernel": "warp per skeleton" if os.environ.get("MOCHA_NO_FK_ROWS") else "thread per skeleton"}
+    out = {"skeletons": F}
     for name, fn, per in (("fk", lambda: kin.fk(lrot, lpos, par), 25 * 7 * 4 * 2),
                           ("fk_vel", lambda: kin.fk_vel(lrot, lpos, lvel, lang, par), 25 * 13 * 4 * 2)):
         ms = timed(fn, 20)
