@@ -497,6 +497,28 @@ int mocha_clip_payload(const mocha_frame_record* d_rec, long long n_frames, cons
                        float* d_src_rot, float* d_src_pos, double* d_ours_rot, double* d_ours_pos, int64_t* d_match,
                        mocha_stream_t stream);
 
+/* ---- raw clip ingestion: preprocess.process_frames for a batch of clips, on the device, into the bank (DESIGN §5d)
+ * Raw clips lie back to back: d_raw_rot Euler angles in degrees and d_raw_pos positions in cm, fp64 [n_frames, J-1, 3]
+ * (motion/bvh.py:load layout; the bank's bone 0 is the root the stage adds). Clip c is raw frames d_clip_first[c] ..
+ * + d_clip_frames[c] (int64 / int32 [n_clips]) with Euler order d_clip_order[c] (int32: 0..5 = xyz xzy yxz yzx zxy
+ * zyx); its rows go to bank rows row0 + d_clip_first[c] .. of d_rot [bank_rows, J, 4], d_pos / d_vel / d_ang
+ * [bank_rows, J, 3] fp32 and d_contacts uint8 [bank_rows, 2], exactly the arrays process_frames returns.
+ * Host arrays: parents [J-1] (raw parents: parents[0] = -1, 0 <= parents[j] < j) and joints [7], the raw indices of
+ * Spine2, LeftShoulder, RightShoulder, LeftUpLeg, RightUpLeg, LeftToeBase, RightToeBase.
+ * d_savgol15 [15 + 2*7*15] / d_savgol31 [31 + 2*15*31] fp64: per filter the correlation weights ndimage applies (the
+ * savgol coefficients reversed, symmetric within DBL_EPSILON), then the maps [wl/2, wl] from the first / last wl
+ * samples to the first / last wl/2 outputs of mode='interp'. max_clip_frames >= every d_clip_frames[c] (it sizes the
+ * grids). A clip with fewer than 31 or more than max_clip_frames frames, an unknown order, or rows outside the raw
+ * buffer or the bank is skipped: nothing of it is written. Five launches on the stream, no synchronisation and no
+ * allocation; workspace of mocha_ingest_workspace_bytes(n_frames, J) bytes. */
+size_t mocha_ingest_workspace_bytes(long long n_frames, int J);
+int mocha_ingest_frames(const double* d_raw_rot, const double* d_raw_pos, long long n_frames, const int64_t* d_clip_first,
+                        const int32_t* d_clip_frames, const int32_t* d_clip_order, int n_clips, int max_clip_frames,
+                        const int32_t* parents, const int32_t* joints, int J, const double* d_savgol15,
+                        const double* d_savgol31, float* d_rot, float* d_pos, float* d_vel, float* d_ang,
+                        uint8_t* d_contacts, long long bank_rows, long long row0, void* workspace,
+                        size_t workspace_bytes, mocha_stream_t stream);
+
 /* ---- element-wise quaternion algebra of motion/quat.py in the caller's precision ------------- */
 /* out[i] = op(a[i], b[i]) for i < n; dense [n, width] arrays, float32 (is_f64 == 0) or float64. Ops and widths
  * (a, b, out): 0 mul (4,4,4) quat.py:112 | 1 inv_mul :122 | 2 mul_inv :125 | 3 mul_vec (4,3,3) :128 |

@@ -186,6 +186,9 @@ SIGNATURES = {
                                   _P, _P]),
     "mocha_record_frames": (_I, [_P, _P, _I, _P, _P, _P, _I, _P, _P, _I, _I, _P, _L, _P, _P, _P]),
     "mocha_clip_payload": (_I, [_P, _L, _P, _P, _P, _P, _I, _P, _P, _P, _I, _I, _P, _I, _I, _P, _P, _P, _P, _P, _P]),
+    "mocha_ingest_workspace_bytes": (_S, [_L, _I]),
+    "mocha_ingest_frames": (_I, [_P, _P, _L, _P, _P, _P, _I, _I, C.POINTER(C.c_int32), C.POINTER(C.c_int32), _I, _P, _P,
+                                 _P, _P, _P, _P, _P, _L, _L, _P, _S, _P]),
     "mocha_quat_op": (_I, [_I, _I, _P, _P, _L, C.c_double, _P, _P]),
     "mocha_fk_chain": (_I, [_I, _P, _P, _P, _P, _L, _I, _P, _P, _P]),
     "mocha_post_frame_packed": (_I, [C.POINTER(PostParams), _P, _P, _I, _P, _I, _I, _I, _I, _I, _P, _P, _P]),

@@ -19,7 +19,7 @@ LIB = os.path.join(HERE, "libmocha_b200.so")
 OBJ_DIR = os.path.join(HERE, "build")
 
 SOURCES = ["api.cu", "gemm_f32.cu", "ops.cu", "gemm_tc.cu", "fused_tail.cu", "fused_attn.cu", "match.cu", "networks.cu",
-           "networks_bf16.cu", "kinematics.cu"]
+           "networks_bf16.cu", "kinematics.cu", "ingest.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -1,15 +1,46 @@
 """Source clip bank: the preprocessed per-frame arrays of many source clips, resident on the device, from which
 `mocha_source_windows` builds every slot's pose window, `side` row and contacts inside the captured frame (DESIGN §5b).
 
-A 240-frame clip takes 312 KB as per-frame arrays against 19.4 MB as the 225 windows features.extract materialises."""
+A 240-frame clip takes 312 KB as per-frame arrays against 19.4 MB as the 225 windows features.extract materialises.
+`add()` preprocesses one clip on the host; `add_raw()` preprocesses a batch of raw clips on the device, straight into
+the bank (DESIGN §5d)."""
 from __future__ import annotations
 
+import ctypes as C
+
 import numpy as np
+import scipy.signal as signal
 import torch
 
 from . import _lib, preprocess, skeleton
 
 _FRAME_KEYS = ("pos", "vel", "rot", "ang", "contacts")
+# Euler order codes of mocha_ingest_frames
+EULER_ORDERS = ("xyz", "xzy", "yxz", "yzx", "zxy", "zyx")
+# raw joints the ingestion stage reads, in mocha_ingest_frames' `joints` order
+INGEST_JOINTS = ("Spine2", "LeftShoulder", "RightShoulder", "LeftUpLeg", "RightUpLeg", "LeftToeBase", "RightToeBase")
+INGEST_MIN_FRAMES = 31      # savgol_filter(root_dir, 31, 3, mode='interp') needs a clip at least that long
+_SAVGOL_CACHE: dict = {}
+
+
+def savgol_tables(wl: int, polyorder: int = 3) -> np.ndarray:
+    """process_frames' savgol_filter(x, wl, polyorder, axis=0, mode='interp') as a table, built from scipy itself:
+    [the correlation weights ndimage applies (wl) | map of the first wl samples to the first wl // 2 outputs
+    (wl // 2, wl) | map of the last wl samples to the last wl // 2 outputs (wl // 2, wl)], float64. ndimage takes its
+    symmetric path when the weights are equal within DBL_EPSILON, which the device sum mirrors: checked here."""
+    w = signal.savgol_coeffs(wl, polyorder)[::-1]
+    h = wl // 2
+    if wl % 2 != 1 or np.abs(w[h + 1:] - w[:h][::-1]).max() > np.finfo(np.float64).eps:
+        raise _lib.MochaError(f"savgol weights of window {wl} are not symmetric within DBL_EPSILON")
+    edge = signal.savgol_filter(np.eye(wl), wl, polyorder, axis=0, mode="interp")
+    return np.ascontiguousarray(np.concatenate([w, edge[:h].ravel(), edge[wl - h:].ravel()]), dtype=np.float64)
+
+
+def _savgol_device(dev) -> tuple:
+    key = str(dev)
+    if key not in _SAVGOL_CACHE:
+        _SAVGOL_CACHE[key] = tuple(torch.from_numpy(savgol_tables(wl)).to(dev) for wl in (15, 31))
+    return _SAVGOL_CACHE[key]
 
 
 class SourceBank:
@@ -71,6 +102,106 @@ class SourceBank:
         self.clip_nwin.append(nwin)
         self.clip_start.append(a)
         return c, nwin
+
+    def add_raw(self, clips) -> list:
+        """Append a batch of raw clip dicts (motion/bvh.py:load layout), preprocessed on the device by
+        mocha_ingest_frames: the rows equal process_frames' arrays (DESIGN §5d). Everything is checked on the host
+        first; a bad clip or a batch that does not fit raises MochaError and leaves the bank unchanged. Then one
+        host-to-device copy of the raw arrays and clip tables, five launches and the bank tables, stream-ordered on the
+        current stream. Returns [(clip_id, nwin)] as add() would, in order."""
+        meta = self._check_raw(clips)
+        if not meta["F"]:
+            return []
+        return self._ingest_raw(self._upload_raw(self._pack_raw(clips, meta)), meta)
+
+    def _check_raw(self, clips) -> dict:
+        J0 = self.J - 1
+        want_parents = self.parents
+        Fs, orders, joints = [], [], None
+        for n, clip in enumerate(clips):
+            rot, pos = np.asarray(clip["rotations"]), np.asarray(clip["positions"])
+            F = int(rot.shape[0]) if rot.ndim == 3 else -1
+            if rot.shape != (F, J0, 3) or pos.shape != (F, J0, 3):
+                raise _lib.MochaError(f"SourceBank.add_raw: clip {n}: rotations / positions must be [F, {J0}, 3], got "
+                                      f"{rot.shape} / {pos.shape}")
+            if clip["order"] not in EULER_ORDERS:
+                raise _lib.MochaError(f"SourceBank.add_raw: clip {n}: unknown Euler order {clip['order']!r}")
+            names = list(clip["names"])
+            missing = [j for j in INGEST_JOINTS + ("Hips",) if j not in names]
+            if missing or len(names) != J0:
+                raise _lib.MochaError(f"SourceBank.add_raw: clip {n}: needs {J0} joint names including {missing}")
+            par = np.asarray(clip["parents"])
+            if par.shape != (J0,) or not np.array_equal(np.concatenate([[-1], par + 1]), want_parents):
+                raise _lib.MochaError(f"SourceBank.add_raw: clip {n}: the clip's skeleton differs from the bank's")
+            idx = [names.index(j) for j in INGEST_JOINTS]
+            if joints is not None and idx != joints:
+                raise _lib.MochaError(f"SourceBank.add_raw: clip {n}: joint names in another order than clip 0's")
+            joints = idx
+            if F < INGEST_MIN_FRAMES or F - self.T // 4 < 1:
+                raise _lib.MochaError(f"SourceBank.add_raw: clip {n}: needs at least {max(INGEST_MIN_FRAMES, self.T // 4 + 1)} "
+                                      f"frames, got {F}")
+            Fs.append(F)
+            orders.append(EULER_ORDERS.index(clip["order"]))
+        total = sum(Fs)
+        if self.n_clips + len(Fs) > self.max_clips or self.n_frames + total > self.max_frames:
+            raise _lib.MochaError(f"SourceBank.add_raw: bank full ({self.n_clips}/{self.max_clips} clips, "
+                                  f"{self.n_frames}/{self.max_frames} frames; batch of {len(Fs)} clips, {total} frames)")
+        first = np.concatenate([[0], np.cumsum(Fs)[:-1]]).astype(np.int64) if Fs else np.zeros(0, np.int64)
+        return {"F": Fs, "order": orders, "joints": joints, "first": first, "total": total}
+
+    def _pack_raw(self, clips, meta) -> np.ndarray:
+        """One host buffer: rotations and positions fp64 [total, J-1, 3] each, then first int64, frames and order
+        int32 (8-byte aligned pieces, viewed on the device after one copy)."""
+        N, n, J0 = meta["total"], len(meta["F"]), self.J - 1
+        raw = N * J0 * 3 * 8
+        buf = np.empty(2 * raw + n * 8 + 2 * ((n * 4 + 7) // 8 * 8), dtype=np.uint8)
+        rot = buf[:raw].view(np.float64).reshape(N, J0, 3)
+        pos = buf[raw:2 * raw].view(np.float64).reshape(N, J0, 3)
+        for clip, a, F in zip(clips, meta["first"], meta["F"]):
+            rot[a:a + F] = np.asarray(clip["rotations"], dtype=np.float64)
+            pos[a:a + F] = np.asarray(clip["positions"], dtype=np.float64)
+        o = 2 * raw
+        buf[o:o + n * 8].view(np.int64)[:] = meta["first"]
+        o += n * 8
+        buf[o:o + n * 4].view(np.int32)[:] = meta["F"]
+        o += (n * 4 + 7) // 8 * 8
+        buf[o:o + n * 4].view(np.int32)[:] = meta["order"]
+        return buf
+
+    def _upload_raw(self, buf: np.ndarray) -> torch.Tensor:
+        return torch.from_numpy(buf).to(self.dev)
+
+    def _ingest_raw(self, dbuf: torch.Tensor, meta) -> list:
+        N, n, J0, J = meta["total"], len(meta["F"]), self.J - 1, self.J
+        raw = N * J0 * 3 * 8
+        o = 2 * raw
+        first = dbuf[o:o + n * 8].view(torch.int64)
+        o += n * 8
+        frames = dbuf[o:o + n * 4].view(torch.int32)
+        o += (n * 4 + 7) // 8 * 8
+        order = dbuf[o:o + n * 4].view(torch.int32)
+        lib = _lib.load()
+        ws = torch.empty(max(1, int(lib.mocha_ingest_workspace_bytes(N, J))), dtype=torch.uint8, device=self.dev)
+        sg15, sg31 = _savgol_device(self.dev)
+        parents = (C.c_int32 * J0)(*[int(p) - 1 if p >= 0 else -1 for p in self.parents[1:]])
+        joints = (C.c_int32 * 7)(*meta["joints"])
+        a, c = self.n_frames, self.n_clips
+        _lib.check(lib.mocha_ingest_frames(
+            _lib.ptr(dbuf), C.c_void_p(dbuf.data_ptr() + raw), N, _lib.ptr(first), _lib.ptr(frames), _lib.ptr(order), n,
+            max(meta["F"]), parents, joints, J, _lib.ptr(sg15), _lib.ptr(sg31), _lib.ptr(self.rot), _lib.ptr(self.pos),
+            _lib.ptr(self.vel), _lib.ptr(self.ang), _lib.ptr(self.contacts), self.max_frames, a, _lib.ptr(ws),
+            ws.numel(), _lib.stream_ptr()), "mocha_ingest_frames")
+        ws.record_stream(torch.cuda.current_stream(self.dev))
+        self.clip_first[c:c + n].copy_(torch.from_numpy(meta["first"] + a))
+        self.clip_frames[c:c + n].copy_(torch.tensor(meta["F"], dtype=torch.int32))
+        out = []
+        for k, F in enumerate(meta["F"]):
+            nwin = F - self.T // 4
+            self.clip_nwin.append(nwin)
+            self.clip_start.append(a + int(meta["first"][k]))
+            out.append((c + k, nwin))
+        self.n_frames, self.n_clips = a + N, c + n
+        return out
 
     def clear(self):
         """Forget every clip (stream-ordered). A slot still holding a cleared id turns idle, or serves the clip that is
