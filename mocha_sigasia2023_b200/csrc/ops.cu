@@ -38,17 +38,21 @@ __global__ void graph_agg_first_kernel(const float* __restrict__ in, const float
   const int KC = Kk * C;
   float* dst = out ? out + (long long)bt * V * KC : nullptr;
   __nv_bfloat16* dst16 = out16 ? out16 + (long long)bt * V * KC : nullptr;
-  // thread -> channel c (fastest, coalesced stores) and a node stripe; no divisions in the loops
-  const int c = threadIdx.x % C, stripe = threadIdx.x / C, nstripes = blockDim.x / C;
+  // thread -> channel c (fastest, coalesced stores) and a node stripe; no divisions in the loops. Rows wider than the
+  // block (C > 256: a 512-wide model's body-part blocks) take several channel passes per thread.
+  const int cw = C < (int)blockDim.x ? C : (int)blockDim.x;
+  const int c0 = threadIdx.x % cw, stripe = threadIdx.x / cw, nstripes = blockDim.x / cw;
   if (stripe < nstripes) {
     for (int w = stripe; w < V; w += nstripes) {
       for (int k = 0; k < Kk; ++k) {
         const int kw = k * V + w;
         const int n = cnt[kw];
-        float acc = 0.f;
-        for (int i = 0; i < n; ++i) acc = fmaf(xs[src[kw * V + i] * C + c], val[kw * V + i], acc);
-        if (dst) dst[w * KC + k * C + c] = acc;
-        if (dst16) dst16[w * KC + k * C + c] = __float2bfloat16_rn(acc);
+        for (int c = c0; c < C; c += cw) {
+          float acc = 0.f;
+          for (int i = 0; i < n; ++i) acc = fmaf(xs[src[kw * V + i] * C + c], val[kw * V + i], acc);
+          if (dst) dst[w * KC + k * C + c] = acc;
+          if (dst16) dst16[w * KC + k * C + c] = __float2bfloat16_rn(acc);
+        }
       }
     }
   }
@@ -1659,7 +1663,6 @@ inline unsigned blocks_for(long long total, int bs) { return (unsigned)((total +
 int graph_agg_first(const float* in, const float* A, float* out, int BT, int V, int C, int Kk, int lrelu,
                     cudaStream_t s, __nv_bfloat16* out16) {
   MOCHA_CHECK_ARG(in && A && (out || out16) && BT > 0 && V > 0 && C > 0 && Kk > 0, "graph_agg_first: bad args");
-  MOCHA_CHECK_ARG(C <= 256, "graph_agg_first: C=%d > 256 unsupported", C);
   if (!out && out16 && V <= GAS_VMAX && Kk <= 4 && (C & 3) == 0 && aligned16(in) && (reinterpret_cast<uintptr_t>(out16) & 7) == 0) {
     const long long total = (long long)BT * (C / 4);
     launch_k(graph_agg_small_kernel, blocks_for(total, 256), 256, 0, s, in, A, out16, total, V, C / 4, Kk, lrelu);
