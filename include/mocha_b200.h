@@ -139,6 +139,12 @@ typedef struct {
      multiply the adjacency column sums, K padded to a multiple of 16: [D, jb_gcn_kaug]; NULL = not provided */
   const float* jb_gcn_w_aug;
   int jb_gcn_kaug;
+  /* optional (tensor-core path, dec_dh == D only): the decoder's to_q / to_k folded into the keys and to_v into
+     to_out. dec_kfold = [G_{0,0}; ...; G_{0,H-1}; G_{1,0}; ...], G_{l,h} = Wq_{l,h}^T Wk_{l,h} ([D, D] each,
+     Wq_{l,h} = rows h*dh..(h+1)*dh of layer l's wq): [dec_depth*heads*D, D]. dec_wvo[l] = [Wo_0 Wv_0 | ... |
+     Wo_{H-1} Wv_{H-1}], Wo_h = columns h*dh..(h+1)*dh of wo, Wv_h = rows of wv: [D, heads*D]. NULL = not provided */
+  const float* dec_kfold;
+  const float* dec_wvo[MOCHA_MAX_DEPTH];
 } mocha_generator_weights;
 
 /* nn.TransformerEncoderLayer / DecoderLayer parameters exactly as PyTorch names them */

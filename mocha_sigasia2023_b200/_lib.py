@@ -71,6 +71,7 @@ class GeneratorWeights(C.Structure):
             "tm_A_b", "tm_bb_gcn_w", "tm_bb_gcn_bias2d", "tm_bb_tcn_w", "tm_bb_tcn_b", "tm_jb_gcn_w",
             "tm_jb_gcn_b", "tm_A2", "tm_jb_tcn_w", "tm_jb_tcn_b", "tm_out_w", "tm_out_b")]
         + [("jb_gcn_w_aug", C.c_void_p), ("jb_gcn_kaug", C.c_int)]
+        + [("dec_kfold", C.c_void_p), ("dec_wvo", C.c_void_p * MAX_DEPTH)]
     )
 
 

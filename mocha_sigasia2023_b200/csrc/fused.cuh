@@ -16,10 +16,12 @@ int tc_tail(const __nv_bfloat16* A0, int lda, int K0, const __nv_bfloat16* W0, c
             __nv_bfloat16* O16, int M, cudaStream_t s, int r0_period = 0);   // r0_period > 0: R0 is a [period, 256] table, row r reads R0[r % period]
 
 // Attention core in one launch (fused_attn.cu): out[b, :, h*dh:(h+1)*dh] = softmax(Q_h K_h^T / sqrt(dh)) V_h.
-// q / k / v: bf16 views [B*nq | B*nkv, ld] with head h at columns h*dh; out: bf16 [B, nq, H*dh] (ldo = H*dh).
+// q / k / v: bf16 views [B*nq | B*nkv, ld] with head h at columns h*dh (or h * the operand's head stride); out: bf16
+// [B, nq, H*dh] (ldo = H*dh).
 // dh in {64, 128, 256}, nkv <= 256, any nq.
 bool tc_attn_fused_supported(int nq, int nkv, int dh);
 int tc_attn_fused(const __nv_bfloat16* q, int ldq, const __nv_bfloat16* k, int ldk, const __nv_bfloat16* v, int ldv, int B, int H,
-                  int nq, int nkv, int dh, __nv_bfloat16* out, int ldo, cudaStream_t s, bool q_shared = false);   // q_shared: one [nq, H*dh] query table for every clip
+                  int nq, int nkv, int dh, __nv_bfloat16* out, int ldo, cudaStream_t s, bool q_shared = false,   // q_shared: one [nq, H*dh] query table for every clip
+                  int q_hs = -1, int k_hs = -1, int v_hs = -1);   // column stride between heads per operand (-1: dh; 0: shared by all heads)
 
 }  // namespace mocha

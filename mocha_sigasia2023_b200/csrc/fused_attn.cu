@@ -43,6 +43,7 @@ __device__ unsigned long long* g_fa_trace = nullptr;
 struct AttnParams {
   int B, H, nq, nkv, dh, npad;   // npad = nkv rounded up to a multiple of 64 (<= 256)
   int q_rows_b;                  // Q rows per clip: nq, or 0 when every clip shares one [nq, H*dh] query table
+  int q_hs, k_hs, v_hs;          // column of head h = h * (operand's head stride); 0: every head reads the same dh columns
   int nqt;                       // query tiles per (clip, head)
   int units;
   float scale_log2e;             // log2(e) / sqrt(dh)
@@ -119,8 +120,8 @@ attn_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUt
         mbar_expect_tx(&bar[A_QKFULL + st], q_bytes + k_bytes);
         const uint32_t base = sbase + st * p.qk_stride;
         for (int kb = 0; kb < dkb; ++kb) {
-          tma_load_2d(base + (uint32_t)kb * 16384u, &tmQ, &bar[A_QKFULL + st], h * p.dh + kb * 64, b * p.q_rows_b + qt * 128);
-          tma_load_2d(base + p.off_k + (uint32_t)kb * (uint32_t)p.npad * 128u, &tmK, &bar[A_QKFULL + st], h * p.dh + kb * 64, b * p.nkv);
+          tma_load_2d(base + (uint32_t)kb * 16384u, &tmQ, &bar[A_QKFULL + st], h * p.q_hs + kb * 64, b * p.q_rows_b + qt * 128);
+          tma_load_2d(base + p.off_k + (uint32_t)kb * (uint32_t)p.npad * 128u, &tmK, &bar[A_QKFULL + st], h * p.k_hs + kb * 64, b * p.nkv);
         }
       };
       auto load_v = [&](uint32_t it) {
@@ -131,7 +132,7 @@ attn_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUt
         mbar_expect_tx(&bar[A_VFULL], v_bytes);
         for (int kb = 0; kb < nkb; ++kb)
           for (int a = 0; a < dkb; ++a)
-            tma_load_2d(sbase + p.off_v + (uint32_t)(kb * dkb + a) * 8192u, &tmV, &bar[A_VFULL], h * p.dh + a * 64, b * p.nkv + kb * 64);
+            tma_load_2d(sbase + p.off_v + (uint32_t)(kb * dkb + a) * 8192u, &tmV, &bar[A_VFULL], h * p.v_hs + a * 64, b * p.nkv + kb * 64);
       };
       // Q / K run QS units ahead of V: the score GEMM of a later unit never waits behind the V refill, which has to wait
       // for the previous unit's second GEMM
@@ -343,15 +344,25 @@ bool tc_attn_fused_supported(int nq, int nkv, int dh) {
   return bytes <= 227 * 1024 && (size_t)nkb * 16384 >= 8 * 4096;   // the P buffer also hosts the output staging boxes
 }
 
-// q/k/v: bf16 views [B*nq | B*nkv, ld*] with head h at columns h*dh; out bf16 [B, nq, H*dh]
+// q/k/v: bf16 views [B*nq | B*nkv, ld*] with head h at columns h*{q,k,v}_hs (-1: dh; 0: all heads share columns
+// [0, dh)); out bf16 [B, nq, H*dh]
 int tc_attn_fused(const __nv_bfloat16* q, int ldq, const __nv_bfloat16* k, int ldk, const __nv_bfloat16* v, int ldv, int B, int H,
-                  int nq, int nkv, int dh, __nv_bfloat16* out, int ldo, cudaStream_t s, bool q_shared) {
+                  int nq, int nkv, int dh, __nv_bfloat16* out, int ldo, cudaStream_t s, bool q_shared, int q_hs, int k_hs,
+                  int v_hs) {
   MOCHA_CHECK_ARG(tc_attn_fused_supported(nq, nkv, dh), "tc_attn_fused: unsupported geometry nq=%d nkv=%d dh=%d", nq, nkv, dh);
   MOCHA_CHECK_ARG(q && k && v && out && B > 0 && H > 0, "tc_attn_fused: null operand");
-  MOCHA_CHECK_ARG(ldo == H * dh && (ldq % 8) == 0 && (ldk % 8) == 0 && (ldv % 8) == 0, "tc_attn_fused: bad leading dimensions");
+  if (q_hs < 0) q_hs = dh;
+  if (k_hs < 0) k_hs = dh;
+  if (v_hs < 0) v_hs = dh;
+  // columns each operand spans: the tensor maps stop there, and every head's slice must lie inside its row
+  const int qcols = (H - 1) * q_hs + dh, kcols = (H - 1) * k_hs + dh, vcols = (H - 1) * v_hs + dh;
+  MOCHA_CHECK_ARG(ldo == H * dh && (ldq % 8) == 0 && (ldk % 8) == 0 && (ldv % 8) == 0 && q_hs % 64 == 0 && k_hs % 64 == 0 &&
+                      v_hs % 64 == 0 && qcols <= ldq && kcols <= ldk && vcols <= ldv,
+                  "tc_attn_fused: bad leading dimensions or head strides");
   AttnParams p{};
   p.B = B; p.H = H; p.nq = nq; p.nkv = nkv; p.dh = dh;
   p.q_rows_b = q_shared ? 0 : nq;
+  p.q_hs = q_hs; p.k_hs = k_hs; p.v_hs = v_hs;
   p.npad = (nkv + 63) / 64 * 64;
   p.nqt = ceil_div(nq, 128);
   p.units = B * H * p.nqt;
@@ -373,11 +384,10 @@ int tc_attn_fused(const __nv_bfloat16* q, int ldq, const __nv_bfloat16* k, int l
   p.off_xch = p.off_bar + 256u;
   const size_t smem = (size_t)p.off_xch + 2048;
   MOCHA_CHECK_ARG(smem <= 227 * 1024, "tc_attn_fused: shared-memory plan of %zu B exceeds 227 KB", smem);
-  const int inner = H * dh;
   CUtensorMap tmQ, tmK, tmV, tmO;
-  MOCHA_TRY(tc_make_tmap(&tmQ, q, (unsigned long long)(q_shared ? 1 : B) * nq, (unsigned long long)inner, 128, (unsigned long long)ldq));
-  MOCHA_TRY(tc_make_tmap(&tmK, k, (unsigned long long)B * nkv, (unsigned long long)inner, p.npad, (unsigned long long)ldk));
-  MOCHA_TRY(tc_make_tmap(&tmV, v, (unsigned long long)B * nkv, (unsigned long long)inner, 64, (unsigned long long)ldv));
+  MOCHA_TRY(tc_make_tmap(&tmQ, q, (unsigned long long)(q_shared ? 1 : B) * nq, (unsigned long long)qcols, 128, (unsigned long long)ldq));
+  MOCHA_TRY(tc_make_tmap(&tmK, k, (unsigned long long)B * nkv, (unsigned long long)kcols, p.npad, (unsigned long long)ldk));
+  MOCHA_TRY(tc_make_tmap(&tmV, v, (unsigned long long)B * nkv, (unsigned long long)vcols, 64, (unsigned long long)ldv));
   MOCHA_TRY(tc_make_out_tmap(&tmO, out, (unsigned long long)ldo, (unsigned long long)nq, (unsigned long long)B,
                              (unsigned long long)ldo, false, 0, true));
   static size_t configured = 0;

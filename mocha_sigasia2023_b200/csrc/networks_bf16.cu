@@ -201,10 +201,16 @@ int decoder_bf16(const mocha_generator_weights* w, const float* src, const float
   float* x2 = ws.take<float>((size_t)R * d.D);
   bf16* x2h = ws.take<bf16>((size_t)R * d.D);
   float* xb = ws.take<float>((size_t)R * d.D);
-  bf16* qkv3 = ws.take<bf16>((size_t)3 * R * inner);
+  // Folded attention (packing.py:decoder_folded, dh == D): to_q / to_k fold into ONE key projection of IN(style) for every
+  // layer and head, to_v into to_out; the query IN(x1) and the value (the style itself) are read by every head as they are.
+  bool folded = w->dec_kfold && d.dec_dh == d.D && tc_attn_fused_supported(n, n, d.dec_dh);
+  for (int l = 0; l < d.dec_depth && folded; ++l) folded = w->dec_wvo[l] != nullptr;
+  const int kf_ld = d.dec_depth * inner;   // [R, depth*H*D]: layer l, head h at columns (l*H + h)*D
+  bf16* kfold = folded ? ws.take<bf16>((size_t)R * kf_ld) : nullptr;
+  bf16* qkv3 = folded ? nullptr : ws.take<bf16>((size_t)3 * R * inner);
   bf16* q = qkv3;
-  bf16* k = qkv3 + (size_t)R * inner;
-  bf16* v = qkv3 + (size_t)2 * R * inner;
+  bf16* k = folded ? nullptr : qkv3 + (size_t)R * inner;
+  bf16* v = folded ? nullptr : qkv3 + (size_t)2 * R * inner;
   bf16* att = ws.take<bf16>((size_t)R * inner);
   float* S = nullptr;   // scores stay in TMEM (softmax fused into the Q K^T epilogue)
   bf16* hid = ws.take<bf16>((size_t)R * d.mlp);
@@ -242,6 +248,8 @@ int decoder_bf16(const mocha_generator_weights* w, const float* src, const float
     MOCHA_CUDA(cudaEventRecord(side->join, side->stream));
     MOCHA_CUDA(cudaStreamWaitEvent(s, side->join, 0));
   }
+  if (folded)
+    MOCHA_TRY(tc.lin(sty_in, d.D, w->dec_kfold, nullptr, 0, nullptr, h16(kfold), R, kf_ld, d.D, ACT_NONE));
   const float* x = src;
   for (int l = 0; l < d.dec_depth; ++l) {
     const mocha_dec_layer& L = w->dec[l];
@@ -258,22 +266,30 @@ int decoder_bf16(const mocha_generator_weights* w, const float* src, const float
       MOCHA_TRY(instance_norm_tokens(x, B, n, d.D, eps, gb, x1, nullptr, nullptr, nullptr, s));
       MOCHA_TRY(instance_norm_tokens(x1, B, n, d.D, eps, nullptr, nullptr, nullptr, nullptr, nullptr, s, qin));
     }
-    const bf16* wq16 = tc_lookup_bf16(L.wq);
-    if (wq16 && L.wk == L.wq + (size_t)inner * d.D && L.wv == L.wk + (size_t)inner * d.D && inner % 64 == 0) {
-      // to_q / to_k / to_v sit back to back in the packed blob: three inputs x three weights in one launch
-      MOCHA_TRY(tc_linear_bf16_grouped(in3, wq16, qkv3, 3, R, inner, d.D, s));
+    const float* wo = L.wo;
+    if (folded) {
+      // head h: softmax(IN(x1) K_{l,h}^T / sqrt(D)) style, K_{l,h} = IN(style) G_{l,h}^T; its out-projection is Wo_h Wv_h
+      MOCHA_TRY(tc_attn_fused(qin, d.D, kfold + (size_t)l * inner, kf_ld, cha16, d.D, B, d.heads, n, n, d.dec_dh, att, inner, s,
+                              false, 0, d.D, 0));
+      wo = w->dec_wvo[l];
     } else {
-      MOCHA_TRY(tc.lin(qin, d.D, L.wq, nullptr, 0, nullptr, h16(q), R, inner, d.D, ACT_NONE));
-      MOCHA_TRY(tc.lin(sty_in, d.D, L.wk, nullptr, 0, nullptr, h16(k), R, inner, d.D, ACT_NONE));
-      MOCHA_TRY(tc.lin(cha16, d.D, L.wv, nullptr, 0, nullptr, h16(v), R, inner, d.D, ACT_NONE));
+      const bf16* wq16 = tc_lookup_bf16(L.wq);
+      if (wq16 && L.wk == L.wq + (size_t)inner * d.D && L.wv == L.wk + (size_t)inner * d.D && inner % 64 == 0) {
+        // to_q / to_k / to_v sit back to back in the packed blob: three inputs x three weights in one launch
+        MOCHA_TRY(tc_linear_bf16_grouped(in3, wq16, qkv3, 3, R, inner, d.D, s));
+      } else {
+        MOCHA_TRY(tc.lin(qin, d.D, L.wq, nullptr, 0, nullptr, h16(q), R, inner, d.D, ACT_NONE));
+        MOCHA_TRY(tc.lin(sty_in, d.D, L.wk, nullptr, 0, nullptr, h16(k), R, inner, d.D, ACT_NONE));
+        MOCHA_TRY(tc.lin(cha16, d.D, L.wv, nullptr, 0, nullptr, h16(v), R, inner, d.D, ACT_NONE));
+      }
+      MOCHA_TRY(attn(s, ws, q, inner, k, inner, v, inner, B, d.heads, n, n, d.dec_dh, att, inner));
     }
-    MOCHA_TRY(attn(s, ws, q, inner, k, inner, v, inner, B, d.heads, n, n, d.dec_dh, att, inner));
     float* dst = (l == d.dec_depth - 1) ? decoded : xb;
     if (use_fused_tail(d.D) && tc_tail_supported(R, inner, d.mlp)) {
-      MOCHA_TRY(tail(s, att, inner, L.wo, L.bo, x1, nullptr, nullptr, d.mlp, ACT_GELU, L.w1, L.b1, L.w2, L.b2, nullptr, nullptr,
+      MOCHA_TRY(tail(s, att, inner, wo, L.bo, x1, nullptr, nullptr, d.mlp, ACT_GELU, L.w1, L.b1, L.w2, L.b2, nullptr, nullptr,
                      0.f, dst, nullptr, R));
     } else {
-      MOCHA_TRY(tc.lin(att, inner, L.wo, L.bo, 0, x1, both(x2, x2h), R, d.D, inner, ACT_NONE));
+      MOCHA_TRY(tc.lin(att, inner, wo, L.bo, 0, x1, both(x2, x2h), R, d.D, inner, ACT_NONE));
       MOCHA_TRY(tc.lin(x2h, d.D, L.w1, L.b1, 0, nullptr, h16(hid), R, d.mlp, d.D, ACT_GELU));
       MOCHA_TRY(tc.lin(hid, d.mlp, L.w2, L.b2, 0, x2, f32(dst), R, d.D, d.mlp, ACT_NONE));
     }

@@ -89,6 +89,31 @@ def _gcn_first_aug(w: torch.Tensor, b: torch.Tensor, A: torch.Tensor) -> torch.T
     return out.contiguous()
 
 
+def decoder_folded(sd: "dict[str, torch.Tensor]", cfg: dict) -> "dict[str, torch.Tensor]":
+    """The decoder attention with to_q / to_k folded into the keys and to_v into to_out (bias-free projections).
+
+    With x^ = IN(x1), s^ = IN(style), s = style and dh == D, head h scores (x^ Wq_h^T)(s^ Wk_h^T)^T = x^ (s^ G_h^T)^T
+    with G_h = Wq_h^T Wk_h, and the output sum_h (P_h s Wv_h^T) Wo_h^T = sum_h (P_h s)(Wo_h Wv_h)^T. The folded
+    matrices have the shapes of the ones they replace only when dh == D; otherwise nothing is returned.
+    "dec_kfold": [depth*H*D, D], rows ordered layer, head, feature; "dec{l}.wvo": [D, H*D]. The products are formed
+    and returned in float64; the weight blob stores them in fp32 like every other slice.
+    """
+    D, H, dh = cfg["decoder_dim"], cfg["decoder_heads"], cfg["decoder_dim_head"]
+    if dh != D:
+        return {}
+    g, out = [], {}
+    for l in range(cfg["decoder_depth"]):
+        p = f"decoder.layers.{l}.1"
+        wq = sd[p + ".to_q.1.weight"].to(torch.float64).reshape(H, dh, D)
+        wk = sd[p + ".to_k.1.weight"].to(torch.float64).reshape(H, dh, D)
+        wv = sd[p + ".to_v.weight"].to(torch.float64).reshape(H, dh, D)
+        wo = sd[p + ".to_out.0.weight"].to(torch.float64).reshape(D, H, dh)
+        g.append(torch.einsum("hki,hkj->hij", wq, wk).reshape(H * D, D))                 # G_h = Wq_h^T Wk_h
+        out[f"dec{l}.wvo"] = torch.einsum("ohk,hkj->ohj", wo, wv).reshape(D, H * D).contiguous()
+    out["dec_kfold"] = torch.cat(g, dim=0).contiguous()
+    return out
+
+
 def generator_tensors(sd: "dict[str, torch.Tensor]", cfg: dict) -> "dict[str, torch.Tensor]":
     sd = {k: v.detach().to(torch.float32).cpu() for k, v in sd.items()}
     out = {}
@@ -137,6 +162,7 @@ def generator_tensors(sd: "dict[str, torch.Tensor]", cfg: dict) -> "dict[str, to
         out[f"dec{l}.b1"] = sd[p + ".2.net.0.bias"]
         out[f"dec{l}.w2"] = sd[p + ".2.net.3.weight"]
         out[f"dec{l}.b2"] = sd[p + ".2.net.3.bias"]
+    out.update(decoder_folded(sd, cfg))
     tA_b = sd["to_mot.1.A_b"]
     out["tm_A_b"] = tA_b
     out["tm_bb_gcn_w"], out["tm_bb_gcn_bias2d"] = _gcn_first(
@@ -199,6 +225,10 @@ class PackedGenerator:
         for l in range(cfg["decoder_depth"]):
             for f in ("sw1", "sb1", "sw2", "sb2", "wq", "wk", "wv", "wo", "bo", "w1", "b1", "w2", "b2"):
                 setattr(w.dec[l], f, b.ptr(f"dec{l}.{f}"))
+        if "dec_kfold" in b.offsets:
+            w.dec_kfold = b.ptr("dec_kfold")
+            for l in range(cfg["decoder_depth"]):
+                w.dec_wvo[l] = b.ptr(f"dec{l}.wvo")
         self.struct = w
         self.dims = w.dims
         self.ntok = (w.dims.T // w.dims.tp) * w.dims.P
