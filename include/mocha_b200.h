@@ -308,6 +308,28 @@ int mocha_topk_merge(const double* d_dist, const int64_t* d_idx, int nshard, int
 int mocha_seed_rows(const uint8_t* d_start, const int64_t* d_idx, int idx_stride, const float* d_table, long long N,
                     long long row_elems, float* d_dst, int B, mocha_stream_t stream);
 
+/* Segmented matching (character banks: several characters' rows back to back in one DB): query q searches only the
+ * rows d_seg_first[q] .. d_seg_first[q] + d_seg_rows[q] - 1 (int64 / int32 [nq], clipped to [0, N)). Returned indices
+ * are DB rows (+ index_offset), as for the unsegmented calls; a segment of fewer than k rows fills the missing entries
+ * with idx -1 / dist +inf, and an empty segment gives only those. Same arguments, workspaces and kernels as
+ * mocha_match_exact / mocha_match_tc otherwise. The exact path equals mocha_match_exact over the segment's rows with
+ * index_offset + first, bit for bit (the per-pair fp64 sum depends on neither the tile shape nor N). */
+int mocha_match_exact_segmented(const float* d_Q, int nq, const float* d_DB, long long N, int D, int k,
+                                long long index_offset, const int64_t* d_seg_first, const int32_t* d_seg_rows,
+                                int64_t* d_idx, double* d_dist, void* workspace, size_t workspace_bytes,
+                                mocha_stream_t stream);
+int mocha_match_tc_segmented(const float* d_Q, const void* d_Q16, int nq, const void* d_DB16, const float* d_DB32,
+                             const float* d_dbnorm, long long N, int D, int k, int kc, long long index_offset,
+                             const int64_t* d_seg_first, const int32_t* d_seg_rows, int64_t* d_idx, double* d_dist,
+                             void* workspace, size_t workspace_bytes, mocha_stream_t stream);
+/* Per-slot segments of a character bank, one launch per frame before the segmented matcher: for every b < B, if
+ * d_start[b] then d_slot_char[b] = d_character[b] (int32 session state, like a source bank's slot_clip); then
+ * d_seg_first[b] / d_seg_rows[b] = d_char_first[c] / d_char_rows[c] of c = d_slot_char[b] (int64 / int32 [n_chars]
+ * tables), or 0 / 0 (an empty segment) when c is outside [0, n_chars). */
+int mocha_slot_segments(const uint8_t* d_start, const int32_t* d_character, int32_t* d_slot_char, int B,
+                        const int64_t* d_char_first, const int32_t* d_char_rows, int n_chars, int64_t* d_seg_first,
+                        int32_t* d_seg_rows, mocha_stream_t stream);
+
 /* ---- peer-memory exchange of the DB-sharded matcher (one process per GPU, NVLink / NVSwitch P2P) ----
  * Fused replacement of "all-gather the [nq,k] lists, then merge" (sharded.py): ONE kernel per rank stores
  * its local lists into a slot of every peer's exchange buffer (plain P2P stores over NVLink), raises a

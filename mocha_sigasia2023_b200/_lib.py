@@ -162,6 +162,9 @@ SIGNATURES = {
     "mocha_match_exact": (_I, [_P, _I, _P, _L, _I, _I, _L, _P, _P, _P, _S, _P]),
     "mocha_match_tc_workspace_bytes": (_S, [_I, _L, _I, _I]),
     "mocha_match_tc": (_I, [_P, _P, _I, _P, _P, _P, _L, _I, _I, _I, _L, _P, _P, _P, _S, _P]),
+    "mocha_match_exact_segmented": (_I, [_P, _I, _P, _L, _I, _I, _L, _P, _P, _P, _P, _P, _S, _P]),
+    "mocha_match_tc_segmented": (_I, [_P, _P, _I, _P, _P, _P, _L, _I, _I, _I, _L, _P, _P, _P, _P, _P, _S, _P]),
+    "mocha_slot_segments": (_I, [_P, _P, _P, _I, _P, _P, _I, _P, _P, _P]),
     "mocha_db_norms_f32": (_I, [_P, _L, _I, _P, _P]),
     "mocha_db_pack_bf16": (_I, [_P, _L, _I, _P, _P, _P]),
     "mocha_topk_merge": (_I, [_P, _P, _I, _I, _I, _P, _P, _P]),

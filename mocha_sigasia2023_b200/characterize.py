@@ -9,6 +9,7 @@ import torch
 
 from . import features, kinematics as kin
 from . import preprocess, skeleton, weights
+from ._lib import MochaError
 from .session import CharacterizationSession, NormStats
 
 
@@ -124,20 +125,34 @@ def characterize(src_clip: dict, cha_clip: dict, raw_stats: dict, gen_sd=None, c
             "trans_rot": np.stack([f["rot"][0] for f in frames]), "n_db": int(n_cha)}
 
 
-def characterize_many(src_clips, cha_clip: dict, raw_stats: dict, gen_sd=None, cvae_sd=None, slots: int = 1,
+def characterize_many(src_clips, cha_clip, raw_stats: dict, gen_sd=None, cvae_sd=None, slots: int = 1,
                       eps_seqs=None, precision: str = "fp32", encode_batch: int = 32, lanes: int = 1,
-                      with_cm_path: bool = False) -> list:
+                      with_cm_path: bool = False, cha_index=None) -> list:
     """The many-clip counterpart of characterize(): every source clip characterized with one target character through
     a source bank, a result bank and one captured admission session of `slots` slots (CharacterizationSession.serve).
     The character DB is built as characterize() builds it, and the session matches with the same fp64 brute-force
     kernel (match_tensor_cores=False).
 
+    cha_clip: one character clip, or a list of them with cha_index (one index into that list per source clip): each
+    character's DB is built as characterize() builds it, the DBs go into one CharacterBank, and every source clip is
+    served toward its own character in the same session; its `match` counts rows of its character's DB.
+
     eps_seqs: None (fresh standard-normal draws) or {index into src_clips: array [nwin-1, 256]} in characterize()'s
     eps_seq layout; clips without an entry draw standard-normal rows. Returns one dict per source clip:
     {src_rotations, src_positions, ours_rotations, ours_positions, match}."""
+    from .character_bank import CharacterBank
     from .result_bank import ResultBank
     from .source_bank import SourceBank
     src_clips = list(src_clips)
+    several = not isinstance(cha_clip, dict)
+    if several:
+        cha_clips = list(cha_clip)
+        if cha_index is None or len(cha_index) != len(src_clips):
+            raise MochaError("characterize_many with a list of character clips needs cha_index, one entry per source clip")
+        if not cha_clips or any(not 0 <= int(c) < len(cha_clips) for c in cha_index):
+            raise MochaError(f"characterize_many: cha_index must index the {len(cha_clips)} character clips")
+    elif cha_index is not None:
+        raise MochaError("characterize_many: cha_index goes with a list of character clips")
     if not src_clips:
         return []
     dev = "cuda"
@@ -149,11 +164,19 @@ def characterize_many(src_clips, cha_clip: dict, raw_stats: dict, gen_sd=None, c
                       raw_stats["norm"]["X_std"], device=dev)
     ids = [bank.add(f)[0] for f in frames]
     results = ResultBank(bank)
-    cha_enc, cha_nm = _character_db(cha_clip, raw_stats, gen_sd, cvae_sd, stats, precision, encode_batch)
-    sess = CharacterizationSession(gen_sd, cvae_sd, weights.DEFAULT_MODEL_CFG, stats, cha_enc, cha_nm, batch=slots,
-                                   device=dev, precision=precision, match_tensor_cores=False, lanes=lanes,
-                                   with_cm_path=with_cm_path, admission=True, source_bank=bank, result_bank=results)
-    sess.capture()
+    kw = dict(batch=slots, device=dev, precision=precision, match_tensor_cores=False, lanes=lanes,
+              with_cm_path=with_cm_path, admission=True, source_bank=bank, result_bank=results)
     eps = None if eps_seqs is None else {ids[i]: e for i, e in eps_seqs.items()}
+    if several:
+        dbs = [_character_db(c, raw_stats, gen_sd, cvae_sd, stats, precision, encode_batch) for c in cha_clips]
+        chars = CharacterBank([d[0] for d in dbs], [d[1] for d in dbs])
+        sess = CharacterizationSession(gen_sd, cvae_sd, weights.DEFAULT_MODEL_CFG, stats, None, None, characters=chars,
+                                       **kw)
+        sess.capture()
+        out = sess.serve(ids, eps=eps, characters={c: int(i) for c, i in zip(ids, cha_index)})
+        return [out[c] for c in ids]
+    cha_enc, cha_nm = _character_db(cha_clip, raw_stats, gen_sd, cvae_sd, stats, precision, encode_batch)
+    sess = CharacterizationSession(gen_sd, cvae_sd, weights.DEFAULT_MODEL_CFG, stats, cha_enc, cha_nm, **kw)
+    sess.capture()
     out = sess.serve(ids, eps=eps)
     return [out[c] for c in ids]

@@ -413,7 +413,7 @@ struct LinearEpiT : LinearEpiData {
   static constexpr uint64_t kHintA = 0, kHintB = 0;                // default L2 policy
   static constexpr bool kTf32 = false;
   static constexpr bool kWholeTile = false;
-  __device__ __forceinline__ void unit_begin(State&) const {}
+  __device__ __forceinline__ void unit_begin(State&, long long, bool) const {}
   __device__ __forceinline__ void kernel_begin(State& st, const EpiCtx& e) const {
     st.rphase = 0; st.col_begin = 0; st.rs = 1.f; st.par = 0;
     if (MODE != 0) {
@@ -921,7 +921,7 @@ struct SoftmaxEpi {
   static constexpr uint64_t kHintA = 0, kHintB = 0;
   static constexpr bool kTf32 = false;
   static constexpr bool kWholeTile = true;
-  __device__ __forceinline__ void unit_begin(State&) const {}
+  __device__ __forceinline__ void unit_begin(State&, long long, bool) const {}
   __device__ __forceinline__ void kernel_begin(State&, const EpiCtx&) const {}
   __device__ __forceinline__ void tile_begin(State&, const EpiCtx&, int, int) const {}
   __device__ __forceinline__ void unit_end(State&, const EpiCtx&, long long, bool, int) const {}
@@ -1000,6 +1000,10 @@ struct MatchEpi {
   float* cand_score;
   int32_t* cand_idx;
   int lists;  // candidate lists per query = 2 * splits (one per column half)
+  // segmented matching (NULL: every query searches all N rows): query r ranks only the rows
+  // seg_first[r] .. seg_first[r] + seg_rows[r] (clipped to [0, N)); other columns are not candidates
+  const int64_t* seg_first;
+  const int32_t* seg_rows;
   static constexpr int kWarpStageBytes = 0;
   static constexpr int kStageBytes = 0;
   static constexpr bool kWholeTile = false;
@@ -1008,26 +1012,35 @@ struct MatchEpi {
   struct State {
     float s[KC];
     int32_t i[KC];
+    int lo, hi;  // the row's candidate columns [lo, hi), read once per unit (no global load per chunk for them)
   };
-  __device__ __forceinline__ void unit_begin(State& st) const {
+  __device__ __forceinline__ void unit_begin(State& st, long long row, bool row_ok) const {
 #pragma unroll
     for (int t = 0; t < KC; ++t) { st.s[t] = INFINITY; st.i[t] = -1; }
+    st.lo = 0;
+    st.hi = (int)N;
+    if (seg_first && row_ok) {
+      const long long f = __ldg(seg_first + row), e = f + __ldg(seg_rows + row);
+      st.lo = (int)min(max(f, 0LL), N);
+      st.hi = (int)min(max(e, 0LL), N);
+    }
   }
   __device__ __forceinline__ void kernel_begin(State&, const EpiCtx&) const {}
   __device__ __forceinline__ void tile_begin(State&, const EpiCtx&, int, int) const {}
   __device__ __forceinline__ void chunk(State& st, const EpiCtx&, long long, bool row_ok, int col0,
                                         const uint32_t (&v)[32], int) const {
-    if (!row_ok || col0 >= N) return;
+    if (!row_ok || col0 >= st.hi || col0 + 32 <= st.lo) return;
     float nrm[32];
-    if ((long long)col0 + 32 <= N) {
+    if (col0 >= st.lo && col0 + 32 <= st.hi) {
 #pragma unroll
       for (int j = 0; j < 32; j += 4) {
         const float4 t = __ldg(reinterpret_cast<const float4*>(dbnorm + col0 + j));
         nrm[j] = t.x; nrm[j + 1] = t.y; nrm[j + 2] = t.z; nrm[j + 3] = t.w;
       }
     } else {
+      // +inf norm: the column is past the last row or outside the row's segment, never a candidate
 #pragma unroll
-      for (int j = 0; j < 32; ++j) nrm[j] = ((long long)col0 + j < N) ? __ldg(dbnorm + col0 + j) : INFINITY;
+      for (int j = 0; j < 32; ++j) nrm[j] = (col0 + j >= st.lo && col0 + j < st.hi) ? __ldg(dbnorm + col0 + j) : INFINITY;
     }
 #pragma unroll
     for (int j = 0; j < 32; ++j) {
@@ -1367,7 +1380,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         ectx.img = zb;                      // TMA-store view of a [B, rows, H*cols] output (host checks the layout)
         ectx.col_off = zh * (int)sh.c_img_h;
       }
-      epi.unit_begin(st);
+      epi.unit_begin(st, row, row_ok);
       const int nt_end = min(sh.tiles_n, (split + 1) * sh.tiles_per_unit);
       for (int nt = split * sh.tiles_per_unit; nt < nt_end; ++nt) {
         // the tile's BN/32 column chunks are split between the two warps that share a lane quarter
@@ -1661,7 +1674,7 @@ tc_gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
       ectx.slab_row0 = (long long)b * sh.rows_out_per_b + r0;
       ectx.slab_rows = max(0, min(32, sh.rows_out_per_b - r0));
       ectx.img = b; ectx.z = b; ectx.row0_in_img = r0;
-      epi.unit_begin(st);
+      epi.unit_begin(st, row, row_ok);
       const int nt_end = min(sh.tiles_n, (split + 1) * sh.tiles_per_unit);
       for (int nt = split * sh.tiles_per_unit; nt < nt_end; ++nt) {
         const int c_begin = ectx.half * (BN / 2), c_end = c_begin + BN / 2;
@@ -2797,7 +2810,8 @@ int tc_match_splits(int nq, long long N) {
 // fp32-storage variant: queries and DB rows stay fp32 in HBM and are consumed as TF32 by tcgen05
 // (kind::tf32, K = 8 per instruction; 32 elements per 128-byte k-block row)
 int tc_match_coarse_tf32(const float* Q, int nq, const float* DB, const float* dbnorm, long long N, int D, int kc,
-                         float* cand_score, int32_t* cand_idx, cudaStream_t s) {
+                         float* cand_score, int32_t* cand_idx, const int64_t* seg_first, const int32_t* seg_rows,
+                         cudaStream_t s) {
   MOCHA_CHECK_ARG(Q && DB && dbnorm && cand_score && cand_idx, "tc_match_coarse_tf32: null operand");
   MOCHA_CHECK_ARG(nq > 0 && N > 0 && N < 2147483647LL, "tc_match_coarse_tf32: bad sizes nq=%d N=%lld", nq, N);
   MOCHA_CHECK_ARG(D >= 32 && D % 4 == 0, "tc_match_coarse_tf32: D=%d must be >= 32 and a multiple of 4", D);
@@ -2827,13 +2841,14 @@ int tc_match_coarse_tf32(const float* Q, int nq, const float* DB, const float* d
     sh.group_m = (int)gm;
   }
   const int num_kb = ceil_div(D, 32);
-  if (kc == 4) return launch_tc<BN, MatchEpi<4, true>>(tmA, tmB, sh, num_kb, MatchEpi<4, true>{dbnorm, N, cand_score, cand_idx, 2 * splits}, s);
-  if (kc == 8) return launch_tc<BN, MatchEpi<8, true>>(tmA, tmB, sh, num_kb, MatchEpi<8, true>{dbnorm, N, cand_score, cand_idx, 2 * splits}, s);
-  return launch_tc<BN, MatchEpi<16, true>>(tmA, tmB, sh, num_kb, MatchEpi<16, true>{dbnorm, N, cand_score, cand_idx, 2 * splits}, s);
+  if (kc == 4) return launch_tc<BN, MatchEpi<4, true>>(tmA, tmB, sh, num_kb, MatchEpi<4, true>{dbnorm, N, cand_score, cand_idx, 2 * splits, seg_first, seg_rows}, s);
+  if (kc == 8) return launch_tc<BN, MatchEpi<8, true>>(tmA, tmB, sh, num_kb, MatchEpi<8, true>{dbnorm, N, cand_score, cand_idx, 2 * splits, seg_first, seg_rows}, s);
+  return launch_tc<BN, MatchEpi<16, true>>(tmA, tmB, sh, num_kb, MatchEpi<16, true>{dbnorm, N, cand_score, cand_idx, 2 * splits, seg_first, seg_rows}, s);
 }
 
 int tc_match_coarse(const __nv_bfloat16* Q16, int nq, const __nv_bfloat16* DB16, const float* dbnorm, long long N,
-                    int D, int kc, float* cand_score, int32_t* cand_idx, cudaStream_t s) {
+                    int D, int kc, float* cand_score, int32_t* cand_idx, const int64_t* seg_first,
+                    const int32_t* seg_rows, cudaStream_t s) {
   MOCHA_CHECK_ARG(Q16 && DB16 && dbnorm && cand_score && cand_idx, "tc_match_coarse: null operand");
   MOCHA_CHECK_ARG(nq > 0 && N > 0 && N < 2147483647LL, "tc_match_coarse: bad sizes nq=%d N=%lld", nq, N);
   MOCHA_CHECK_ARG(D >= BLOCK_K && D % 8 == 0, "tc_match_coarse: D=%d must be >= 64 and a multiple of 8", D);
@@ -2866,9 +2881,9 @@ int tc_match_coarse(const __nv_bfloat16* Q16, int nq, const __nv_bfloat16* DB16,
     sh.group_m = (int)gm;
   }
   const int num_kb = ceil_div(D, BLOCK_K);
-  if (kc == 4) return launch_tc<BN, MatchEpi<4>>(tmA, tmB, sh, num_kb, MatchEpi<4>{dbnorm, N, cand_score, cand_idx, 2 * splits}, s);
-  if (kc == 8) return launch_tc<BN, MatchEpi<8>>(tmA, tmB, sh, num_kb, MatchEpi<8>{dbnorm, N, cand_score, cand_idx, 2 * splits}, s);
-  return launch_tc<BN, MatchEpi<16>>(tmA, tmB, sh, num_kb, MatchEpi<16>{dbnorm, N, cand_score, cand_idx, 2 * splits}, s);
+  if (kc == 4) return launch_tc<BN, MatchEpi<4>>(tmA, tmB, sh, num_kb, MatchEpi<4>{dbnorm, N, cand_score, cand_idx, 2 * splits, seg_first, seg_rows}, s);
+  if (kc == 8) return launch_tc<BN, MatchEpi<8>>(tmA, tmB, sh, num_kb, MatchEpi<8>{dbnorm, N, cand_score, cand_idx, 2 * splits, seg_first, seg_rows}, s);
+  return launch_tc<BN, MatchEpi<16>>(tmA, tmB, sh, num_kb, MatchEpi<16>{dbnorm, N, cand_score, cand_idx, 2 * splits, seg_first, seg_rows}, s);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -2881,7 +2896,8 @@ int tc_match_coarse(const __nv_bfloat16* Q16, int nq, const __nv_bfloat16* DB16,
 namespace {
 __global__ void splitk_reduce_kernel(const float* __restrict__ partial, int slices, int nq, int Np, long long N,
                                      const float* __restrict__ dbnorm, float* __restrict__ cand_score,
-                                     int32_t* __restrict__ cand_idx) {
+                                     int32_t* __restrict__ cand_idx, const int64_t* __restrict__ seg_first,
+                                     const int32_t* __restrict__ seg_rows) {
   pdl_trigger();
   pdl_wait();
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -2890,7 +2906,11 @@ __global__ void splitk_reduce_kernel(const float* __restrict__ partial, int slic
   float acc = 0.f;
   const long long img = (long long)nq * Np;
   for (int z = 0; z < slices; ++z) acc += partial[z * img + i];
-  const bool ok = n < N;
+  bool ok = n < N;
+  if (seg_first) {   // segmented: a column outside the query's rows is no candidate
+    const long long q = i / Np, f = seg_first[q];
+    ok = ok && n >= f && n < f + seg_rows[q];
+  }
   cand_score[i] = ok ? fmaf(-2.f, acc, __ldg(dbnorm + n)) : INFINITY;
   cand_idx[i] = ok ? n : -1;
 }
@@ -2917,7 +2937,8 @@ size_t tc_match_splitk_ws_bytes(int nq, long long N, int D) {
 
 // candidate lists: cand_score / cand_idx are [nq, Np] with Np = round_up(N, 128) (index -1 past N)
 int tc_match_coarse_splitk(const __nv_bfloat16* Q16, int nq, const __nv_bfloat16* DB16, const float* dbnorm, long long N,
-                           int D, float* partial, float* cand_score, int32_t* cand_idx, cudaStream_t s) {
+                           int D, float* partial, float* cand_score, int32_t* cand_idx, const int64_t* seg_first,
+                           const int32_t* seg_rows, cudaStream_t s) {
   const int slices = tc_match_splitk_slices(nq, N, D);
   MOCHA_CHECK_ARG(slices >= 2 && Q16 && DB16 && partial, "tc_match_coarse_splitk: not applicable");
   constexpr int BN = 128;
@@ -2937,7 +2958,8 @@ int tc_match_coarse_splitk(const __nv_bfloat16* Q16, int nq, const __nv_bfloat16
   LinearEpi epi{partial, Np, Np, nullptr, 0, nullptr, ACT_NONE, nullptr, 0};
   MOCHA_TRY(dispatch_bn(BN, tmA, DB16, (unsigned long long)N, (unsigned long long)D, sh, Np, kb_per, epi, s));
   const long long total = (long long)nq * Np;
-  launch_k(splitk_reduce_kernel, (unsigned)((total + 255) / 256), 256, 0, s, partial, slices, nq, Np, N, dbnorm, cand_score, cand_idx);
+  launch_k(splitk_reduce_kernel, (unsigned)((total + 255) / 256), 256, 0, s, partial, slices, nq, Np, N, dbnorm, cand_score, cand_idx,
+           seg_first, seg_rows);
   count_launch();
   MOCHA_LAUNCH_CHECK("splitk_reduce_kernel");
   return MOCHA_OK;

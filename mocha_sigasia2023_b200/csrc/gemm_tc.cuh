@@ -96,17 +96,22 @@ int tc_attention_ex(const float* q, const __nv_bfloat16* qh, int ldq, const floa
 constexpr int MATCH_KC_MAX = 16;
 // Number of N-splits the coarse pass will use for (nq, N); candidates are [nq, splits, kc].
 int tc_match_splits(int nq, long long N);
+// Every coarse pass takes optional per-query segments (seg_first / seg_rows [nq], NULL = all N rows): query q's
+// candidates are then the rows seg_first[q] .. + seg_rows[q] only (clipped to [0, N)).
 // split-K coarse pass for small problems (0 slices = not applicable); candidates are [nq, round_up(N,128)]
 int tc_match_splitk_slices(int nq, long long N, int D);
 size_t tc_match_splitk_ws_bytes(int nq, long long N, int D);
 int tc_match_coarse_splitk(const __nv_bfloat16* Q16, int nq, const __nv_bfloat16* DB16, const float* dbnorm, long long N,
-                           int D, float* partial, float* cand_score, int32_t* cand_idx, cudaStream_t s);
+                           int D, float* partial, float* cand_score, int32_t* cand_idx, const int64_t* seg_first,
+                           const int32_t* seg_rows, cudaStream_t s);
 // cand_score [nq, splits, kc] fp32 (ascending), cand_idx [nq, splits, kc] int32 (-1 = empty)
 int tc_match_coarse(const __nv_bfloat16* Q16, int nq, const __nv_bfloat16* DB16, const float* dbnorm,
-                    long long N, int D, int kc, float* cand_score, int32_t* cand_idx, cudaStream_t s);
+                    long long N, int D, int kc, float* cand_score, int32_t* cand_idx, const int64_t* seg_first,
+                    const int32_t* seg_rows, cudaStream_t s);
 
 // fp32-storage DB: same pass with fp32 operands consumed as TF32 (dbnorm = ||x||^2 of the fp32 rows)
 int tc_match_coarse_tf32(const float* Q, int nq, const float* DB, const float* dbnorm, long long N, int D, int kc,
-                         float* cand_score, int32_t* cand_idx, cudaStream_t s);
+                         float* cand_score, int32_t* cand_idx, const int64_t* seg_first, const int32_t* seg_rows,
+                         cudaStream_t s);
 
 }  // namespace mocha

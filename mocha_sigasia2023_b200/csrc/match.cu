@@ -20,16 +20,29 @@ constexpr int EXQ = 4;  // queries per pass of the exact kernel
 // fp32 -> fp64 conversion amortised over the tile); warp shuffles + a small smem pass reduce over D.
 // <1,4> serves batch-1 streaming (385 CTAs for the reference-size DB), <8,8> serves batched queries
 // (L2 traffic per pair drops 5x, which is what bounds the small tile).
+// Segmented matching (seg_first / seg_rows non-NULL): query q needs only the rows seg_first[q] .. + seg_rows[q], and
+// a tile none of whose queries' segments meets its rows exits (the pairs it skips are never read by topk_rows_kernel).
 template <int RB, int QB>
 __global__ void __launch_bounds__(256)
 match_exact_tile_kernel(const float* __restrict__ Q, int nq, const float* __restrict__ DB, long long N, int D,
-                        double* __restrict__ dist2) {
+                        double* __restrict__ dist2, const int64_t* __restrict__ seg_first,
+                        const int32_t* __restrict__ seg_rows) {
   pdl_trigger();
   pdl_wait();
   __shared__ double red[8][RB * QB];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long row0 = (long long)blockIdx.x * RB;
   const int q0 = blockIdx.y * QB;
+  if (seg_first) {
+    bool meets = false;
+#pragma unroll
+    for (int j = 0; j < QB; ++j)
+      if (q0 + j < nq) {
+        const long long f = seg_first[q0 + j];
+        meets |= f < row0 + RB && f + seg_rows[q0 + j] > row0;
+      }
+    if (!meets) return;   // uniform over the block
+  }
   const float* xr[RB];
   const float* qr[QB];
 #pragma unroll
@@ -154,20 +167,29 @@ __device__ __forceinline__ void local_insert(T (&ls)[KMAX], I (&li)[KMAX], int k
   }
 }
 
-// one block per query: top-k over a row of squared distances
+// one block per query: top-k over a row of squared distances (segmented: over the query's rows only, clipped to
+// [0, N); missing entries are -1 / +inf)
 __global__ void __launch_bounds__(256)
 topk_rows_kernel(const double* __restrict__ dist2, long long N, int k, long long index_offset,
-                 int64_t* __restrict__ out_idx, double* __restrict__ out_dist) {
+                 int64_t* __restrict__ out_idx, double* __restrict__ out_dist, const int64_t* __restrict__ seg_first,
+                 const int32_t* __restrict__ seg_rows) {
   pdl_trigger();
   pdl_wait();
   __shared__ double red_d[8]; __shared__ long long red_i[8]; __shared__ int red_t[8];
   __shared__ double od[KMAX]; __shared__ long long oi[KMAX];
   const int q = blockIdx.x;
   const double* row = dist2 + (long long)q * N;
+  long long lo = 0, hi = N;
+  if (seg_first) {
+    lo = seg_first[q];
+    hi = lo + seg_rows[q];
+    lo = lo < 0 ? 0 : lo;
+    hi = hi > N ? N : hi;
+  }
   double ls[KMAX]; long long li[KMAX];
 #pragma unroll
   for (int t = 0; t < KMAX; ++t) { ls[t] = INFINITY; li[t] = -1; }
-  for (long long n = threadIdx.x; n < N; n += 256) local_insert(ls, li, k, row[n], n);
+  for (long long n = lo + threadIdx.x; n < hi; n += 256) local_insert(ls, li, k, row[n], n);
   block_topk_pop<256, double, long long>(ls, li, k, od, oi, red_d, red_i, red_t);
   if (threadIdx.x < k) {
     out_idx[(long long)q * k + threadIdx.x] = oi[threadIdx.x] >= 0 ? oi[threadIdx.x] + index_offset : -1;
@@ -440,29 +462,46 @@ extern "C" size_t mocha_match_exact_workspace_bytes(int nq, long long N, int k) 
   return align_up((size_t)nq * (size_t)N * sizeof(double), 256) + 256;
 }
 
-extern "C" int mocha_match_exact(const float* Q, int nq, const float* DB, long long N, int D, int k,
-                                 long long index_offset, int64_t* idx, double* dist, void* workspace,
-                                 size_t workspace_bytes, mocha_stream_t stream) {
-  MOCHA_CHECK_ARG(Q && DB && idx, "mocha_match_exact: null argument");
-  MOCHA_CHECK_ARG(nq > 0 && N > 0 && D > 0, "mocha_match_exact: empty problem nq=%d N=%lld D=%d", nq, N, D);
-  MOCHA_CHECK_ARG(k >= 1 && k <= KMAX && k <= N, "mocha_match_exact: k=%d out of range (1..min(%d,N))", k, KMAX);
+static int match_exact(const char* name, const float* Q, int nq, const float* DB, long long N, int D, int k,
+                       long long index_offset, const int64_t* seg_first, const int32_t* seg_rows, int64_t* idx,
+                       double* dist, void* workspace, size_t workspace_bytes, cudaStream_t s) {
+  MOCHA_CHECK_ARG(Q && DB && idx, "%s: null argument", name);
+  MOCHA_CHECK_ARG(nq > 0 && N > 0 && D > 0, "%s: empty problem nq=%d N=%lld D=%d", name, nq, N, D);
+  MOCHA_CHECK_ARG(k >= 1 && k <= KMAX && k <= N, "%s: k=%d out of range (1..min(%d,N))", name, k, KMAX);
   Workspace ws(workspace, workspace_bytes);
   double* dist2 = ws.take<double>((size_t)nq * (size_t)N);
   if (ws.overflow)
-    return set_error(MOCHA_ERR_WORKSPACE, "mocha_match_exact: workspace too small (%zu B given, %zu B needed)",
+    return set_error(MOCHA_ERR_WORKSPACE, "%s: workspace too small (%zu B given, %zu B needed)", name,
                      workspace_bytes, ws.off);
-  cudaStream_t s = (cudaStream_t)stream;
-  MOCHA_CHECK_ARG(N <= 2147483647LL && (nq + EXQ - 1) / EXQ <= 65535, "mocha_match_exact: problem too large for the exact kernel (use mocha_match_tc)");
+  MOCHA_CHECK_ARG(N <= 2147483647LL && (nq + EXQ - 1) / EXQ <= 65535, "%s: problem too large for the exact kernel (use mocha_match_tc)", name);
   if (nq >= 16 && N >= 64)
-    launch_k(match_exact_tile_kernel<8, 8>, dim3((unsigned)((N + 7) / 8), (unsigned)((nq + 7) / 8)), 256, 0, s, Q, nq, DB, N, D, dist2);
+    launch_k(match_exact_tile_kernel<8, 8>, dim3((unsigned)((N + 7) / 8), (unsigned)((nq + 7) / 8)), 256, 0, s, Q, nq, DB, N, D, dist2,
+             seg_first, seg_rows);
   else
-    launch_k(match_exact_tile_kernel<1, EXQ>, dim3((unsigned)N, (unsigned)((nq + EXQ - 1) / EXQ)), 256, 0, s, Q, nq, DB, N, D, dist2);
+    launch_k(match_exact_tile_kernel<1, EXQ>, dim3((unsigned)N, (unsigned)((nq + EXQ - 1) / EXQ)), 256, 0, s, Q, nq, DB, N, D, dist2,
+             seg_first, seg_rows);
   count_launch();
   MOCHA_LAUNCH_CHECK("match_exact_tile_kernel");
-  launch_k(topk_rows_kernel, nq, 256, 0, s, dist2, N, k, index_offset, idx, dist);
+  launch_k(topk_rows_kernel, nq, 256, 0, s, dist2, N, k, index_offset, idx, dist, seg_first, seg_rows);
   count_launch();
   MOCHA_LAUNCH_CHECK("topk_rows_kernel");
   return MOCHA_OK;
+}
+
+extern "C" int mocha_match_exact(const float* Q, int nq, const float* DB, long long N, int D, int k,
+                                 long long index_offset, int64_t* idx, double* dist, void* workspace,
+                                 size_t workspace_bytes, mocha_stream_t stream) {
+  return match_exact("mocha_match_exact", Q, nq, DB, N, D, k, index_offset, nullptr, nullptr, idx, dist, workspace,
+                     workspace_bytes, (cudaStream_t)stream);
+}
+
+extern "C" int mocha_match_exact_segmented(const float* Q, int nq, const float* DB, long long N, int D, int k,
+                                           long long index_offset, const int64_t* seg_first, const int32_t* seg_rows,
+                                           int64_t* idx, double* dist, void* workspace, size_t workspace_bytes,
+                                           mocha_stream_t stream) {
+  MOCHA_CHECK_ARG(seg_first && seg_rows, "mocha_match_exact_segmented: null segment table");
+  return match_exact("mocha_match_exact_segmented", Q, nq, DB, N, D, k, index_offset, seg_first, seg_rows, idx, dist,
+                     workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 extern "C" size_t mocha_match_tc_workspace_bytes(int nq, long long N, int D, int kc) {
@@ -473,16 +512,15 @@ extern "C" size_t mocha_match_tc_workspace_bytes(int nq, long long N, int D, int
   return 2 * (align_up((size_t)nq * lists * 4, 256)) + tc_match_splitk_ws_bytes(nq, N, D) + 512;
 }
 
-extern "C" int mocha_match_tc(const float* Q, const void* Q16, int nq, const void* DB16, const float* DB32,
-                              const float* dbnorm, long long N, int D, int k, int kc, long long index_offset,
-                              int64_t* idx, double* dist, void* workspace, size_t workspace_bytes,
-                              mocha_stream_t stream) {
-  MOCHA_CHECK_ARG(Q && dbnorm && idx && (DB16 || DB32), "mocha_match_tc: null argument");
-  MOCHA_CHECK_ARG(!DB16 || Q16, "mocha_match_tc: bf16 DB needs the bf16 query copy");
-  MOCHA_CHECK_ARG(k >= 1 && k <= kc && kc <= KMAX, "mocha_match_tc: need 1 <= k <= kc <= %d", KMAX);
-  MOCHA_CHECK_ARG(k <= N, "mocha_match_tc: k=%d > N=%lld", k, N);
+static int match_tc(const char* name, const float* Q, const void* Q16, int nq, const void* DB16, const float* DB32,
+                    const float* dbnorm, long long N, int D, int k, int kc, long long index_offset,
+                    const int64_t* seg_first, const int32_t* seg_rows, int64_t* idx, double* dist, void* workspace,
+                    size_t workspace_bytes, cudaStream_t s) {
+  MOCHA_CHECK_ARG(Q && dbnorm && idx && (DB16 || DB32), "%s: null argument", name);
+  MOCHA_CHECK_ARG(!DB16 || Q16, "%s: bf16 DB needs the bf16 query copy", name);
+  MOCHA_CHECK_ARG(k >= 1 && k <= kc && kc <= KMAX, "%s: need 1 <= k <= kc <= %d", name, KMAX);
+  MOCHA_CHECK_ARG(k <= N, "%s: k=%d > N=%lld", name, k, N);
   Workspace ws(workspace, workspace_bytes);
-  cudaStream_t s = (cudaStream_t)stream;
   if (DB16 && tc_match_splitk_slices(nq, N, D) > 0) {
     // small problem: K-sliced coarse pass, every row is a candidate of the fp64 re-rank's top-kc merge
     const size_t np = (size_t)((N + 127) / 128) * 128;
@@ -490,9 +528,10 @@ extern "C" int mocha_match_tc(const float* Q, const void* Q16, int nq, const voi
     int32_t* ci = ws.take<int32_t>((size_t)nq * np);
     float* partial = ws.take<float>(tc_match_splitk_ws_bytes(nq, N, D) / 4 - 64);
     if (ws.overflow)
-      return set_error(MOCHA_ERR_WORKSPACE, "mocha_match_tc: workspace too small (%zu B given, %zu B needed)",
+      return set_error(MOCHA_ERR_WORKSPACE, "%s: workspace too small (%zu B given, %zu B needed)", name,
                        workspace_bytes, ws.off);
-    MOCHA_TRY(tc_match_coarse_splitk((const __nv_bfloat16*)Q16, nq, (const __nv_bfloat16*)DB16, dbnorm, N, D, partial, cs, ci, s));
+    MOCHA_TRY(tc_match_coarse_splitk((const __nv_bfloat16*)Q16, nq, (const __nv_bfloat16*)DB16, dbnorm, N, D, partial, cs, ci,
+                                     seg_first, seg_rows, s));
     launch_k(match_rerank_kernel, nq, 256, 0, s, Q, (const __nv_bfloat16*)DB16, DB32, D, cs, ci, (int)np, kc, k, index_offset,
                                            idx, dist);
     count_launch();
@@ -504,17 +543,35 @@ extern "C" int mocha_match_tc(const float* Q, const void* Q16, int nq, const voi
   float* cs = ws.take<float>((size_t)nq * ncand);
   int32_t* ci = ws.take<int32_t>((size_t)nq * ncand);
   if (ws.overflow)
-    return set_error(MOCHA_ERR_WORKSPACE, "mocha_match_tc: workspace too small (%zu B given, %zu B needed)",
+    return set_error(MOCHA_ERR_WORKSPACE, "%s: workspace too small (%zu B given, %zu B needed)", name,
                      workspace_bytes, ws.off);
   if (DB16)
-    MOCHA_TRY(tc_match_coarse((const __nv_bfloat16*)Q16, nq, (const __nv_bfloat16*)DB16, dbnorm, N, D, kc, cs, ci, s));
+    MOCHA_TRY(tc_match_coarse((const __nv_bfloat16*)Q16, nq, (const __nv_bfloat16*)DB16, dbnorm, N, D, kc, cs, ci,
+                              seg_first, seg_rows, s));
   else  // fp32-storage DB: TF32 tensor-core pass straight from the fp32 rows
-    MOCHA_TRY(tc_match_coarse_tf32(Q, nq, DB32, dbnorm, N, D, kc, cs, ci, s));
+    MOCHA_TRY(tc_match_coarse_tf32(Q, nq, DB32, dbnorm, N, D, kc, cs, ci, seg_first, seg_rows, s));
   launch_k(match_rerank_kernel, nq, 256, 0, s, Q, (const __nv_bfloat16*)DB16, DB32, D, cs, ci, (int)ncand, kc, k,
                                          index_offset, idx, dist);
   count_launch();
   MOCHA_LAUNCH_CHECK("match_rerank_kernel");
   return MOCHA_OK;
+}
+
+extern "C" int mocha_match_tc(const float* Q, const void* Q16, int nq, const void* DB16, const float* DB32,
+                              const float* dbnorm, long long N, int D, int k, int kc, long long index_offset,
+                              int64_t* idx, double* dist, void* workspace, size_t workspace_bytes,
+                              mocha_stream_t stream) {
+  return match_tc("mocha_match_tc", Q, Q16, nq, DB16, DB32, dbnorm, N, D, k, kc, index_offset, nullptr, nullptr, idx,
+                  dist, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+extern "C" int mocha_match_tc_segmented(const float* Q, const void* Q16, int nq, const void* DB16, const float* DB32,
+                                        const float* dbnorm, long long N, int D, int k, int kc, long long index_offset,
+                                        const int64_t* seg_first, const int32_t* seg_rows, int64_t* idx, double* dist,
+                                        void* workspace, size_t workspace_bytes, mocha_stream_t stream) {
+  MOCHA_CHECK_ARG(seg_first && seg_rows, "mocha_match_tc_segmented: null segment table");
+  return match_tc("mocha_match_tc_segmented", Q, Q16, nq, DB16, DB32, dbnorm, N, D, k, kc, index_offset, seg_first,
+                  seg_rows, idx, dist, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 extern "C" int mocha_db_pack_bf16(const float* rows, long long N, int D, void* rows16, float* norm,
@@ -587,6 +644,40 @@ extern "C" int mocha_seed_rows(const uint8_t* start, const int64_t* idx, int idx
            reinterpret_cast<const float4*>(table), N, row_elems / 4, reinterpret_cast<float4*>(dst));
   count_launch();
   MOCHA_LAUNCH_CHECK("seed_rows_kernel");
+  return MOCHA_OK;
+}
+
+// Per-slot matcher segments of a character bank (one thread per slot): a starting slot takes its new character, then
+// every slot's segment is that character's rows; a character id outside [0, n_chars) gives an empty segment.
+__global__ void __launch_bounds__(128) slot_segments_kernel(const uint8_t* __restrict__ start, const int32_t* __restrict__ character,
+                                                            int32_t* __restrict__ slot_char, int B,
+                                                            const int64_t* __restrict__ char_first,
+                                                            const int32_t* __restrict__ char_rows, int n_chars,
+                                                            int64_t* __restrict__ seg_first, int32_t* __restrict__ seg_rows) {
+  pdl_trigger();
+  pdl_wait();
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  int c = slot_char[b];
+  if (start[b]) {
+    c = character[b];
+    slot_char[b] = c;
+  }
+  const bool ok = c >= 0 && c < n_chars;
+  seg_first[b] = ok ? char_first[c] : 0;
+  seg_rows[b] = ok ? char_rows[c] : 0;
+}
+
+extern "C" int mocha_slot_segments(const uint8_t* start, const int32_t* character, int32_t* slot_char, int B,
+                                   const int64_t* char_first, const int32_t* char_rows, int n_chars, int64_t* seg_first,
+                                   int32_t* seg_rows, mocha_stream_t stream) {
+  MOCHA_CHECK_ARG(start && character && slot_char && char_first && char_rows && seg_first && seg_rows,
+                  "mocha_slot_segments: null argument");
+  MOCHA_CHECK_ARG(B > 0 && n_chars > 0, "mocha_slot_segments: bad sizes (B=%d, n_chars=%d)", B, n_chars);
+  launch_k(slot_segments_kernel, (unsigned)((B + 127) / 128), 128, 0, (cudaStream_t)stream, start, character, slot_char, B,
+           char_first, char_rows, n_chars, seg_first, seg_rows);
+  count_launch();
+  MOCHA_LAUNCH_CHECK("slot_segments_kernel");
   return MOCHA_OK;
 }
 

@@ -16,6 +16,7 @@ import torch
 
 from . import _lib, kinematics, packing
 from .balltree import BallTree
+from .character_bank import _indexed
 
 
 @dataclass
@@ -35,7 +36,7 @@ class NormStats:
 class CharacterizationSession:
     def __init__(self, gen_sd, cvae_sd, cfg, stats: NormStats, cha_encoded, cha_cnt_nm, batch: int,
                  device="cuda", precision="fp32", with_cm_path=False, match_tensor_cores=None, post_params=None,
-                 lanes: int = 1, admission: bool = False, source_bank=None, result_bank=None):
+                 lanes: int = 1, admission: bool = False, source_bank=None, result_bank=None, characters=None):
         """gen_sd / cvae_sd: reference-layout state dicts. cha_encoded [N,90,256] and cha_cnt_nm [N,23040]
         (already (cnt-mean)/std scaled): the target character's feature DB, CUDA or CPU tensors.
 
@@ -59,7 +60,20 @@ class CharacterizationSession:
         result_bank (a ResultBank of the same source_bank): the last launch of each lane's frame, mocha_record_frames,
         records every serving slot's post-IK pose, integrated source root and matched DB row into the clip's record
         rows (the `post` path; the reference exports no other). serve() runs a list of bank clips through the slots and
-        returns each clip's bvh.save payload, built on the device."""
+        returns each clip's bvh.save payload, built on the device.
+
+        characters (a CharacterBank; needs admission=True, and cha_encoded = cha_cnt_nm = None): one session serves
+        every character of the bank. Every frame takes one more input, the int32 [B] row `character` (step_host(...,
+        character=), step_bank(..., character=), or a "character" entry of pinned_inputs()), read where start is set,
+        like `clip`. A started slot keeps its character until its next start, and each frame's matcher searches only
+        that character's rows (mocha_slot_segments, then the segmented matcher, on the match side stream); match_idx
+        holds rows of the whole bank. A slot whose character id is outside the bank matches nothing (index -1) and
+        keeps its seed. The matcher choice (match_tensor_cores) uses the bank's total row count."""
+        if characters is not None:
+            if not admission:
+                raise _lib.MochaError("characters (a CharacterBank) needs CharacterizationSession(admission=True)")
+            if cha_encoded is not None or cha_cnt_nm is not None:
+                raise _lib.MochaError("a session with a CharacterBank takes cha_encoded = cha_cnt_nm = None")
         if source_bank is not None and not admission:
             raise _lib.MochaError("source_bank needs CharacterizationSession(admission=True)")
         if result_bank is not None and source_bank is None:
@@ -84,16 +98,22 @@ class CharacterizationSession:
         self.cnt_mean, self.cnt_std = tab(stats.cnt_mean), tab(stats.cnt_std)
         self.m0, self.s0 = tab(stats.src_cnt_mean), tab(stats.src_cnt_std)
         self.m1, self.s1 = tab(stats.cha_encoded_mean), tab(stats.cha_encoded_std)
-        self.cha_encoded = torch.as_tensor(cha_encoded, dtype=torch.float32).to(dev).contiguous()
-        if isinstance(cha_cnt_nm, BallTree):      # a ready tree (e.g. BallTree.from_feature_db)
+        self.chars = characters
+        if characters is not None:
+            if characters.dev != _indexed(dev):
+                raise _lib.MochaError(f"the character bank is on {characters.dev}, this session on {dev}")
+            self.cha_encoded, self.tree = characters.encoded, characters.tree
+        elif isinstance(cha_cnt_nm, BallTree):      # a ready tree (e.g. BallTree.from_feature_db)
+            self.cha_encoded = torch.as_tensor(cha_encoded, dtype=torch.float32).to(dev).contiguous()
             self.tree = cha_cnt_nm
         else:
+            self.cha_encoded = torch.as_tensor(cha_encoded, dtype=torch.float32).to(dev).contiguous()
             self.tree = BallTree(torch.as_tensor(cha_cnt_nm, dtype=torch.float32).to(dev), device=dev,
                                  use_tensor_cores=match_tensor_cores)
         # matcher choice is fixed here: the tensor-core path needs the bf16 DB packed (which fixes the origin,
         # tree.center, of the bf16 query the encode stage emits) before the first frame runs
         t = self.tree
-        use_tc = t.use_tensor_cores
+        use_tc = match_tensor_cores if characters is not None else t.use_tensor_cores
         if use_tc is None or use_tc == "auto":
             # throughput mode: tensor-core coarse pass + fp64 re-rank (split-K when the DB is small);
             # parity mode (fp32) keeps the brute-force fp64 kernel unless the problem is large
@@ -124,6 +144,13 @@ class CharacterizationSession:
             self.slot_clip = torch.full((B,), -1, dtype=torch.int32, device=dev)
             self.slot_cursor = torch.zeros((B,), dtype=torch.int32, device=dev)
             self._input_names = ("start", "clip", "eps")
+        if characters is not None:
+            self.character = torch.zeros((B,), dtype=torch.int32, device=dev)    # character id of each starting slot
+            self.slot_char = torch.full((B,), -1, dtype=torch.int32, device=dev)
+            self.seg_first = torch.zeros((B,), dtype=torch.int64, device=dev)    # each slot's matcher segment
+            self.seg_rows = torch.zeros((B,), dtype=torch.int32, device=dev)
+            self.all_rows = torch.ones((B,), dtype=torch.uint8, device=dev)     # second decode's gather (seed_rows)
+            self._input_names += ("character",)
         self.results = result_bank
         if result_bank is not None:
             self.slot_count = torch.zeros((B,), dtype=torch.int32, device=dev)   # windows recorded by each slot's clip
@@ -180,6 +207,8 @@ class CharacterizationSession:
             self.h_start = torch.zeros((B,), dtype=torch.uint8).pin_memory()
         if self.bank is not None:
             self.h_clip = torch.zeros((B,), dtype=torch.int32).pin_memory()
+        if self.chars is not None:
+            self.h_character = torch.zeros((B,), dtype=torch.int32).pin_memory()
         self.h_out = torch.zeros(self.post.out.shape, dtype=torch.uint8).pin_memory()
         self.side = torch.zeros((B, d.T * 3 + 3 + 3), **f32)
 
@@ -218,7 +247,17 @@ class CharacterizationSession:
         wp, wn = self._ws(ws)
         q, q16 = self.cnt_nm[lo:hi], self.cnt_nm16[lo:hi]
         idx, dist = self.match_idx[lo:hi], self.match_dist[lo:hi]
-        if self._use_tc:
+        if self.chars is not None:
+            seg = (_lib.ptr(self.seg_first[lo:hi]), _lib.ptr(self.seg_rows[lo:hi]))
+            if self._use_tc:
+                _lib.check(lib.mocha_match_tc_segmented(
+                    _lib.ptr(q), _lib.ptr(q16), hi - lo, _lib.ptr(t._db16), _lib.ptr(t.data), _lib.ptr(t._norm), t.N, t.D,
+                    1, t.kc, 0, *seg, _lib.ptr(idx), _lib.ptr(dist), wp, wn, self._s()), "match_tc_segmented")
+            else:
+                _lib.check(lib.mocha_match_exact_segmented(_lib.ptr(q), hi - lo, _lib.ptr(t.data), t.N, t.D, 1, 0, *seg,
+                                                           _lib.ptr(idx), _lib.ptr(dist), wp, wn, self._s()),
+                           "match_exact_segmented")
+        elif self._use_tc:
             t._ensure_bf16()
             _lib.check(lib.mocha_match_tc(_lib.ptr(q), _lib.ptr(q16), hi - lo, _lib.ptr(t._db16),
                                           _lib.ptr(t.data), _lib.ptr(t._norm), t.N, t.D, 1, t.kc, 0,
@@ -255,6 +294,12 @@ class CharacterizationSession:
         side = self.match_streams[k]
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side):
+            if self.chars is not None:
+                c = self.chars
+                _lib.check(self.lib.mocha_slot_segments(
+                    _lib.ptr(self.start[sl]), _lib.ptr(self.character[sl]), _lib.ptr(self.slot_char[sl]), hi - lo,
+                    _lib.ptr(c.char_first), _lib.ptr(c.char_rows), c.n_chars, _lib.ptr(self.seg_first[sl]),
+                    _lib.ptr(self.seg_rows[sl]), self._s()), "slot_segments")
             self._match(lo, hi, self.match_ws[k])
         self._cvae_step(lo, hi, ws)
         torch.cuda.current_stream().wait_stream(side)       # join: a started clip's decoder needs its match
@@ -262,7 +307,12 @@ class CharacterizationSession:
         _lib.check(self.lib.mocha_seed_rows(_lib.ptr(self.start[sl]), _lib.ptr(self.match_idx[sl]), 1,
                                             _lib.ptr(self.cha_encoded), self.cha_encoded.shape[0], self.ntok * self.D,
                                             _lib.ptr(self.prev_cha[sl]), hi - lo, self._s()), "seed_rows")
-        if self.with_cm_path:
+        if self.with_cm_path and self.chars is not None:
+            # a slot without a character matched nothing (index -1): the gather leaves its row as it is
+            _lib.check(self.lib.mocha_seed_rows(_lib.ptr(self.all_rows[sl]), _lib.ptr(self.match_idx[sl]), 1,
+                                                _lib.ptr(self.cha_encoded), self.cha_encoded.shape[0], self.ntok * self.D,
+                                                _lib.ptr(self.cm_cha[sl]), hi - lo, self._s()), "seed_rows")
+        elif self.with_cm_path:
             torch.index_select(self.cha_encoded, 0, self.match_idx[sl, 0], out=self.cm_cha[sl])
         self._decode(self.encoded[sl], self.prev_cha[sl], self.decoded[sl], self.Y[sl], ws)
         self.post.step_packed(self.Y[sl], self.side[sl], self.contacts[sl], lo=lo, start=self.start[sl])
@@ -331,6 +381,7 @@ class CharacterizationSession:
         state_backup = (self.prev_cha.clone(), self.post.state.clone(),
                         self.cm_post.state.clone() if self.cm_post else None)
         slots_backup = (self.slot_clip.clone(), self.slot_cursor.clone()) if self.bank is not None else None
+        char_backup = self.slot_char.clone() if self.chars is not None else None
         rec_backup = ((self.slot_count.clone(), self.results.clip_done.clone(), self.results.clip_built.clone())
                       if self.results is not None else None)
         s = torch.cuda.Stream()
@@ -349,6 +400,8 @@ class CharacterizationSession:
         if slots_backup is not None:
             self.slot_clip.copy_(slots_backup[0])
             self.slot_cursor.copy_(slots_backup[1])
+        if char_backup is not None:
+            self.slot_char.copy_(char_backup)
         if rec_backup is not None:      # record rows the warm-up wrote are rewritten by the next real frame
             self.slot_count.copy_(rec_backup[0])
             self.results.clip_done.copy_(rec_backup[1])
@@ -366,13 +419,15 @@ class CharacterizationSession:
             self._frame_body(init)
         self.frame += 1
 
-    def step_host(self, X, src_hips_vel, src_rvel, src_rang, contacts, eps=None, start=None):
+    def step_host(self, X, src_hips_vel, src_rvel, src_rang, contacts, eps=None, start=None, character=None):
         """End-to-end call with HOST (numpy) inputs: pinned staging -> H2D -> frame -> D2H.
         start (admission mode only): uint8 [B], 1 = the slot starts a new clip on this frame; None = no slot starts.
+        character (sessions with a character bank only): int32 [B] character ids, read where start is set; None = all 0.
         Returns the frame outputs as a dict of float64 numpy arrays [B, ...]."""
         B, T = self.B, self.T
         if self.bank is not None:
             raise _lib.MochaError("a session with a source bank takes step_bank(start, clip, eps)")
+        self._stage_character(character)
         if self.admission:
             self.h_start.numpy()[...] = 0 if start is None else np.asarray(start, dtype=np.uint8)
             self.start.copy_(self.h_start, non_blocking=True)
@@ -397,12 +452,14 @@ class CharacterizationSession:
         torch.cuda.current_stream().synchronize()
         return self._decode_out(self.h_out.numpy())
 
-    def step_bank(self, start, clip, eps=None):
+    def step_bank(self, start, clip, eps=None, character=None):
         """End-to-end call of a session with a source bank: host (numpy) start row uint8 [B] (None = no slot starts),
-        clip row int32 [B] (bank clip ids, read where start is set; None = all 0) and optionally eps [B, D].
+        clip row int32 [B] (bank clip ids, read where start is set; None = all 0) and optionally eps [B, D]; with a
+        character bank, the int32 [B] character row (read where start is set; None = all 0).
         Returns the frame outputs as a dict of float64 numpy arrays [B, ...]."""
         if self.bank is None:
             raise _lib.MochaError("step_bank() needs CharacterizationSession(..., source_bank=...)")
+        self._stage_character(character)
         self.h_start.numpy()[...] = 0 if start is None else np.asarray(start, dtype=np.uint8)
         self.h_clip.numpy()[...] = 0 if clip is None else np.asarray(clip, dtype=np.int32)
         self.start.copy_(self.h_start, non_blocking=True)
@@ -417,13 +474,22 @@ class CharacterizationSession:
         torch.cuda.current_stream().synchronize()
         return self._decode_out(self.h_out.numpy())
 
+    def _stage_character(self, character):
+        if self.chars is None:
+            if character is not None:
+                raise _lib.MochaError("a character row needs CharacterizationSession(..., characters=CharacterBank)")
+            return
+        self.h_character.numpy()[...] = 0 if character is None else np.asarray(character, dtype=np.int32)
+        self.character.copy_(self.h_character, non_blocking=True)
+
     # ---------------------------------------------------------------------------------------------
     # pipelined end-to-end streaming: the H2D copy of frame i+1 overlaps the kernels of frame i
     # ---------------------------------------------------------------------------------------------
     def pinned_inputs(self):
         """A set of pinned host tensors a caller fills for one frame (shapes of step_host's arguments,
         with src_hips_vel/src_rvel/src_rang packed as `side` [B, T*3+6]; admission mode adds the uint8 [B] `start` row).
-        A session with a source bank takes `start`, `clip` (int32 [B]) and `eps` only."""
+        A session with a source bank takes `start`, `clip` (int32 [B]) and `eps` only; a character bank adds the int32 [B]
+        `character` row."""
         return {k: torch.zeros(getattr(self, k).shape, dtype=getattr(self, k).dtype).pin_memory()
                 for k in self._input_names}
 
@@ -471,7 +537,7 @@ class CharacterizationSession:
         self.step_device()
         return t, s
 
-    def serve(self, clip_ids, eps=None) -> dict:
+    def serve(self, clip_ids, eps=None, characters=None) -> dict:
         """Run the source bank's clips `clip_ids` through the slots and return {clip_id: payload}, each payload a dict
         of numpy arrays {src_rotations, src_positions [nwin,24,3] float32, ours_rotations, ours_positions [nwin,24,3]
         float64, match [nwin] int64}: what characterize() returns for one clip (test_fullframework.py:672-721).
@@ -487,6 +553,11 @@ class CharacterizationSession:
         eps None: eps.normal_() every frame, as step_bank does (the draws then depend on the schedule). Otherwise
         {clip_id: array [nwin-1, D]} in characterize()'s eps_seq layout: window w >= 1 of the clip uses row w-1,
         wherever and whenever it runs; clips without a table draw standard-normal rows on the host.
+
+        characters (required with a character bank, refused without): {clip_id: character id} (any mapping or
+        sequence indexed by clip id), checked against the bank before the first frame. Each clip is served toward its
+        character, and its payload's `match` is the row within that character's DB (the bank row minus
+        char_first[c]), what a single-character session records. ResultBank.read() keeps returning bank rows.
         """
         from .result_bank import PAYLOAD_KEYS, serving_schedule
         if self.results is None:
@@ -497,6 +568,17 @@ class CharacterizationSession:
         if not ids:
             return {}
         self.results._check_ids(ids)
+        if self.chars is not None:
+            if characters is None:
+                raise _lib.MochaError("serve(): this session has a character bank: pass characters={clip_id: character}")
+            try:
+                char_of = np.array([int(characters[c]) for c in ids], dtype=np.int64)
+            except (KeyError, IndexError) as e:
+                raise _lib.MochaError(f"serve(): no character for clip {e.args[0] if e.args else '?'}") from None
+            self.chars.check_ids(char_of)
+            char_of = char_of.astype(np.int32)
+        elif characters is not None:
+            raise _lib.MochaError("serve(characters=...) needs CharacterizationSession(..., characters=CharacterBank)")
         bank, B, D = self.bank, self.B, self.D
         nwins = np.array([bank.clip_nwin[c] for c in ids], dtype=np.int64)
         tables, rng = None, None
@@ -521,7 +603,8 @@ class CharacterizationSession:
         total = int(nwins.sum())
         host = [torch.empty((total,) + tuple(t.shape[1:]), dtype=t.dtype).pin_memory()
                 for t in self.results.payload_arrays()]
-        names = ("start", "clip") + (("eps",) if tables is not None else ())
+        names = (("start", "clip") + (("character",) if self.chars is not None else ())
+                 + (("eps",) if tables is not None else ()))
         pins = [{k: torch.zeros(getattr(self, k).shape, dtype=getattr(self, k).dtype).pin_memory() for k in names}
                 for _ in range(2)]
         pin_ready = [None, None]
@@ -532,6 +615,8 @@ class CharacterizationSession:
         slot_first = np.zeros(B, dtype=np.int64)
         self.start.fill_(1)                              # drop whatever the slots held: start them idle
         self.clip.fill_(-1)
+        if self.chars is not None:
+            self.character.fill_(-1)
         self.step_device()
         self.start.zero_()
         j = 0
@@ -542,6 +627,8 @@ class CharacterizationSession:
             st = start_rows[f]
             p["start"].numpy()[...] = st
             p["clip"].numpy()[...] = ids_np[clip_rows[f]]
+            if self.chars is not None:
+                p["character"].numpy()[...] = char_of[clip_rows[f]]
             new = np.nonzero(st)[0]
             slot_clip[new], slot_first[new] = clip_rows[f][new], f
             if tables is not None:
@@ -579,6 +666,10 @@ class CharacterizationSession:
         side.synchronize()
         main.synchronize()
         hv = [h.numpy() for h in host]
+        if self.chars is not None:              # bank rows -> rows of each clip's character DB
+            m = hv[PAYLOAD_KEYS.index("match")]
+            for k in range(len(ids)):
+                m[off[k]:off[k] + int(nwins[k])] -= self.chars.char_first_host[char_of[k]]
         return {ids[k]: {name: a[off[k]:off[k] + int(nwins[k])] for name, a in zip(PAYLOAD_KEYS, hv)}
                 for k in range(len(ids))}
 
@@ -589,10 +680,11 @@ class CharacterizationSession:
         return self._decode_out(s["h_out"].numpy())
 
     def h2d_bytes(self):
+        chars = self.h_character.numel() * 4 if self.chars is not None else 0
         if self.bank is not None:
-            return self.h_start.numel() + self.h_clip.numel() * 4 + self.h_eps.numel() * 4
+            return self.h_start.numel() + self.h_clip.numel() * 4 + self.h_eps.numel() * 4 + chars
         return (self.h_X.numel() * 4 + self.h_side.numel() * 4 + self.h_contacts.numel() + self.h_eps.numel() * 4
-                + (self.h_start.numel() if self.admission else 0))
+                + (self.h_start.numel() if self.admission else 0) + chars)
 
     def d2h_bytes(self):
         return self.h_out.numel()
