@@ -530,8 +530,7 @@ __device__ void ik_two_bone_dev(D3 bone_root, D3 bone_mid, D3 bone_end, D3 targe
 }
 
 // ------------------------------------------------------------------------------------------------
-// Frame-0 pieces shared by both post-process kernels (one definition, so the general kernel's init frame and the
-// step kernel's per-clip init agree bit for bit).
+// Frame-0 pieces of the post-process (:337-434).
 // ------------------------------------------------------------------------------------------------
 // source root at frame 0 (:476-483): integrated from the identity in fp64, stored as float32 values like the reference
 __device__ __forceinline__ void src_root_init_dev(mocha_frame_out& O, V3<float> rv, V3<float> ra, double dt) {
@@ -564,189 +563,32 @@ __device__ __forceinline__ void contact_init_dev(mocha_clip_state& S, const moch
 }
 
 // ------------------------------------------------------------------------------------------------
-// per-frame post-process, one WARP per clip: lanes split the 60-frame speed-ratio reduction, the 24
-// joints of the pose assembly, the 25 bones of the blending and the two feet of the contact / IK step;
-// lane 0 integrates the roots. Phases exchange data through the clip's output struct (__syncwarp).
-// start != NULL: clip b runs the frame-0 branch iff start[b] != 0 (per-clip admission; `init` is ignored).
-// ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128)
-post_frame_kernel(const mocha_post_params P, const float* __restrict__ Y,
-                  const float* __restrict__ src_hips_vel, const float* __restrict__ src_rvel,
-                  const float* __restrict__ src_rang, const uint8_t* __restrict__ contacts, int B,
-                  int T, int V, int Cin, int init, const uint8_t* __restrict__ start, mocha_clip_state* __restrict__ states,
-                  mocha_frame_out* __restrict__ outs, int hv_stride, int rv_stride) {
-  pdl_trigger();
-  pdl_wait();
-  const int b = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  if (b >= B) return;  // warp-uniform
-  if (start) init = start[b] != 0;   // warp-uniform (one warp per clip)
-  mocha_clip_state& S = states[b];
-  mocha_frame_out& O = outs[b];
-  const int J = P.J;
-  const double dt = P.dt;
-  const float* Yb = Y + (long long)b * T * V * Cin;
-  const float* last = Yb + (long long)(T - 1) * V * Cin;
-
-  // speed ratio (test_fullframework.py:492-496): mean |hips vel| over the window, fp32 like NumPy
-  float num = 0.f, den = 0.f;
-  for (int t = lane; t < T; t += 32) {
-    const float* yv = Yb + ((long long)t * V + 0) * Cin + 9;
-    num += sqrtf(yv[0] * yv[0] + yv[1] * yv[1] + yv[2] * yv[2]);
-    const float* sv = src_hips_vel + (long long)b * hv_stride + t * 3;
-    den += sqrtf(sv[0] * sv[0] + sv[1] * sv[1] + sv[2] * sv[2]);
-  }
-  num = warp_sum(num);
-  den = warp_sum(den);
-  float ratio = (num / (float)T) / (den / (float)T);
-  if (ratio > 3.0f || ratio < 0.33f) ratio = 1.0f;
-
-  DQ rootrot = q4<double>(1.0, 0.0, 0.0, 0.0);
-  D3 rootpos = v3<double>(0.0, 0.0, 0.0);
-  if (lane == 0) {
-    const D3 yrvel = v3<double>((double)(src_rvel[(long long)b * rv_stride + 0] * ratio), (double)(src_rvel[(long long)b * rv_stride + 1] * ratio),
-                                (double)(src_rvel[(long long)b * rv_stride + 2] * ratio));
-    const D3 yrang = v3<double>((double)src_rang[(long long)b * rv_stride + 0], (double)src_rang[(long long)b * rv_stride + 1], (double)src_rang[(long long)b * rv_stride + 2]);
-    // root integration (:500-503 / :345-348)
-    const DQ prev_rot = init ? q4<double>(1.0, 0.0, 0.0, 0.0) : ld4(S.root_rot);
-    const D3 prev_pos = init ? v3<double>(0.0, 0.0, 0.0) : ld3(S.root_pos);
-    const D3 rootvel = qrot(prev_rot, yrvel);
-    const D3 rootang = qrot(prev_rot, yrang);
-    rootpos = prev_pos + dt * rootvel;
-    rootrot = qmul(prev_rot, q_from_scaled_angle_axis(dt * rootang));
-    st3(O.pos[0], rootpos); st3(O.vel[0], rootvel); st4(O.rot[0], rootrot); st3(O.ang[0], rootang);
-  } else if (lane == 1) {
-    // source root (:476-483): the reference keeps it in float32 arrays, so it integrates in fp32
-    const V3<float> rv = v3<float>(src_rvel[(long long)b * rv_stride + 0], src_rvel[(long long)b * rv_stride + 1], src_rvel[(long long)b * rv_stride + 2]);
-    const V3<float> ra = v3<float>(src_rang[(long long)b * rv_stride + 0], src_rang[(long long)b * rv_stride + 1], src_rang[(long long)b * rv_stride + 2]);
-    if (init) {
-      src_root_init_dev(O, rv, ra, dt);
-    } else {
-      const Q4<float> pr = q4<float>((float)S.src_root_rot[0], (float)S.src_root_rot[1], (float)S.src_root_rot[2],
-                                     (float)S.src_root_rot[3]);
-      const V3<float> pp = v3<float>((float)S.src_root_pos[0], (float)S.src_root_pos[1], (float)S.src_root_pos[2]);
-      const float dtf = (float)dt;
-      const V3<float> wv = qrot(pr, rv), wa = qrot(pr, ra);
-      const V3<float> np_ = pp + dtf * wv;
-      const Q4<float> nr = qmul(pr, q_from_scaled_angle_axis(dtf * wa));
-      st3(O.src_root_vel, v3<double>((double)wv.x, (double)wv.y, (double)wv.z));
-      st3(O.src_root_ang, v3<double>((double)wa.x, (double)wa.y, (double)wa.z));
-      st3(O.src_root_pos, v3<double>((double)np_.x, (double)np_.y, (double)np_.z));
-      st4(O.src_root_rot, q4<double>((double)nr.w, (double)nr.x, (double)nr.y, (double)nr.z));
-    }
-    for (int c = 0; c < 3; ++c) S.src_root_pos[c] = O.src_root_pos[c];
-    for (int c = 0; c < 4; ++c) S.src_root_rot[c] = O.src_root_rot[c];
-  }
-
-  // assemble the 25-bone pose (:505-508): joint values are fp32 results promoted to fp64; lane = joint
-  for (int j = lane; j < V; j += 32) {
-    const float* y = last + (long long)j * Cin;
-    O.pos[j + 1][0] = (double)y[0]; O.pos[j + 1][1] = (double)y[1]; O.pos[j + 1][2] = (double)y[2];
-    const Q4<float> q = q_from_xy(v3<float>(y[3], y[5], y[7]), v3<float>(y[4], y[6], y[8]));
-    O.rot[j + 1][0] = (double)q.w; O.rot[j + 1][1] = (double)q.x; O.rot[j + 1][2] = (double)q.y; O.rot[j + 1][3] = (double)q.z;
-    O.vel[j + 1][0] = (double)y[9]; O.vel[j + 1][1] = (double)y[10]; O.vel[j + 1][2] = (double)y[11];
-    O.ang[j + 1][0] = (double)y[12]; O.ang[j + 1][1] = (double)y[13]; O.ang[j + 1][2] = (double)y[14];
-  }
-  __syncwarp();
-
-  if (init) {
-    // frame 0 (:375-434): lists start from the raw pose; contacts reset from the toe's FK state
-    for (int j = lane; j < J; j += 32) {
-      for (int c = 0; c < 3; ++c) {
-        O.blend_pos[j][c] = O.pos[j][c]; O.ik_pos[j][c] = O.pos[j][c];
-        S.prev_pos[j][c] = O.pos[j][c]; S.prev_ik_pos[j][c] = O.pos[j][c];
-      }
-      for (int c = 0; c < 4; ++c) O.ik_rot[j][c] = O.rot[j][c];
-    }
-    if (lane < 2) {
-      int chain[MAXJ]; int n = 0;
-      for (int j = P.contact_bones[lane]; j >= 0; j = P.parents[j]) chain[n++] = j;
-      contact_init_dev(S, O, chain, n, lane);
-    }
-    if (lane == 0) { st3(S.root_pos, rootpos); st4(S.root_rot, rootrot); }
-    return;
-  }
-
-  // position blending (:532-536, :626); lane = bone
-  for (int j = lane; j < J; j += 32) {
-    for (int c = 0; c < 3; ++c) {
-      O.ik_pos[j][c] = (S.prev_ik_pos[j][c] + O.vel[j][c] * dt) * 0.5 + O.pos[j][c] * 0.5;
-      O.blend_pos[j][c] = (S.prev_pos[j][c] + O.vel[j][c] * dt) * 0.5 + O.pos[j][c] * 0.5;
-    }
-    for (int c = 0; c < 4; ++c) O.ik_rot[j][c] = O.rot[j][c];
-  }
-  __syncwarp();
-
-  if (P.ik_enabled && lane < 2) {
-    const int f = lane;  // the two feet touch disjoint bones and disjoint state slots
-    const int toe = P.contact_bones[f], heel = P.parents[toe], knee = P.parents[heel], hip = P.parents[knee],
-              rootb = P.parents[hip];
-    // quat.fk_partial (motion/quat.py:241-272) along the toe's ancestor chain, on the blended pose
-    int chain[MAXJ]; int n = 0;
-    for (int j = toe; j >= 0; j = P.parents[j]) chain[n++] = j;
-    D3 gpos[MAXJ]; DQ grot[MAXJ];
-    {
-      const int r = chain[n - 1];
-      gpos[r] = ld3(O.ik_pos[r]); grot[r] = ld4(O.rot[r]);
-      for (int k = n - 2; k >= 0; --k) {
-        const int j = chain[k], p = chain[k + 1];
-        gpos[j] = qrot(grot[p], ld3(O.ik_pos[j])) + gpos[p];
-        grot[j] = qmul(grot[p], ld4(O.rot[j]));
-      }
-    }
-    ContactState c;
-    c.state = S.contact_state[f] != 0; c.lock = S.contact_lock[f] != 0;
-    c.position = ld3(S.contact_position[f]); c.velocity = ld3(S.contact_velocity[f]);
-    c.point = ld3(S.contact_point[f]); c.target = ld3(S.contact_target[f]);
-    c.off_pos = ld3(S.contact_offset_position[f]); c.off_vel = ld3(S.contact_offset_velocity[f]);
-    contact_update_dev(c, gpos[toe], contacts[b * 2 + f] != 0, P.ik_unlock_radius, P.ik_foot_height,
-                       P.ik_blending_halflife, dt);
-    // the clamp aliases contact_positions[bs] in the reference (:581-582): it persists
-    c.position.y = fmax(c.position.y, P.ik_foot_height);
-    S.contact_state[f] = c.state; S.contact_lock[f] = c.lock;
-    st3(S.contact_position[f], c.position); st3(S.contact_velocity[f], c.velocity);
-    st3(S.contact_point[f], c.point); st3(S.contact_target[f], c.target);
-    st3(S.contact_offset_position[f], c.off_pos); st3(S.contact_offset_velocity[f], c.off_vel);
-
-    const D3 target = c.position + (gpos[heel] - gpos[toe]);
-    const D3 fwd = qrot(grot[knee], v3<double>(0.0, 1.0, 0.0));
-    DQ new_hip, new_knee;
-    ik_two_bone_dev(gpos[hip], gpos[knee], gpos[heel], target, fwd, grot[hip], grot[knee], grot[rootb],
-                    P.ik_max_length_buffer, new_hip, new_knee);
-    st4(O.ik_rot[hip], new_hip);
-    st4(O.ik_rot[knee], new_knee);
-  }
-  __syncwarp();
-
-  // carry state
-  if (lane == 0) { st3(S.root_pos, ld3(O.blend_pos[0])); st4(S.root_rot, rootrot); }
-  for (int j = lane; j < J; j += 32)
-    for (int c = 0; c < 3; ++c) { S.prev_pos[j][c] = O.blend_pos[j][c]; S.prev_ik_pos[j][c] = O.ik_pos[j][c]; }
-}
-
-// ------------------------------------------------------------------------------------------------
-// Steady-state frame (init == 0) of the same post-process, shaped for latency: the kernel above walks its phases through
-// the clip's structs in GLOBAL memory (every phase boundary is an L2 round trip, the chain walk indexes local arrays), which
-// made it a 20 us tail on a step whose last kernel it is. Here one single-warp block per clip (clips spread over the SMs)
-// fetches everything the frame reads - state struct, last pose row, hips velocities, source root motion, contacts - in ONE
-// round of independent loads, runs the phases on shared-memory copies of the two structs (same expressions, same order:
-// fp64 results as above), and writes both structs back with 16-byte stores. The ancestor chains of the two contact bones
-// depend only on the parameters and are built before the grid dependency resolves.
-// MASKED: start[b] != 0 runs clip b's frame 0 instead (the general kernel's init branch: root from the identity, lists
-// from the raw pose, contacts reset from the toe FK), so clips can start on any frame of a batch. The flag is one byte per
-// block, read with the frame's other loads; the unmasked instantiation is the steady-state kernel alone.
+// Per-frame post-process, shaped for latency (it is the last kernel of a step): one single-warp block per clip (clips
+// spread over the SMs) fetches everything the frame reads - state struct, last pose row, hips velocities, source root
+// motion, contacts - in ONE round of independent loads, runs the phases on shared-memory copies of the two structs (no
+// L2 round trip between phases), and writes both structs back. The ancestor chains of the two contact bones depend only
+// on the parameters and are built before the grid dependency resolves. Lanes split the 60-frame speed-ratio reduction,
+// the 24 joints of the pose assembly and the 25 bones of the blending; lane 0 integrates the roots, lanes 0-1 run the
+// two feet's contact / IK step.
+// Frame 0 (root from the identity, lists from the raw pose, contacts reset from the toe FK) runs for clip b iff
+// start[b] != 0, or for every clip iff init_all != 0 when start is NULL, so clips can start on any frame of a batch;
+// the flag is one byte per block, read with the frame's other loads.
+// FRAME0 = false compiles the frame-0 branch out, for launches that are a steady-state step in every clip: with the
+// branch compiled in, the steady-state step of a 128-clip frame is about 3 us slower (NVIDIA B200, 1000 W power limit).
+// W is the unit of the global struct copies: double2 when both struct arrays are 16-byte aligned, double when a caller
+// offsets them by 8 bytes (the structs themselves only need 8).
 // ------------------------------------------------------------------------------------------------
 static_assert(sizeof(mocha_clip_state) % 16 == 0 && sizeof(mocha_frame_out) % 16 == 0, "struct copies use 16-byte vectors");
-constexpr int PF_S16 = (int)(sizeof(mocha_clip_state) / 16), PF_O16 = (int)(sizeof(mocha_frame_out) / 16);
-constexpr int PF_YMAX = 24 * 15;   // last pose row: V <= 24 joints x 15 features
+constexpr int PF_O16 = (int)(sizeof(mocha_frame_out) / 16);
+constexpr int PF_YMAX = 24 * 15;   // last pose row: post_frame_launch admits V = J - 1 <= 24 joints and Cin = 15
 
-template <bool MASKED>
+template <typename W, bool FRAME0>
 __global__ void __launch_bounds__(32)
-post_frame_step_kernel(const __grid_constant__ mocha_post_params P, const float* __restrict__ Y,
-                       const float* __restrict__ src_hips_vel, const float* __restrict__ src_rvel,
-                       const float* __restrict__ src_rang, const uint8_t* __restrict__ contacts,
-                       const uint8_t* __restrict__ start, int T, int V, int Cin, mocha_clip_state* __restrict__ states,
-                       mocha_frame_out* __restrict__ outs, int hv_stride, int rv_stride) {
+post_frame_kernel(const __grid_constant__ mocha_post_params P, const float* __restrict__ Y,
+                  const float* __restrict__ src_hips_vel, const float* __restrict__ src_rvel,
+                  const float* __restrict__ src_rang, const uint8_t* __restrict__ contacts, int init_all,
+                  const uint8_t* __restrict__ start, int T, int V, int Cin, mocha_clip_state* __restrict__ states,
+                  mocha_frame_out* __restrict__ outs, int hv_stride, int rv_stride) {
   pdl_trigger();
   __shared__ __align__(16) mocha_frame_out Osh;
   __shared__ __align__(16) mocha_clip_state Ssh;
@@ -771,12 +613,13 @@ post_frame_step_kernel(const __grid_constant__ mocha_post_params P, const float*
   const float* Yb = Y + (long long)b * T * V * Cin;
   const float* last = Yb + (long long)(T - 1) * V * Cin;
   const int nlast = V * Cin;
-  const double2* Sg = reinterpret_cast<const double2*>(states + b);
-  double2 sreg[(PF_S16 + 31) / 32];
+  constexpr int NS = (int)(sizeof(mocha_clip_state) / sizeof(W)), NO = (int)(sizeof(mocha_frame_out) / sizeof(W));
+  const W* Sg = reinterpret_cast<const W*>(states + b);
+  W sreg[(NS + 31) / 32];
 #pragma unroll
-  for (int k = 0; k < (PF_S16 + 31) / 32; ++k) {
+  for (int k = 0; k < (NS + 31) / 32; ++k) {
     const int i = lane + 32 * k;
-    sreg[k] = i < PF_S16 ? Sg[i] : make_double2(0.0, 0.0);
+    sreg[k] = i < NS ? Sg[i] : W{};
   }
   float yreg[(PF_YMAX + 31) / 32];
 #pragma unroll
@@ -798,12 +641,12 @@ post_frame_step_kernel(const __grid_constant__ mocha_post_params P, const float*
 #pragma unroll
   for (int c = 0; c < 3; ++c) { rvf[c] = src_rvel[(long long)b * rv_stride + c]; raf[c] = src_rang[(long long)b * rv_stride + c]; }
   const bool contact_in = lane < 2 ? contacts[b * 2 + lane] != 0 : false;
-  const bool init = MASKED && start[b] != 0;   // block-uniform
+  const bool init = FRAME0 && (start ? start[b] != 0 : init_all != 0);   // block-uniform
 
 #pragma unroll
-  for (int k = 0; k < (PF_S16 + 31) / 32; ++k) {
+  for (int k = 0; k < (NS + 31) / 32; ++k) {
     const int i = lane + 32 * k;
-    if (i < PF_S16) reinterpret_cast<double2*>(&Ssh)[i] = sreg[k];
+    if (i < NS) reinterpret_cast<W*>(&Ssh)[i] = sreg[k];
   }
 #pragma unroll
   for (int k = 0; k < (PF_YMAX + 31) / 32; ++k) {
@@ -945,10 +788,10 @@ post_frame_step_kernel(const __grid_constant__ mocha_post_params P, const float*
   for (int j = lane; j < J; j += 32)
     for (int c = 0; c < 3; ++c) { S.prev_pos[j][c] = O.blend_pos[j][c]; S.prev_ik_pos[j][c] = O.ik_pos[j][c]; }
   __syncwarp();
-  double2* Og = reinterpret_cast<double2*>(outs + b);
-  for (int i = lane; i < PF_O16; i += 32) Og[i] = reinterpret_cast<const double2*>(&Osh)[i];
-  double2* Sw = reinterpret_cast<double2*>(states + b);
-  for (int i = lane; i < PF_S16; i += 32) Sw[i] = reinterpret_cast<const double2*>(&Ssh)[i];
+  W* Og = reinterpret_cast<W*>(outs + b);
+  for (int i = lane; i < NO; i += 32) Og[i] = reinterpret_cast<const W*>(&Osh)[i];
+  W* Sw = reinterpret_cast<W*>(states + b);
+  for (int i = lane; i < NS; i += 32) Sw[i] = reinterpret_cast<const W*>(&Ssh)[i];
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1166,6 +1009,7 @@ int post_frame_launch(const mocha_post_params* params, const float* Y, const flo
                       mocha_stream_t stream) {
   MOCHA_CHECK_ARG(params && Y && src_hips_vel && src_rvel && src_rang && contacts && state && out && B > 0,
                   "mocha_post_frame: null/empty argument");
+  // with these two checks the kernel's last pose row fits its shared buffer: V * Cin <= PF_YMAX
   MOCHA_CHECK_ARG(params->J == V + 1 && params->J <= 25, "mocha_post_frame: J=%d must equal V+1=%d and be <= 25",
                   params->J, V + 1);
   MOCHA_CHECK_ARG(Cin == 15 && T > 0, "mocha_post_frame: pose feature layout needs Cin=15");
@@ -1178,19 +1022,11 @@ int post_frame_launch(const mocha_post_params* params, const float* Y, const flo
     MOCHA_CHECK_ARG(params->contact_bones[f] > 0 && params->contact_bones[f] < params->J && depth >= 4,
                     "mocha_post_frame: contact bone %d needs 4 ancestors", params->contact_bones[f]);
   }
-  // steady state: the latency-shaped kernel (shared-memory structs, one load round); frame 0 and unaligned struct arrays
-  // take the general kernel. A per-clip start row (start != NULL) takes the masked step kernel under the same rule.
   const bool aligned = ((reinterpret_cast<uintptr_t>(state) | reinterpret_cast<uintptr_t>(out)) & 15) == 0;
-  const bool step_kernel = aligned && V * Cin <= PF_YMAX;
-  if (start && step_kernel)
-    launch_k(post_frame_step_kernel<true>, B, 32, 0, (cudaStream_t)stream, *params, Y, src_hips_vel, src_rvel, src_rang, contacts,
-             start, T, V, Cin, state, out, hv_stride, rv_stride);
-  else if (!start && !init && step_kernel)
-    launch_k(post_frame_step_kernel<false>, B, 32, 0, (cudaStream_t)stream, *params, Y, src_hips_vel, src_rvel, src_rang, contacts,
-             nullptr, T, V, Cin, state, out, hv_stride, rv_stride);
-  else
-    launch_k(post_frame_kernel, nblk((long long)B * 32, 128), 128, 0, (cudaStream_t)stream, *params, Y, src_hips_vel, src_rvel, src_rang,
-                                                                   contacts, B, T, V, Cin, init, start, state, out, hv_stride, rv_stride);
+  const auto kernel = !aligned ? post_frame_kernel<double, true>
+                      : start || init ? post_frame_kernel<double2, true> : post_frame_kernel<double2, false>;
+  launch_k(kernel, B, 32, 0, (cudaStream_t)stream, *params, Y, src_hips_vel, src_rvel, src_rang, contacts, init, start, T, V,
+           Cin, state, out, hv_stride, rv_stride);
   count_launch();
   MOCHA_LAUNCH_CHECK("post_frame_kernel");
   return MOCHA_OK;

@@ -6,6 +6,7 @@ from __future__ import annotations
 
 import ctypes as C
 
+import numpy as np
 import torch
 
 from . import _lib, skeleton
@@ -190,6 +191,20 @@ def make_post_params(parents=None, contact_bones=None, dt=1.0 / 60.0, ik_enabled
     return p
 
 
+# mocha_frame_out as a numpy record: one clip's frame outputs, fp64
+FRAME_OUT_DTYPE = np.dtype([("pos", "f8", (25, 3)), ("rot", "f8", (25, 4)), ("vel", "f8", (25, 3)), ("ang", "f8", (25, 3)),
+                            ("blend_pos", "f8", (25, 3)), ("ik_pos", "f8", (25, 3)), ("ik_rot", "f8", (25, 4)),
+                            ("src_root_pos", "f8", (3,)), ("src_root_rot", "f8", (4,)), ("src_root_vel", "f8", (3,)),
+                            ("src_root_ang", "f8", (3,))])
+assert FRAME_OUT_DTYPE.itemsize == C.sizeof(_lib.FrameOut)
+
+
+def decode_frame_out(raw):
+    """uint8 bytes of [B] mocha_frame_out structs (host numpy) -> dict of float64 arrays [B, ...]."""
+    rec = raw.view(FRAME_OUT_DTYPE)
+    return {k: rec[k].copy() for k in FRAME_OUT_DTYPE.names}
+
+
 class PostProcessor:
     """Device-resident per-clip post-process state + the fused per-frame kernel (mocha_post_frame)."""
 
@@ -246,12 +261,4 @@ class PostProcessor:
 
     def read(self):
         """Copy the frame outputs to the host as a dict of float64 numpy arrays [B, ...]."""
-        import numpy as np
-        raw = self.out.cpu().numpy()
-        dt = np.dtype([("pos", "f8", (25, 3)), ("rot", "f8", (25, 4)), ("vel", "f8", (25, 3)), ("ang", "f8", (25, 3)),
-                       ("blend_pos", "f8", (25, 3)), ("ik_pos", "f8", (25, 3)), ("ik_rot", "f8", (25, 4)),
-                       ("src_root_pos", "f8", (3,)), ("src_root_rot", "f8", (4,)), ("src_root_vel", "f8", (3,)),
-                       ("src_root_ang", "f8", (3,))])
-        assert dt.itemsize == C.sizeof(_lib.FrameOut)
-        rec = raw.view(dt)
-        return {k: rec[k].copy() for k in dt.names}
+        return decode_frame_out(self.out.cpu().numpy())

@@ -450,7 +450,7 @@ class CharacterizationSession:
         self.step_device()
         self.h_out.copy_(self.post.out, non_blocking=True)
         torch.cuda.current_stream().synchronize()
-        return self._decode_out(self.h_out.numpy())
+        return kinematics.decode_frame_out(self.h_out.numpy())
 
     def step_bank(self, start, clip, eps=None, character=None):
         """End-to-end call of a session with a source bank: host (numpy) start row uint8 [B] (None = no slot starts),
@@ -472,7 +472,7 @@ class CharacterizationSession:
         self.step_device()
         self.h_out.copy_(self.post.out, non_blocking=True)
         torch.cuda.current_stream().synchronize()
-        return self._decode_out(self.h_out.numpy())
+        return kinematics.decode_frame_out(self.h_out.numpy())
 
     def _stage_character(self, character):
         if self.chars is None:
@@ -677,7 +677,7 @@ class CharacterizationSession:
         """Wait for a submitted frame and return its outputs (dict of float64 numpy arrays [B, ...])."""
         s = self._slots[ticket % 2]
         s["done"].synchronize()
-        return self._decode_out(s["h_out"].numpy())
+        return kinematics.decode_frame_out(s["h_out"].numpy())
 
     def h2d_bytes(self):
         chars = self.h_character.numel() * 4 if self.chars is not None else 0
@@ -688,12 +688,3 @@ class CharacterizationSession:
 
     def d2h_bytes(self):
         return self.h_out.numel()
-
-    @staticmethod
-    def _decode_out(raw):
-        dt = np.dtype([("pos", "f8", (25, 3)), ("rot", "f8", (25, 4)), ("vel", "f8", (25, 3)), ("ang", "f8", (25, 3)),
-                       ("blend_pos", "f8", (25, 3)), ("ik_pos", "f8", (25, 3)), ("ik_rot", "f8", (25, 4)),
-                       ("src_root_pos", "f8", (3,)), ("src_root_rot", "f8", (4,)), ("src_root_vel", "f8", (3,)),
-                       ("src_root_ang", "f8", (3,))])
-        rec = raw.view(dt)
-        return {k: rec[k].copy() for k in dt.names}

@@ -1,7 +1,8 @@
 """Clip admission (CharacterizationSession(admission=True)): a new clip can start in any slot on any frame of a running
 session, inside the one captured graph.
 
-- the masked post-process entry point against the init / steady entry points it stands in for, bit for bit;
+- the masked post-process entry point against the init / steady entry points it stands in for, and every one of them
+  on struct arrays 8 bytes off 16-byte alignment against the aligned arrays, bit for bit;
 - the seed copy against torch.where(start, table[idx], dst);
 - staggered starts and slot reuse are time-shift invariant: clip c at local frame f equals clip c run from frame 0 of a
   default session of the same batch size, bit for bit (bf16 and fp32), and the CPU oracle (fp32) within DESIGN §2's
@@ -35,7 +36,7 @@ def _post_inputs(B, seed):
 
 
 def _post_unaligned(pp, Y, side, ct, state0, out0, init=0, start=None):
-    """One frame on copies of the struct arrays placed 8 bytes off 16-byte alignment: that takes the general kernel."""
+    """One frame on copies of the struct arrays placed 8 bytes off 16-byte alignment (8-byte struct copies)."""
     B, T, V, Cin = Y.shape
     st = torch.empty(B * SS + 8, dtype=torch.uint8, device="cuda")
     ot = torch.empty(B * OS + 8, dtype=torch.uint8, device="cuda")
@@ -68,20 +69,22 @@ def test_masked_post_matches_init_and_step_entry_points():
         pp.step_packed(Y, side, ct, **kw)
         return pp.state.view(B, SS).clone(), pp.out.view(B, OS).clone()
 
-    s_init, o_init = run(init=1)                         # general kernel, frame 0
-    s_step, o_step = run(init=0)                         # steady-state kernel
+    s_init, o_init = run(init=1)                         # frame 0 in every clip
+    s_step, o_step = run(init=0)                         # steady state in every clip
     assert not torch.equal(s_init, s_step)
-    # the general kernel's steady step, for the masked launch on unaligned struct arrays
-    s_gstep, o_gstep = _post_unaligned(pp, Y, side, ct, state0, out0, init=0)
+    for init, want_s, want_o in ((1, s_init, o_init), (0, s_step, o_step)):
+        got_s, got_o = _post_unaligned(pp, Y, side, ct, state0, out0, init=init)
+        assert torch.equal(got_s, want_s), f"state (unaligned struct arrays), init={init}"
+        assert torch.equal(got_o, want_o), f"frame outputs (unaligned struct arrays), init={init}"
     for row in ([1, 0, 0, 1, 1, 0, 1, 0], [0] * B, [1] * B):
         start = torch.tensor(row, dtype=torch.uint8, device="cuda")
         m = start.bool()[:, None]
-        got_s, got_o = run(start=start)                  # masked step kernel
+        got_s, got_o = run(start=start)
         assert torch.equal(got_s, torch.where(m, s_init, s_step)), f"state, start row {row}"
         assert torch.equal(got_o, torch.where(m, o_init, o_step)), f"frame outputs, start row {row}"
-        got_s, got_o = _post_unaligned(pp, Y, side, ct, state0, out0, start=start)   # general kernel, per-clip flag
-        assert torch.equal(got_s, torch.where(m, s_init, s_gstep)), f"state (general kernel), start row {row}"
-        assert torch.equal(got_o, torch.where(m, o_init, o_gstep)), f"frame outputs (general kernel), start row {row}"
+        un_s, un_o = _post_unaligned(pp, Y, side, ct, state0, out0, start=start)
+        assert torch.equal(un_s, got_s), f"state (unaligned struct arrays), start row {row}"
+        assert torch.equal(un_o, got_o), f"frame outputs (unaligned struct arrays), start row {row}"
 
 
 @pytest.mark.gpu
